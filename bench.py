@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU code (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                   # + what the timed search computed, as DIR/<name>.npy
 
 Workload "C2" (BASELINE.json configs[1], SURVEY.md §8d): the simplified_piece mesh voxelised at a
 256-long grid (precision 0.823812/235.5, wall 10) and embedded in a 256^3 lattice whose node
@@ -31,6 +32,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # no .pyc files in the tree the benchmark runs from (which may be read-only)
 
 ANTS_PER_GPU = 4096
 STEP_CAP = 8192
@@ -377,6 +379,25 @@ def field_digest(acs):
     return int((t * w).sum(dtype=np.uint64))
 
 
+DUMP_TAU_SLOTS = 1 << 22     # pheromone slots in --dump-outputs: 16 MB of the 403 MB field
+
+
+def dump_outputs(acs, out_dir):
+    """--dump-outputs: what a caller of the timed search receives after its last step, as out_dir/<name>.npy — the best path
+    (node ids, directions, length), the search counters (in the order of ACS_Rank.counters(); in a sharded run those of rank 0's
+    shard, while the best path and the field are the same on every rank) and the pheromone field at a fixed
+    sample of slots (drawn with seed 0, ascending).  The workload and the search are seeded: with the same arguments every run
+    searches the same inputs, so two builds of the project can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    ids, dirs, L = acs.bestPath()
+    tau = acs.pheromone()
+    slots = np.unique(np.random.default_rng(0).integers(0, tau.size, DUMP_TAU_SLOTS))
+    arrays = {"best_path_ids": ids.astype(np.float64), "best_path_dirs": dirs.astype(np.float64), "best_length": np.array([L], np.float32),
+              "counters": np.array(list(acs.counters().values()), np.float64), "pheromone_sample": tau[slots]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------
 # this repo's arm
 # ---------------------------------------------------------------------------------------------------
@@ -449,6 +470,8 @@ def run_ours(args):
     sampler.mark_end()
     sampler.stop()
     c1 = acs.counters()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(acs, args.dump_outputs)     # before the kernels-alone leg below runs more updates on this handle
     if phase_in_timed:
         kms = acs.kernelMs()
         sk_ms, sk_n = acs.streamKernelMs()                  # the streaming kernel alone, by its own events inside the loop
@@ -888,10 +911,14 @@ def main():
     ap.add_argument("--no-k26", action="store_true", help="skip the K = 26 extension leg")
     ap.add_argument("--no-sub", action="store_true", help="skip the sub-records of the other BASELINE configurations (C3, C4, C5) and the full-search leg")
     ap.add_argument("--no-parity-check", action="store_true", help="N > 1: skip the sharded-vs-single-GPU self-check")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the timed search's best path, counters and a "
+                                                          "fixed sample of its pheromone field as DIR/<name>.npy")
     ap.add_argument("--worker-mode", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--worker", type=int, default=0, help=argparse.SUPPRESS)
     ap.add_argument("--budget-s", type=float, default=150.0, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed (--impl ours)")
     select_workload(args.workload)
     if args.ants <= 0:
         args.ants = ANTS_PER_GPU

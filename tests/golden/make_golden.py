@@ -16,8 +16,12 @@ Outputs (all under tests/golden/):
   ref_bspline.npz   BS_Basic<float, 3, D, CI, CF> of the unmodified core/BSplineBasic.h for eight setups: knots, control
                     points, curve points and return values at 261 times each (`python tests/golden/make_golden.py bspline`
                     regenerates only this file; the inputs are a pure function of the case, see bspline_inputs)
-Everything here is produced by reference code, not by the oracle restatement; the tests then
-hold the oracle (and through it the GPU) to these values on machines without /root/reference.
+  ref_live.json     what tests/test_oracle_vs_reference.py compares with, for exactly its inputs: voxel grid, grid file
+                    and its reload, a search on the `test` mesh, the all-pairs driver, GTSP on unrounded distances,
+                    36 B-spline setups (`python tests/golden/make_golden.py live` regenerates only this file; its
+                    "source" field names the code that produced it, see live_fixtures)
+Everything else here is produced by reference code, not by the oracle restatement; the tests then
+hold the oracle (and through it the GPU) to these values on machines without the reference sources.
 """
 import hashlib
 import json
@@ -166,10 +170,125 @@ def main():
             print("gtsp", n, ran, L)
     with open(os.path.join(HERE, "ref_kat.json"), "w") as f:
         json.dump(kat, f, indent=1)
+    live_fixtures()
     print("wrote fixtures to", HERE)
+
+
+# ---- inputs of tests/test_oracle_vs_reference.py (shared, so that the fixture and the tests cannot drift apart) -----------
+def search_points(G):
+    xs, ys, zs = G.coords()
+    return (xs[1], ys[1], zs[1]), (xs[-2], ys[-3], zs[-2])
+
+
+def all_pairs_points(G):
+    xs, ys, zs = G.coords()
+    return [(xs[2], ys[2], zs[2]), (xs[2], ys[-4], zs[3]), (xs[3], ys[5], zs[-3])]
+
+
+def gtsp_distances():
+    P = np.random.default_rng(21).random((24, 3))
+    return np.sqrt(((P[:, None] - P[None]) ** 2).sum(-1))
+
+
+def bspline_live_cases():
+    """Random valid setups of every (DEGREE, CI, CF) the harness instantiates, three sizes each (one rng, consumed in order)."""
+    rng = np.random.default_rng(3)
+    for (d, ci, cf) in [(0, 0, 0), (1, 0, 0), (2, 0, 0), (3, 0, 0), (2, 1, 1), (3, 1, 1), (2, 2, 2), (3, 2, 2), (4, 2, 2), (5, 2, 2), (3, 2, 1), (3, 0, 2)]:
+        for n, tf in [(max(1, d + 1 - ci - cf), 1.0), (57, 150.0), (1000, 123.456)]:
+            mid = rng.random((n, 9), dtype=np.float32) * 2 - 1
+            init = np.concatenate([mid[0, :3], rng.random(3 * ci) - 0.5]).astype(np.float32)
+            fin = np.concatenate([mid[-1, :3], rng.random(3 * cf) - 0.5]).astype(np.float32)
+            u = np.concatenate([np.linspace(-1, tf * 1.01, 301), [0, tf, tf * (1 - 1e-7), np.nan]]).astype(np.float32)
+            pre = rng.random((u.size, 3), dtype=np.float32)
+            yield (d, ci, cf, n, tf), (init, fin, mid, tf, u, pre)
+
+
+def live_fixtures():
+    """ref_live.json: what tests/test_oracle_vs_reference.py compares with.  Computed by the unmodified reference
+    (oracle/_ref/libwrref.so) where it is built.  Without it the values come from the oracle restatement, which that module
+    held bit-equal to the reference, live, on these very inputs when the restatement's sources last changed; "source"
+    records which of the two produced the file, and a run with the reference built re-records (and so re-checks) it."""
+    use_ref = O.have_ref()
+    meshes = dict(np.load(os.path.join(HERE, "meshes.npz")))
+    out = {"source": "reference (oracle/_ref/libwrref.so)" if use_ref else
+           "oracle restatement, as held bit-equal to the reference by tests/test_oracle_vs_reference.py when oracle/ last changed"}
+    # voxel grid, the grid file (the reference's dump carries the LAST triangle's box) and the reload of that file
+    tris = meshes["simplified_piece"]
+    with tempfile.TemporaryDirectory() as td:
+        f = os.path.join(td, "grid.in")
+        if use_ref:
+            R = O.Ref(); R.voxelize(tris, 0.015, 4, file=f)
+            dims, (free, xs, ys, zs) = R.dims, R.grid()
+            R3 = O.Ref(); R3.read_grid_file(f)
+            reload = R3.grid()
+        else:
+            G = O.Grid.from_triangles(tris, 0.015, 4, O.VOX_AABB); G.write_file(f, compat=True)
+            dims, (free, xs, ys, zs) = G.dims, (G.isfree(),) + G.coords()
+            H = O.Grid.read_file(f)
+            reload = (H.isfree(),) + H.coords()
+        out["grid"] = dict(dims=list(dims), sha256_isfree=sha(free), sha256_xyz=[sha(v) for v in (xs, ys, zs)],
+                           sha256_file=hashlib.sha256(open(f, "rb").read()).hexdigest(),
+                           reload_sha256_isfree=sha(reload[0]), reload_sha256_xyz=[sha(v) for v in reload[1:]])
+    # a search on the `test` mesh: best path, length and the whole pheromone field after 1, 3 and 25 iterations
+    G = O.Grid.from_triangles(meshes["test"], 0.08, 4, O.VOX_AABB)
+    p, q = search_points(G)
+    if use_ref:
+        R = O.Ref(); R.voxelize(meshes["test"], 0.08, 4); R.acs_init()
+    else:
+        A = O.Acs(G, rng_mode=O.RNG_SEQUENTIAL, sort_mode=O.SORT_STD, seed=99)
+    out["search"] = {"set_points": list(R.set_points(p, q) if use_ref else A.set_points(p, q))}
+    for iters in (1, 3, 25):
+        if use_ref:
+            R.compute(3.0, iters, 99); ids, dirs, L = R.best(); tau = R.pheromone(); R.reset()
+        else:
+            A.begin(3.0); A.iterate(iters); ids, dirs, L = A.best(); tau = A.pheromone(); A.reset()
+        out["search"][str(iters)] = dict(L_bits=int(np.float32(L).view(np.int32)), sha256_ids=sha(ids.astype(np.int64)),
+                                         sha256_dirs=sha(dirs.astype(np.int32)), sha256_tau=sha(tau))
+    # the all-pairs driver (searchBestPathOfPoints, ACSRank_3D.hpp:427-504): one Philox stream over the pairs, never reseeded
+    G = O.Grid.from_triangles(meshes["cubic"], 0.01, 5, O.VOX_AABB)
+    pts = all_pairs_points(G)
+    pairs = []
+    if use_ref:
+        R = O.Ref(); R.voxelize(meshes["cubic"], 0.01, 5)
+        with tempfile.TemporaryDirectory() as td:
+            cnt, lens = R.search_all(pts, 0.4, 4242, td)
+            graph = open(os.path.join(td, "graph.in")).read()
+        assert cnt == 3 and graph.startswith("3 3")   # "%d %d\r" header rewrite (:500-501)
+        for i in range(3):
+            for j in range(i + 1, 3):
+                ids, L = R.pair_best(i, j)
+                assert np.float32(L).tobytes() == np.float32(lens[i, j]).tobytes()
+                pairs.append(dict(L_bits=int(np.float32(L).view(np.int32)), sha256_ids=sha(ids.astype(np.int64))))
+    else:
+        A = O.Acs(G, rng_mode=O.RNG_SEQUENTIAL, sort_mode=O.SORT_STD, seed=4242)
+        for k, (i, j) in enumerate([(0, 1), (0, 2), (1, 2)]):
+            assert A.set_points(pts[i], pts[j])[0]
+            A.begin(0.4, seq_pos=None if k else 0); A.iterate(150)
+            ids, _, L = A.best(); A.reset()
+            pairs.append(dict(L_bits=int(np.float32(L).view(np.int32)), sha256_ids=sha(ids.astype(np.int64))))
+    out["all_pairs"] = pairs
+    # seam ordering on unrounded distances, stagnation stop
+    D = gtsp_distances()
+    if use_ref:
+        with tempfile.TemporaryDirectory() as td:
+            T = O.RefGtsp(D, os.path.join(td, "g.in")); ran, _ = T.run(30, 5)
+    else:
+        T = O.Gtsp(D, seed=5, rng_mode=O.RNG_SEQUENTIAL); ran = T.iterate(30, early_stop=True)
+    tour, L = T.best()
+    out["gtsp"] = dict(ran=int(ran), tour=tour.ravel().tolist(), L_hex=float(L).hex(), sha256_pheromone=sha(T.pheromone()))
+    # BS_Basic<float, 3, D, CI, CF>: points, return values, knots, control points
+    out["bspline"] = []
+    for case, (init, fin, mid, tf, u, pre) in bspline_live_cases():
+        pts_, ok, knots, cps = O.bspline(case[0], case[1], case[2], init, fin, mid, tf, u, out=pre, use_ref=use_ref)
+        out["bspline"].append(dict(case=list(case), sha256=[sha(pts_), sha(ok), sha(knots), sha(cps)]))
+    with open(os.path.join(HERE, "ref_live.json"), "w") as fp:
+        json.dump(out, fp, indent=1)
+    print("ref_live.json from", out["source"])
 
 
 if __name__ == "__main__" and sys.argv[1:] == ["bspline"]:
     bspline_fixtures()
+elif __name__ == "__main__" and sys.argv[1:] == ["live"]:
+    live_fixtures()
 elif __name__ == "__main__":
     main()

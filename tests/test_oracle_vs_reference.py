@@ -1,118 +1,100 @@
-"""CPU: the oracle restatement against the UNMODIFIED reference run live (oracle/_ref/libwrref.so,
-built by oracle/Makefile from /root/reference).  Skipped where that library is absent."""
+"""CPU: the oracle restatement against what the UNMODIFIED reference computes for these inputs, stored in
+tests/golden/ref_live.json (tests/golden/make_golden.py live: recorded through oracle/_ref/libwrref.so where that is built,
+its "source" field says by what), bit for bit."""
+import hashlib
+import json
 import os
+import sys
 import tempfile
 
 import numpy as np
 import pytest
 
-from conftest import C1_POINTS
+from conftest import GOLDEN
+
+sys.path.insert(0, GOLDEN)
+import make_golden as MG  # noqa: E402
+
+
+def sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 @pytest.fixture(scope="module")
-def O(oracle):
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref/libwrref.so not built (no /root/reference here)")
-    oracle.ref()
-    return oracle
+def live():
+    with open(os.path.join(GOLDEN, "ref_live.json")) as f:
+        return json.load(f)
 
 
-def test_voxel_grid_and_grid_file_round_trip(O, meshes):
-    tris = meshes["simplified_piece"]
-    R = O.Ref(); R.voxelize(tris, 0.015, 4)
-    free, xs, ys, zs = R.grid()
-    G = O.Grid.from_triangles(tris, 0.015, 4, O.VOX_AABB)
-    assert G.dims == R.dims and np.array_equal(G.isfree(), free)
-    for a, b in zip(G.coords(), (xs, ys, zs)):
-        assert np.array_equal(a.view(np.uint32), b.view(np.uint32))
+def test_voxel_grid_and_grid_file_round_trip(oracle, meshes, live):
+    want = live["grid"]
+    G = oracle.Grid.from_triangles(meshes["simplified_piece"], 0.015, 4, oracle.VOX_AABB)
+    xs, ys, zs = G.coords()
+    assert list(G.dims) == want["dims"] and sha(G.isfree()) == want["sha256_isfree"]
+    assert [sha(v) for v in (xs, ys, zs)] == want["sha256_xyz"]
     with tempfile.TemporaryDirectory() as td:
         # the reference's dump carries the LAST triangle's box (model_grid_map.hpp:279): its own reload
         # rebuilds wrong coordinates; compat=True reproduces that, compat=False writes the global box
-        f_ref = os.path.join(td, "ref.in"); f_compat = os.path.join(td, "compat.in"); f_fixed = os.path.join(td, "fixed.in")
-        R2 = O.Ref(); R2.voxelize(tris, 0.015, 4, file=f_ref)
+        f_compat = os.path.join(td, "compat.in"); f_fixed = os.path.join(td, "fixed.in")
         G.write_file(f_compat, compat=True); G.write_file(f_fixed, compat=False)
-        assert open(f_ref).read() == open(f_compat).read()
-        R3 = O.Ref(); R3.read_grid_file(f_ref)
-        free3, xs3, ys3, zs3 = R3.grid()
-        H = O.Grid.read_file(f_compat)
-        assert np.array_equal(H.isfree(), free3)
-        for a, b in zip(H.coords(), (xs3, ys3, zs3)):
-            assert np.array_equal(a.view(np.uint32), b.view(np.uint32))
-        assert not np.array_equal(xs3, xs)        # the reference bug, reproduced
-        F = O.Grid.read_file(f_fixed)
+        assert hashlib.sha256(open(f_compat, "rb").read()).hexdigest() == want["sha256_file"]
+        H = oracle.Grid.read_file(f_compat)
+        assert sha(H.isfree()) == want["reload_sha256_isfree"]
+        assert [sha(v) for v in H.coords()] == want["reload_sha256_xyz"]
+        assert not np.array_equal(H.coords()[0], xs)        # the reference bug, reproduced
+        F = oracle.Grid.read_file(f_fixed)
         assert np.allclose(F.coords()[0], xs, atol=1e-6)
 
 
-def test_search_live_on_second_mesh(O, meshes):
-    """A search on a mesh the fixtures do not cover: best path, length and the full pheromone field
+def test_search_live_on_second_mesh(oracle, meshes, live):
+    """A search on a mesh the other fixtures do not cover: best path, length and the full pheromone field
     after 1, 3 and 25 iterations, bit for bit, under the shared sequential Philox stream."""
-    tris = meshes["test"]
-    R = O.Ref(); R.voxelize(tris, 0.08, 4); R.acs_init()
-    G = O.Grid.from_triangles(tris, 0.08, 4, O.VOX_AABB)
-    A = O.Acs(G, rng_mode=O.RNG_SEQUENTIAL, sort_mode=O.SORT_STD, seed=99)
-    xs, ys, zs = G.coords()
-    p, q = (xs[1], ys[1], zs[1]), (xs[-2], ys[-3], zs[-2])
-    assert R.set_points(p, q) == A.set_points(p, q)
+    want = live["search"]
+    G = oracle.Grid.from_triangles(meshes["test"], 0.08, 4, oracle.VOX_AABB)
+    A = oracle.Acs(G, rng_mode=oracle.RNG_SEQUENTIAL, sort_mode=oracle.SORT_STD, seed=99)
+    p, q = MG.search_points(G)
+    assert list(A.set_points(p, q)) == want["set_points"]
     for iters in (1, 3, 25):
-        calls = R.compute(3.0, iters, 99)
         A.begin(3.0); A.iterate(iters)
-        rb, ob = R.best(), A.best()
-        assert np.float32(rb[2]).tobytes() == np.float32(ob[2]).tobytes()
-        assert np.array_equal(rb[0], ob[0]) and np.array_equal(rb[1], ob[1])
-        assert np.array_equal(R.pheromone().view(np.uint32), A.pheromone().view(np.uint32))
-        R.reset(); A.reset()
+        ids, dirs, L = A.best()
+        w = want[str(iters)]
+        assert int(np.float32(L).view(np.int32)) == w["L_bits"]
+        assert sha(ids.astype(np.int64)) == w["sha256_ids"] and sha(dirs.astype(np.int32)) == w["sha256_dirs"]
+        assert sha(A.pheromone()) == w["sha256_tau"]
+        A.reset()
     assert A.counters()["finite_fallthrough"] == 0
 
 
-def test_all_pairs_driver_through_files(O, meshes):
-    """The genuine searchBestPathOfPoints (ACSRank_3D.hpp:427-504) through its file interface."""
-    R = O.Ref(); R.voxelize(meshes["cubic"], 0.01, 5)
-    G = O.Grid.from_triangles(meshes["cubic"], 0.01, 5, O.VOX_AABB)
-    xs, ys, zs = G.coords()
-    pts = [(xs[2], ys[2], zs[2]), (xs[2], ys[-4], zs[3]), (xs[3], ys[5], zs[-3])]
-    with tempfile.TemporaryDirectory() as td:
-        cnt, lens = R.search_all(pts, 0.4, 4242, td)
-        graph = open(os.path.join(td, "graph.in")).read()
-    assert cnt == 3
-    A = O.Acs(G, rng_mode=O.RNG_SEQUENTIAL, sort_mode=O.SORT_STD, seed=4242)
-    k = 0
-    for i in range(3):
-        for j in range(i + 1, 3):
-            assert A.set_points(pts[i], pts[j])[0]
-            A.begin(0.4, seq_pos=None if k else 0); A.iterate(150)   # the driver never reseeds between pairs
-            ids, dirs, L = A.best()
-            A.reset()
-            rid, rL = R.pair_best(i, j)
-            assert np.float32(L).tobytes() == np.float32(rL).tobytes() == np.float32(lens[i, j]).tobytes() and np.array_equal(ids, rid)
-            k += 1
-    assert graph.startswith("3 3\r") or graph.startswith("3 3")   # "%d %d\r" header rewrite (:500-501)
+def test_all_pairs_driver_through_files(oracle, meshes, live):
+    """The genuine searchBestPathOfPoints (ACSRank_3D.hpp:427-504), which drives the pairs through its file interface:
+    every pair's best path and length."""
+    G = oracle.Grid.from_triangles(meshes["cubic"], 0.01, 5, oracle.VOX_AABB)
+    pts = MG.all_pairs_points(G)
+    A = oracle.Acs(G, rng_mode=oracle.RNG_SEQUENTIAL, sort_mode=oracle.SORT_STD, seed=4242)
+    pairs = [(i, j) for i in range(3) for j in range(i + 1, 3)]
+    assert len(pairs) == len(live["all_pairs"]) == 3
+    for k, ((i, j), w) in enumerate(zip(pairs, live["all_pairs"])):
+        assert A.set_points(pts[i], pts[j])[0]
+        A.begin(0.4, seq_pos=None if k else 0); A.iterate(150)   # the driver never reseeds between pairs
+        ids, dirs, L = A.best()
+        A.reset()
+        assert int(np.float32(L).view(np.int32)) == w["L_bits"] and sha(ids.astype(np.int64)) == w["sha256_ids"]
 
 
-def test_gtsp_live(O):
-    P = np.random.default_rng(21).random((24, 3))
-    D = np.sqrt(((P[:, None] - P[None]) ** 2).sum(-1))
-    with tempfile.TemporaryDirectory() as td:
-        Rg = O.RefGtsp(D, os.path.join(td, "g.in"))
-        ran, calls = Rg.run(30, 5)
-    T = O.Gtsp(D, seed=5, rng_mode=O.RNG_SEQUENTIAL)
-    assert T.iterate(30, early_stop=True) == ran
-    assert np.array_equal(T.best()[0], Rg.best()[0]) and T.best()[1] == Rg.best()[1]
-    assert np.array_equal(T.pheromone().view(np.uint64), Rg.pheromone().view(np.uint64))
+def test_gtsp_live(oracle, live):
+    want = live["gtsp"]
+    T = oracle.Gtsp(MG.gtsp_distances(), seed=5, rng_mode=oracle.RNG_SEQUENTIAL)
+    assert T.iterate(30, early_stop=True) == want["ran"]
+    tour, L = T.best()
+    assert tour.ravel().tolist() == want["tour"] and float(L).hex() == want["L_hex"]
+    assert sha(T.pheromone()) == want["sha256_pheromone"]
 
 
-def test_bspline_restatement_equals_reference_header(oracle):
-    """Live: random valid setups of every (DEGREE, CI, CF) the harness instantiates, restatement == unmodified BSplineBasic.h."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
-    rng = np.random.default_rng(3)
-    bits = lambda a: a.view(np.uint32) if a.dtype == np.float32 else a   # noqa: E731
-    for (d, ci, cf) in [(0, 0, 0), (1, 0, 0), (2, 0, 0), (3, 0, 0), (2, 1, 1), (3, 1, 1), (2, 2, 2), (3, 2, 2), (4, 2, 2), (5, 2, 2), (3, 2, 1), (3, 0, 2)]:
-        for n, tf in [(max(1, d + 1 - ci - cf), 1.0), (57, 150.0), (1000, 123.456)]:
-            mid = rng.random((n, 9), dtype=np.float32) * 2 - 1
-            init = np.concatenate([mid[0, :3], rng.random(3 * ci) - 0.5]).astype(np.float32)
-            fin = np.concatenate([mid[-1, :3], rng.random(3 * cf) - 0.5]).astype(np.float32)
-            u = np.concatenate([np.linspace(-1, tf * 1.01, 301), [0, tf, tf * (1 - 1e-7), np.nan]]).astype(np.float32)
-            pre = rng.random((u.size, 3), dtype=np.float32)
-            a = oracle.bspline(d, ci, cf, init, fin, mid, tf, u, out=pre)
-            b = oracle.bspline(d, ci, cf, init, fin, mid, tf, u, out=pre, use_ref=True)
-            assert all(np.array_equal(bits(x), bits(y)) for x, y in zip(a, b)), (d, ci, cf, n, tf)
+def test_bspline_restatement_equals_reference_header(oracle, live):
+    """Random valid setups of every (DEGREE, CI, CF) the harness instantiates, restatement == unmodified BSplineBasic.h."""
+    cases = list(MG.bspline_live_cases())
+    assert len(cases) == len(live["bspline"]) == 36
+    for (case, (init, fin, mid, tf, u, pre)), w in zip(cases, live["bspline"]):
+        assert list(case) == w["case"]
+        pts, ok, knots, cps = oracle.bspline(case[0], case[1], case[2], init, fin, mid, tf, u, out=pre)
+        assert [sha(pts), sha(ok), sha(knots), sha(cps)] == w["sha256"], case
