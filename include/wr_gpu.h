@@ -83,7 +83,7 @@ typedef struct {
     float rho;            /* evaporation factor, :321 (0.8)                        */
     float tau0;           /* initial pheromone, :324 (1)                           */
     int fixed_colony;     /* 0: adaptive colony_num of :247; >0: that many ants    */
-    int step_cap;         /* 0: auto (min(N-1, 65534)); else max steps per ant     */
+    int step_cap;         /* 0: auto (min(N-1, 65532)); else max steps per ant     */
     int K;                /* neighbourhood: 6 (reference) or 26 (the extension disabled at :367-385; one GPU) */
     uint64_t seed;        /* Philox key; draw = f(seed; search, iteration, ant, step) */
     int update_mode;      /* WR_UPDATE_*; default WR_UPDATE_RANKSET (adaptive)     */

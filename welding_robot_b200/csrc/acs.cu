@@ -886,8 +886,11 @@ static int launch_rank(wr_acs* a, const int* d_all_steps)
         const int nchunks = (cm + kRankChunk - 1) / kRankChunk;
         k_rank_chunks<<<nchunks, kRankSmallThreads, kRankChunkSmem, s>>>(a->d_state, d_all_steps, d_L, a->cap, a->rank_bits, a->sort_ants.keys_b, a->sort_ants.vals_b);
         const int stage = std::min(nchunks, 24);
+        // 16-bit staged keys hold K = 6 step counts up to cap + 1 (a dead ant) while that fits: the automatic cap (<= 65532)
+        // always does, an explicit step_cap of 65535 or more does not.  Those, and K = 26 (bits of L), compare in global memory.
+        const int keys16 = a->K == 6 && (long long)a->cap + 1 <= 0xFFFF;
         k_rank_merge<<<(cm + kRankMergeThreads - 1) / kRankMergeThreads, kRankMergeThreads, (size_t)stage * kRankChunk * sizeof(uint16_t), s>>>(
-            a->d_state, a->sort_ants.keys_b, a->sort_ants.vals_b, a->sort_ants.keys_a, a->sort_ants.vals_a, a->d_order, a->K == kK26 ? 0 : 1);
+            a->d_state, a->sort_ants.keys_b, a->sort_ants.vals_b, a->sort_ants.keys_a, a->sort_ants.vals_a, a->d_order, keys16);
         k_rank_finish_prefix<<<1, 1024, 0, s>>>(a->d_state, a->sort_ants.keys_a, a->sort_ants.vals_a, a->cap, a->d_Ltab, a->d_rec_off, a->w_max,
                                                 a->K == kK26 ? d_all_steps : nullptr, a->d_best_n, a->d_best_ids, a->d_onbest);
     }

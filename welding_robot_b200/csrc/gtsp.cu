@@ -287,11 +287,39 @@ extern "C" int wr_gtsp_destroy(wr_gtsp* g)
     return WR_OK;
 }
 
+// TMA ring depth 3 (two CTAs per SM at N = 256) measured best: 2 -> 33.0k, 3 -> 34.7k, 4 -> 31.9k, 6 -> 21.3k colony-iterations/s
+// at N = 256 x 1024 colonies (per-CTA latency wants more CTAs per SM, L2 capacity wants fewer resident matrices)
+constexpr int kGtspStages = 3;
+constexpr size_t kGtspSmemMax = 227 * 1024;
+
+// dynamic shared memory of k_gtsp_iterate for n cities: the ring of matrix rows, then per ant (one per thread) its
+// check-points and visited bits, then the reduction and barrier words
+static size_t gtsp_smem(int n, int stages)
+{
+    const size_t npad = (size_t)((n + 1) & ~1), threads = (size_t)(n + 31) / 32 * 32;
+    const size_t nck = (size_t)(n + kGtspIv - 1) / kGtspIv, nwords = (size_t)(n + 31) / 32;
+    return (size_t)stages * kGtspRows * npad * sizeof(double) + nck * threads * sizeof(double) + nwords * threads * sizeof(uint32_t) +
+           32 * sizeof(double) + 32 * sizeof(int) + kGtspMaxStages * sizeof(uint64_t) + 4 * sizeof(int);
+}
+
+// the largest city count whose shared memory fits one CTA (464)
+static int gtsp_max_cities()
+{
+    int n = 2;
+    while (n < 1024 && gtsp_smem(n + 1, kGtspStages) <= kGtspSmemMax) n++;
+    return n;
+}
+
 // readFromGraphFile :224-253 (matrix passed in memory) + init_param :187-218
 extern "C" int wr_gtsp_create(const double* dis, int n, int cnt, int batch, int colony_first, uint64_t seed, wr_gtsp** out)
 {
     WR_REQUIRE(dis && out && n >= 2 && batch >= 1 && colony_first >= 0, WR_ERR_INVALID, "wr_gtsp_create: bad argument");
-    WR_REQUIRE(n <= 512, WR_ERR_INVALID, "wr_gtsp_create: at most 512 cities (one ant per thread, check-points in shared memory)");
+    const int nmax = gtsp_max_cities();
+    if (n > nmax) {
+        set_error("wr_gtsp_create: at most %d cities (one ant per thread: its check-points and visited bits, with a %d-stage ring of "
+                  "matrix rows, must fit %zu B of shared memory; %d cities need %zu B)", nmax, kGtspStages, kGtspSmemMax, n, gtsp_smem(n, kGtspStages));
+        return WR_ERR_INVALID;
+    }
     WR_REQUIRE(colony_first + batch <= 65536, WR_ERR_INVALID, "wr_gtsp_create: colony ids must stay below 65536 (Philox stream tag)");
     *out = nullptr;
     wr_gtsp* g = new wr_gtsp();
@@ -309,9 +337,7 @@ extern "C" int wr_gtsp_create(const double* dis, int n, int cnt, int batch, int 
             hh[(size_t)i * npad + j] = host_power(1 / (d + 1e-8), 6);  // herustic :211, beta = 6 :191, power() :117-118
         }
     const size_t mat = (size_t)n * npad;
-    // TMA ring depth 3 (two CTAs per SM at N = 256) measured best: 2 -> 33.0k, 3 -> 34.7k, 4 -> 31.9k, 6 -> 21.3k colony-iterations/s
-    // at N = 256 x 1024 colonies (per-CTA latency wants more CTAs per SM, L2 capacity wants fewer resident matrices)
-    g->stages = 3;
+    g->stages = kGtspStages;
     g->mat_stride = mat;
 #define WR_CUDA_G(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { set_error("%s failed: %s", #expr, cudaGetErrorString(_e)); wr_gtsp_destroy(g); return WR_ERR_CUDA; } } while (0)
     WR_CUDA_G(cudaGetDevice(&g->device));
@@ -337,10 +363,7 @@ extern "C" int wr_gtsp_create(const double* dis, int n, int cnt, int batch, int 
         WR_CUDA_G(cudaMemcpy(g->d_best_start, bs.data(), batch * sizeof(int), cudaMemcpyHostToDevice));
     }
     g->threads = (n + 31) / 32 * 32;
-    const int nck = (n + kGtspIv - 1) / kGtspIv, nwords = (n + 31) / 32;
-    g->smem = (size_t)g->stages * kGtspRows * npad * sizeof(double) + (size_t)nck * g->threads * sizeof(double) +
-              (size_t)nwords * g->threads * sizeof(uint32_t) + 32 * sizeof(double) + 32 * sizeof(int) + kGtspMaxStages * sizeof(uint64_t) + 4 * sizeof(int);
-    if (g->smem > 227 * 1024) { set_error("wr_gtsp_create: %d cities need %zu B of shared memory", n, g->smem); wr_gtsp_destroy(g); return WR_ERR_INVALID; }
+    g->smem = gtsp_smem(n, g->stages);   // <= kGtspSmemMax: n <= gtsp_max_cities()
     WR_CUDA_G(cudaFuncSetAttribute(k_gtsp_iterate<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g->smem));
     WR_CUDA_G(cudaFuncSetAttribute(k_gtsp_iterate<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g->smem));
     WR_CUDA_G(cudaFuncSetAttribute(k_gtsp_iterate<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g->smem));

@@ -207,9 +207,9 @@ __global__ void __launch_bounds__(kRankSmallThreads) k_rank_chunks(const IterSta
     for (int i = threadIdx.x; i < nc; i += kRankSmallThreads) { ck[first + i] = kbuf[src][i]; cv[first + i] = (uint32_t)first + vbuf[src][i]; }
 }
 
-// One CTA per 1024 consecutive elements of one chunk.  The other chunks' keys are staged in shared memory 16 bits wide (a
-// key is a step count <= cap + 1 < 65536, or — K = 26 — compared through global memory), so the 12-step binary searches
-// run at shared-memory latency instead of one L2 round trip per step.
+// One CTA per 1024 consecutive elements of one chunk.  With keys16 the other chunks' keys are staged in shared memory 16 bits
+// wide (launch_rank sets it only for K = 6 step-count keys with cap + 1 <= 0xFFFF; K = 26 keys and larger caps are compared
+// through global memory), so the 12-step binary searches run at shared-memory latency instead of one L2 round trip per step.
 constexpr int kRankMergeThreads = 1024;
 __global__ void __launch_bounds__(kRankMergeThreads) k_rank_merge(const IterState* st, const uint32_t* __restrict__ ck, const uint32_t* __restrict__ cv,
                                                                    uint32_t* __restrict__ out_keys, uint32_t* __restrict__ out_vals, int* __restrict__ order_of_ant,
