@@ -129,8 +129,10 @@ int wr_acs_search_pairs(wr_acs* a, const int64_t* start_ids, const int64_t* goal
  * alone leaves the GPU idle.  Per-query pheromone lives in one hash table keyed by (query, node) (a node without an entry
  * is worth the scalar every never-deposited slot holds), the geometric factor is computed per step.  Results are
  * bit-identical to wr_acs_search_pairs on the same handle state (query q takes Philox search index next_search + q either
- * way).  Colonies above 4096 ants, K = 26, WR_UPDATE_ATOMIC and handles whose field is not in its initial / reset() state
- * run as the sequential loop; so does a chunk whose table fills up.  Same arguments as wr_acs_search_pairs. */
+ * way).  Both neighbourhoods batch; K = 26 entries hold the node's 26 slots, and a K = 26 batch never builds the dense
+ * N x 26 heuristic table (the factor is computed per step for each query's goal).  Colonies above 4096 ants,
+ * WR_UPDATE_ATOMIC and handles whose field is not in its initial / reset() state run as the sequential loop; so does a
+ * single query, and a chunk whose table or overflow pool fills up.  Same arguments as wr_acs_search_pairs. */
 int wr_acs_search_batch(wr_acs* a, const int64_t* start_ids, const int64_t* goal_ids, int nqueries, float predict_path_len,
                         int n_iterations, float* L, int* path_nodes, int64_t* path_ids, int* path_dirs, int path_cap);
 /* Result `index` of the last wr_acs_search_pairs / wr_acs_search_batch (kept in the handle, packed by true length — call

@@ -18,6 +18,7 @@
 #include "rank_small.cuh"
 #include "rankset.cuh"
 #include "batch.cuh"
+#include "batch26.cuh"
 #include "wr_internal.cuh"
 
 namespace wr {
@@ -1324,9 +1325,11 @@ struct wr_batch {   // buffers of the batch path, kept by the handle between cal
     uint32_t* best_ids = nullptr; uint8_t* best_dirs = nullptr;
     float* res_L = nullptr; int* res_n = nullptr;
     uint32_t* overflow_list = nullptr; unsigned long long* gtab = nullptr; int4* resume = nullptr;
+    uint32_t* gkeys = nullptr;   // K = 26: tile keys of the HBM visited tables (gtab holds their masks)
+    float* ant_L = nullptr;      // K = 26: [qc][cm] length of every ant
     unsigned long long* cnt_save = nullptr;
     uint32_t pool = 0;
-    int qc = 0, cm = 0;   // queries per chunk / colony the per-query buffers were sized for
+    int qc = 0, cm = 0, K = 6;   // queries per chunk / colony / neighbourhood the buffers were sized for
     bool mem_limited = false;   // qc is what fits into memory, not what was asked for
 };
 
@@ -1338,10 +1341,35 @@ static void free_batch(wr_acs* a)
     cudaStreamSynchronize(s);
     cudaFree(b->tab.ent); cudaFree(b->tab.list); cudaFree(b->tab.count);
     void* ptrs[] = {b->qs, b->d_starts, b->d_goals, b->steps, b->path_ids, b->path_dirs, b->ranked_keys, b->ranked_vals, b->best_ids, b->best_dirs, b->res_L, b->res_n,
-                    b->overflow_list, b->gtab, b->resume, b->cnt_save};
+                    b->overflow_list, b->gtab, b->resume, b->gkeys, b->ant_L, b->cnt_save};
     for (void* p : ptrs) cudaFree(p);
     delete b;
     a->batch = nullptr;
+}
+
+// the table kernels of a batch for its entries of EW words: kBatchEntryWords (K = 6) or kBatchEntryWords26 (K = 26)
+template <int EW>
+static void batch_table_fill(const wr_batch* b, cudaStream_t s) { k_batch_fill<EW><<<kNumSMs * 8, 256, 0, s>>>(reinterpret_cast<uint4*>(b->tab.ent), b->T); }
+static void launch_batch_fill(const wr_batch* b, cudaStream_t s)
+{
+    if (b->K == kK26) batch_table_fill<kBatchEntryWords26>(b, s);
+    else batch_table_fill<kBatchEntryWords>(b, s);
+}
+static void launch_batch_wipe(const wr_batch* b, cudaStream_t s)
+{
+    if (b->K == kK26) k_batch_wipe<kBatchEntryWords26><<<kNumSMs * 4, 256, 0, s>>>(b->tab);
+    else k_batch_wipe<kBatchEntryWords><<<kNumSMs * 4, 256, 0, s>>>(b->tab);
+}
+// ranking, evaporation and deposits of one iteration of every query of a chunk of n
+template <int EW>
+static void batch_rank_update(const wr_acs* a, const wr_batch* b, int n, int maxn, size_t rank_smem, cudaStream_t s)
+{
+    const int cm = b->cm;
+    k_batch_rank<EW><<<n, kRankSmallThreads, rank_smem, s>>>(a->d_state, b->qs, b->tab, b->steps, b->ant_L, cm, maxn, a->cap, a->rank_bits, a->d_Ltab, b->ranked_keys,
+                                                              b->ranked_vals, b->path_ids, b->path_dirs, b->best_ids, b->best_dirs);
+    k_batch_evaporate<EW><<<kNumSMs * 8, 256, 0, s>>>(b->tab, a->p.rho);
+    k_batch_deposit<EW><<<n, kBatchDepThreads, 0, s>>>(a->d_state, b->qs, b->tab, b->ranked_keys, b->ranked_vals, cm, b->path_ids, b->path_dirs, a->cap, a->d_Ltab,
+                                                       a->p.rho, b->steps);
 }
 
 static int batch_table_entries(int table_env_default)
@@ -1354,27 +1382,31 @@ static int batch_table_entries(int table_env_default)
 static int alloc_batch(wr_acs* a, int want_q, int cm, int* qc_out)
 {
     const size_t cap = a->cap;
-    if (a->batch && a->batch->cm == cm && (a->batch->qc >= want_q || a->batch->mem_limited)) { *qc_out = a->batch->qc; return WR_OK; }
+    const bool k26 = a->K == kK26;
+    if (a->batch && a->batch->cm == cm && a->batch->K == a->K && (a->batch->qc >= want_q || a->batch->mem_limited)) { *qc_out = a->batch->qc; return WR_OK; }
     free_batch(a);
     size_t free_b = 0, total_b = 0;
     WR_CUDA(cudaMemGetInfo(&free_b, &total_b));
     if (const char* e = getenv("WR_BATCH_MEM_MB")) free_b = std::min(free_b, (size_t)atoll(e) << 20);
-    const size_t per_q = (size_t)cm * cap * 5 + (size_t)cm * 10 + (cap + 1) * 5 + sizeof(BatchQuery) + 64;
+    const size_t per_q = (size_t)cm * cap * 5 + (size_t)cm * (k26 ? 14 : 10) + (cap + 1) * 5 + sizeof(BatchQuery) + 64;
     const size_t fit = std::min<size_t>(std::max<size_t>(1, (free_b / 2) / per_q), (size_t)1 << 16);
     const int qc = (int)std::min<size_t>((size_t)want_q, fit);
     wr_batch* b = new wr_batch();
     a->batch = b;
-    b->qc = qc; b->cm = cm; b->mem_limited = (size_t)want_q > fit;
-    // pheromone table: one for the whole chunk.  A quarter of the free memory at most, 2^17 entries (4 MB) per query at most
+    b->qc = qc; b->cm = cm; b->K = a->K; b->mem_limited = (size_t)want_q > fit;
+    // pheromone table: one for the whole chunk.  A quarter of the free memory at most, 2^17 entries (4 MB; K = 26: 16 MB) per
+    // query at most
+    const int ew = k26 ? kBatchEntryWords26 : kBatchEntryWords;
+    const size_t ebytes = (size_t)ew * sizeof(uint32_t);
     size_t T = (size_t)1 << 16;
-    while (T < (size_t)qc << 17 && T * 2 * 32 <= free_b / 4 && T < ((size_t)1 << 30)) T <<= 1;
+    while (T < (size_t)qc << 17 && T * 2 * ebytes <= free_b / 4 && T < ((size_t)1 << 30)) T <<= 1;
     if (const char* e = getenv("WR_BATCH_LOG2")) T = (size_t)1 << std::max(8, std::min(30, atoi(e)));
     b->T = T;
     b->tab.tmask = (uint32_t)(T - 1); b->tab.shift = 32 - ceil_log2(T); b->tab.limit = (uint32_t)(T / 2);
-    WR_CUDA(cudaMalloc(&b->tab.ent, T * 32));
+    WR_CUDA(cudaMalloc(&b->tab.ent, T * ebytes));
     WR_CUDA(cudaMalloc(&b->tab.list, (size_t)b->tab.limit * sizeof(uint32_t)));
     WR_CUDA(cudaMalloc(&b->tab.count, 4 * sizeof(uint32_t)));
-    k_batch_fill<<<kNumSMs * 8, 256, 0, a->stream>>>(reinterpret_cast<uint4*>(b->tab.ent), T);
+    launch_batch_fill(b, a->stream);
     WR_CUDA(cudaMemsetAsync(b->tab.count, 0, 4 * sizeof(uint32_t), a->stream));
     const size_t nq = qc;
     WR_CUDA(cudaMalloc(&b->qs, nq * sizeof(BatchQuery)));
@@ -1389,12 +1421,16 @@ static int alloc_batch(wr_acs* a, int want_q, int cm, int* qc_out)
     WR_CUDA(cudaMalloc(&b->best_dirs, nq * (cap + 1)));
     WR_CUDA(cudaMalloc(&b->res_L, nq * sizeof(float)));
     WR_CUDA(cudaMalloc(&b->res_n, nq * sizeof(int)));
-    // HBM visited tables for ants whose shared-memory table fills up: a pool (2 GB at most), handed out on demand
+    if (k26) WR_CUDA(cudaMalloc(&b->ant_L, nq * cm * sizeof(float)));
+    // HBM visited tables for ants whose shared-memory table fills up: a pool (2 GB at most), handed out on demand.  K = 6:
+    // k_walk_batch's 64-bit key|mask entries; K = 26: k_walk26's format, u32 tile keys + u64 masks
     const size_t Eg = (size_t)1 << a->gtable_log2_for_cap();
-    size_t pool = std::min<size_t>(nq * cm, std::max<size_t>(16, ((size_t)2 << 30) / (Eg * 8)));
+    const size_t gbytes = k26 ? 12 : 8;
+    size_t pool = std::min<size_t>(nq * cm, std::max<size_t>(16, ((size_t)2 << 30) / (Eg * gbytes)));
     b->pool = (uint32_t)pool;
     WR_CUDA(cudaMalloc(&b->overflow_list, pool * sizeof(uint32_t)));
     WR_CUDA(cudaMalloc(&b->gtab, pool * Eg * sizeof(unsigned long long)));
+    if (k26) WR_CUDA(cudaMalloc(&b->gkeys, pool * Eg * sizeof(uint32_t)));
     WR_CUDA(cudaMalloc(&b->resume, pool * sizeof(int4)));
     WR_CUDA(cudaMalloc(&b->cnt_save, 16 * sizeof(unsigned long long)));
     WR_CUDA(cudaGetLastError());
@@ -1417,36 +1453,46 @@ extern "C" int wr_acs_search_batch(wr_acs* a, const int64_t* start_ids, const in
     const int cm = a->p.fixed_colony > 0 ? a->p.fixed_colony : (int)(0.35 * (double)predict / (double)a->g->precision);   // :247 with best = inf
     WR_REQUIRE(cm >= 0 && cm < (1 << 24), WR_ERR_INVALID, "wr_acs_search_batch: colony size out of range");
     // What the batch path does not cover runs as the sequential loop (same results by definition): colonies that fill the
-    // GPU on their own, the K = 26 extension, the unordered atomic mode, a pheromone field that is not in its initial state
-    const bool batchable = cm >= 1 && cm <= kBatchMaxColony && a->K == 6 && a->p.update_mode != WR_UPDATE_ATOMIC && a->field_clean && nq > 1 && batch_enabled();
+    // GPU on their own, the unordered atomic mode, a pheromone field that is not in its initial state
+    const bool batchable = cm >= 1 && cm <= kBatchMaxColony && a->p.update_mode != WR_UPDATE_ATOMIC && a->field_clean && nq > 1 && batch_enabled();
+    const bool k26 = a->K == kK26;
     const uint32_t first_search = a->next_search;
     if (!batchable) {
         rc = run_pairs_sequential(a, start_ids, goal_ids, 0, nq, predict, n_iterations);
         if (rc == WR_OK) export_results(a, nq, L, path_nodes, path_ids, path_dirs, path_cap);
         return rc;
     }
-    rc = grid_ensure_open6(a->g, s);
-    if (rc != WR_OK) return rc;
+    if (!k26) {
+        rc = grid_ensure_open6(a->g, s);
+        if (rc != WR_OK) return rc;
+    }
     int qc = 0;
     rc = alloc_batch(a, nq, cm, &qc);
     if (rc != WR_OK) return rc;
     wr_batch* b = a->batch;
     const int entries = batch_table_entries(320);   // 42 KB per CTA: five CTAs per SM, like the register bound (C5: 256 -> 1898, 320 -> 2095, 384 -> 1989, 512 -> 1636 queries/s)
-    const size_t smem1 = kWalk2Lut + 128 + (size_t)kAntsPerCta * entries * sizeof(unsigned long long);
+    // K = 26: four ants per CTA, each with k_walk26's shared-memory visited table of 1 << walk_table_log2 entries (12 B each)
+    const size_t smem1 = k26 ? ((size_t)kWalk26Ants << a->table_log2) * 12 : kWalk2Lut + 128 + (size_t)kAntsPerCta * entries * sizeof(unsigned long long);
     WR_REQUIRE(smem1 <= 227 * 1024, WR_ERR_INVALID, "wr_acs_search_batch: WR_BATCH_TABLE too large");
     const bool alpha1 = a->p.alpha == 1;
     const int maxn = (std::max(cm, 32) + 31) / 32 * 32;
     const size_t rank_smem = (size_t)12 * maxn + 32 * 256 * sizeof(uint32_t);
-    WR_CUDA(cudaFuncSetAttribute(k_walk_batch3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-    WR_CUDA(cudaFuncSetAttribute(k_walk_batch3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-    WR_CUDA(cudaFuncSetAttribute(k_batch_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rank_smem));
+    if (k26) {
+        WR_CUDA(cudaFuncSetAttribute(k_walk_batch26<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+    } else {
+        WR_CUDA(cudaFuncSetAttribute(k_walk_batch3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+        WR_CUDA(cudaFuncSetAttribute(k_walk_batch3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+    }
+    if (k26) WR_CUDA(cudaFuncSetAttribute(k_batch_rank<kBatchEntryWords26>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rank_smem));
+    else WR_CUDA(cudaFuncSetAttribute(k_batch_rank<kBatchEntryWords>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rank_smem));
     const int per_sm = std::max(1, std::min(16, (int)((227 * 1024) / (smem1 + 1024))));
     BatchArgs w;
-    w.st = a->d_state; w.qs = b->qs; w.colony_max = cm; w.items_per_query = (cm + 3) / 4;
-    w.tab = b->tab; w.open6 = a->g->d_open6; w.coords = a->g->d_coords; w.rx = a->g->rx; w.ry = a->g->ry; w.rz = a->g->rz;
+    w.st = a->d_state; w.qs = b->qs; w.colony_max = cm; w.items_per_query = k26 ? cm : (cm + 3) / 4;   // K = 26: one ant per work item
+    w.tab = b->tab; w.open6 = a->g->d_open6; w.occ = a->g->d_bits; w.coords = a->g->d_coords; w.rx = a->g->rx; w.ry = a->g->ry; w.rz = a->g->rz;
     w.seed_lo = (uint32_t)a->p.seed; w.seed_hi = (uint32_t)(a->p.seed >> 32); w.alpha = a->p.alpha; w.beta = a->p.beta; w.cap = a->cap;
     w.ant_steps = b->steps; w.path_ids = b->path_ids; w.path_dirs = b->path_dirs; w.table_entries = entries;
     w.overflow_list = b->overflow_list; w.gtab = b->gtab; w.gtable_log2 = a->gtable_log2_for_cap(); w.resume = b->resume; w.pool = b->pool;
+    w.table_log2 = a->table_log2; w.gkeys = b->gkeys; w.precision = a->g->precision; w.ant_L = b->ant_L;
     for (int c0 = 0; c0 < nq && rc == WR_OK; c0 += qc) {
         const int n = std::min(qc, nq - c0);
         w.nq = n;
@@ -1460,32 +1506,34 @@ extern "C" int wr_acs_search_batch(wr_acs* a, const int64_t* start_ids, const in
         WR_CUDA(cudaMemcpyAsync(b->cnt_save, d_cnt, sizeof(unsigned long long) * 9, cudaMemcpyDeviceToDevice, s));
         k_batch_begin<<<(n + 255) / 256, 256, 0, s>>>(a->d_state, b->qs, n, b->d_starts, b->d_goals, first_search + (uint32_t)c0, predict, a->p.tau0, b->tab.count);
         const int items = n * w.items_per_query;
-        const int blocks1 = std::max(1, std::min((items + 3) / 4, kNumSMs * per_sm));
-        const int blocks2 = std::max(1, std::min((int)((b->pool + kAntsPerCta - 1) / kAntsPerCta), kNumSMs * 4));
+        const int blocks1 = std::max(1, std::min((items + 3) / 4, kNumSMs * per_sm));   // four work items per CTA for either K
+        const int pass2_ants = k26 ? kWalk26Ants : kAntsPerCta;
+        const int blocks2 = std::max(1, std::min((int)((b->pool + pass2_ants - 1) / pass2_ants), kNumSMs * 4));
         for (int it = 0; it < n_iterations; it++) {
             k_batch_iter_begin<<<(n + 255) / 256, 256, 0, s>>>(a->d_state, b->qs, n, a->p.fixed_colony, cm, a->g->precision, a->p.tau0, it > 0 ? 1 : 0, a->p.rho);
-            if (alpha1) {
+            if (k26) {
+                k_walk_batch26<false><<<blocks1, kWalk26Threads, smem1, s>>>(w);
+                k_walk_batch26<true><<<blocks2, kWalk26Threads, 0, s>>>(w);
+            } else if (alpha1) {
                 k_walk_batch3<true><<<blocks1, kWalkThreads, smem1, s>>>(w);
                 k_walk_batch<true><<<blocks2, kWalkThreads, kWalk2Lut, s>>>(w);
             } else {
                 k_walk_batch3<false><<<blocks1, kWalkThreads, smem1, s>>>(w);
                 k_walk_batch<false><<<blocks2, kWalkThreads, kWalk2Lut, s>>>(w);
             }
-            k_batch_rank<<<n, kRankSmallThreads, rank_smem, s>>>(a->d_state, b->qs, b->tab, b->steps, cm, maxn, a->cap, a->rank_bits, a->d_Ltab, b->ranked_keys, b->ranked_vals,
-                                                                  b->path_ids, b->path_dirs, b->best_ids, b->best_dirs);
-            k_batch_evaporate<<<kNumSMs * 8, 256, 0, s>>>(b->tab, a->p.rho);
-            k_batch_deposit<<<n, kBatchDepThreads, 0, s>>>(a->d_state, b->qs, b->tab, b->ranked_keys, b->ranked_vals, cm, b->path_ids, b->path_dirs, a->cap, a->d_Ltab, a->p.rho);
+            if (k26) batch_rank_update<kBatchEntryWords26>(a, b, n, maxn, rank_smem, s);
+            else batch_rank_update<kBatchEntryWords>(a, b, n, maxn, rank_smem, s);
         }
         k_batch_results<<<(n + 255) / 256, 256, 0, s>>>(b->qs, n, b->res_L, b->res_n);
         WR_CUDA(cudaGetLastError());
         uint32_t cnt[4] = {0, 0, 0, 0};
         WR_CUDA(cudaMemcpyAsync(cnt, b->tab.count, sizeof cnt, cudaMemcpyDeviceToHost, s));
         WR_CUDA(cudaStreamSynchronize(s));
-        k_batch_wipe<<<kNumSMs * 4, 256, 0, s>>>(b->tab);
+        launch_batch_wipe(b, s);
         a->batch_last_entries = cnt[0];
         if (cnt[1]) {   // pheromone table or overflow-table pool exhausted: this chunk's searches run one after the other instead
             a->batch_fallbacks++;
-            k_batch_fill<<<kNumSMs * 8, 256, 0, s>>>(reinterpret_cast<uint4*>(b->tab.ent), b->T);   // entries claimed beyond the list
+            launch_batch_fill(b, s);   // entries claimed beyond the list
             WR_CUDA(cudaMemcpyAsync(d_cnt, b->cnt_save, sizeof(unsigned long long) * 9, cudaMemcpyDeviceToDevice, s));
             k_set_base<<<1, 1, 0, s>>>(a->d_state, a->p.tau0);   // the batch advanced the handle's scalar; the dense field itself is untouched
             a->next_search = first_search + (uint32_t)c0;

@@ -21,6 +21,8 @@
 //                        are small (<= 4096 ants), the parallelism comes from the number of queries.
 // Every query draws from its own Philox search index (wr_common.cuh), so a batch equals the same searches run one after
 // the other through wr_acs_search_pairs bit for bit — and those equal the oracle's.
+// K = 26 (batch26.cuh) shares the table code — templated on the entry's words EW, so the K = 6 kernels keep a constant
+// stride — with a 128-byte entry, ranking by the bits of L and deposits with the ant's own L; only the walk is its own kernel.
 #pragma once
 #include "rank_small.cuh"
 #include "walk2.cuh"
@@ -29,7 +31,8 @@
 namespace wr {
 
 constexpr int kBatchMaxColony = 4096;       // larger colonies fill the GPU on their own: wr_acs_search_pairs
-constexpr int kBatchEntryWords = 8;         // key (2 words: node+1 | query << 32 | on-best << 63), tau[6]
+constexpr int kBatchEntryWords = 8;         // K = 6: key (2 words: node+1 | query << 32 | on-best << 63), tau[6]
+constexpr int kBatchEntryWords26 = 32;      // K = 26: the same key, tau[26] in the slot26 enumeration, 4 unused words (one 128 B line)
 constexpr unsigned long long kBatchFlagBit = 1ull << 63;
 
 struct BatchQuery {   // device-side state of one query (the part of IterState that differs between queries)
@@ -46,7 +49,7 @@ struct BatchQuery {   // device-side state of one query (the part of IterState t
 };
 
 struct BatchTable {
-    uint32_t* ent;       // [T][8]
+    uint32_t* ent;       // [T][EW]: kBatchEntryWords (K = 6) or kBatchEntryWords26 words per entry
     uint32_t* list;      // [limit] entries claimed since the batch began
     uint32_t* count;     // [0] claimed entries [1] failure flag (table or overflow-table pool exhausted: the batch is re-run) [2] pool tables in use
     uint32_t tmask;
@@ -57,12 +60,13 @@ struct BatchTable {
 __device__ __forceinline__ uint32_t batch_hash(uint32_t node, uint32_t q) { return (node * 2654435761u) ^ (q * 0x85EBCA6Bu + (q << 13)); }
 
 // entry of (query, node), or 0xFFFFFFFF if it has none
+template <int EW>
 __device__ __forceinline__ uint32_t batch_find(const BatchTable& t, uint32_t node, uint32_t q)
 {
     const unsigned long long want = (unsigned long long)(node + 1u) | ((unsigned long long)q << 32);
     uint32_t h = batch_hash(node, q) >> t.shift;
     for (uint32_t probes = 0; probes <= t.tmask; probes++) {   // bounded: a failing batch (claims raced past the limit) may have filled a tiny table
-        const unsigned long long k = *reinterpret_cast<const volatile unsigned long long*>(t.ent + (size_t)h * kBatchEntryWords);
+        const unsigned long long k = *reinterpret_cast<const volatile unsigned long long*>(t.ent + (size_t)h * EW);
         if ((k & ~kBatchFlagBit) == want) return h;
         if (k == 0ull) return 0xFFFFFFFFu;
         h = (h + 1) & t.tmask;
@@ -70,14 +74,15 @@ __device__ __forceinline__ uint32_t batch_find(const BatchTable& t, uint32_t nod
     return 0xFFFFFFFFu;
 }
 
-// ... created if missing (its six slots hold the sentinel: the table is filled with sentinels, keys zero)
+// ... created if missing (its slots hold the sentinel: the table is filled with sentinels, keys zero)
+template <int EW>
 __device__ __forceinline__ uint32_t batch_find_or_insert(const BatchTable& t, uint32_t node, uint32_t q)
 {
     const unsigned long long want = (unsigned long long)(node + 1u) | ((unsigned long long)q << 32);
     uint32_t h = batch_hash(node, q) >> t.shift;
     volatile uint32_t* fail = t.count + 1;
     for (uint32_t probes = 0; probes <= t.tmask; probes++) {
-        unsigned long long* kp = reinterpret_cast<unsigned long long*>(t.ent + (size_t)h * kBatchEntryWords);
+        unsigned long long* kp = reinterpret_cast<unsigned long long*>(t.ent + (size_t)h * EW);
         unsigned long long k = *reinterpret_cast<volatile unsigned long long*>(kp);
         if (k == 0ull) {
             if (*fail) return 0xFFFFFFFFu;
@@ -100,7 +105,8 @@ struct BatchArgs {
     BatchQuery* qs;
     int nq, colony_max, items_per_query;
     BatchTable tab;
-    const uint8_t* open6;     // per node: bit k <=> neighbour k in bounds and free
+    const uint8_t* open6;     // per node: bit k <=> neighbour k in bounds and free (K = 6)
+    const uint32_t* occ;      // K = 26: the grid's occupancy, one bit per node, 1 = occupied
     const float* coords;      // xs | ys | zs
     int rx, ry, rz;
     uint32_t seed_lo, seed_hi;
@@ -112,25 +118,38 @@ struct BatchArgs {
     uint8_t* path_dirs;
     int table_entries;        // shared-memory visited-tile entries per ant (pass 1)
     uint32_t* overflow_list;  // [pool] (query * colony_max + ant) of the parked ants
-    unsigned long long* gtab; // [pool][1 << gtable_log2] HBM visited tables
+    unsigned long long* gtab; // [pool][1 << gtable_log2] HBM visited tables (K = 26: their masks)
     int gtable_log2;
     int4* resume;             // [pool]
     uint32_t pool;
+    // K = 26 (batch26.cuh)
+    int table_log2;           // shared-memory visited-tile table of an ant: 1 << table_log2 entries (pass 1)
+    uint32_t* gkeys;          // [pool][1 << gtable_log2] tile keys of the HBM visited tables (masks in gtab)
+    float precision;          // step lengths precision, precision*1.414f, precision*1.732f
+    float* ant_L;             // [nq][colony_max] length of every ant, +inf if it died
 };
 
+template <int EW>
 __global__ void k_batch_fill(uint4* __restrict__ ent4, size_t n_entries)
-{   // keys 0, every slot the sentinel
+{   // keys 0, every slot (and the unused words of a K = 26 entry) the sentinel
     const uint4 a = make_uint4(0u, 0u, kSentinelBits, kSentinelBits), b = make_uint4(kSentinelBits, kSentinelBits, kSentinelBits, kSentinelBits);
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_entries; i += (size_t)gridDim.x * blockDim.x) { ent4[2 * i] = a; ent4[2 * i + 1] = b; }
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_entries; i += (size_t)gridDim.x * blockDim.x) {
+        ent4[EW / 4 * i] = a;
+#pragma unroll
+        for (int j = 1; j < EW / 4; j++) ent4[EW / 4 * i + j] = b;
+    }
 }
 // after a batch: only the claimed entries need restoring
+template <int EW>
 __global__ void k_batch_wipe(BatchTable t)
 {
     const uint32_t n = min(t.count[0], t.limit);
     const uint4 a = make_uint4(0u, 0u, kSentinelBits, kSentinelBits), b = make_uint4(kSentinelBits, kSentinelBits, kSentinelBits, kSentinelBits);
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        uint4* e = reinterpret_cast<uint4*>(t.ent + (size_t)t.list[i] * kBatchEntryWords);
-        e[0] = a; e[1] = b;
+        uint4* e = reinterpret_cast<uint4*>(t.ent + (size_t)t.list[i] * EW);
+        e[0] = a;
+#pragma unroll
+        for (int j = 1; j < EW / 4; j++) e[j] = b;
     }
 }
 
@@ -676,7 +695,11 @@ __global__ void __launch_bounds__(kWalkThreads, 5) k_walk_batch3(BatchArgs a)
 // Ranking, best decision and best path of every query: one CTA per query.
 // dynamic shared memory: keys[2][maxn] (u32) + vals[2][maxn] (u16) + whist[32][256] (u32)
 // ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kRankSmallThreads) k_batch_rank(IterState* st, BatchQuery* qs, BatchTable tab, const int* __restrict__ ant_steps, int colony_max, int maxn,
+// EW = kBatchEntryWords26 (K = 26): keys are the bits of each query's ant_L row, as k_rank_small's K = 26 branch (ant_L is
+// unused for K = 6).
+template <int EW>
+__global__ void __launch_bounds__(kRankSmallThreads) k_batch_rank(IterState* st, BatchQuery* qs, BatchTable tab, const int* __restrict__ ant_steps,
+                                                                   const float* __restrict__ ant_L, int colony_max, int maxn,
                                                                    int cap, int key_bits, const float* __restrict__ Ltab, uint32_t* __restrict__ ranked_keys,
                                                                    uint16_t* __restrict__ ranked_vals, const uint32_t* __restrict__ path_ids,
                                                                    const uint8_t* __restrict__ path_dirs, uint32_t* __restrict__ best_ids, uint8_t* __restrict__ best_dirs)
@@ -692,13 +715,20 @@ __global__ void __launch_bounds__(kRankSmallThreads) k_batch_rank(IterState* st,
     BatchQuery& b = qs[q];
     const int n = b.colony;
     const int* steps_q = ant_steps + (size_t)q * colony_max;
-    const int src = rank_sort_chunk(kbuf, vbuf, whist, warp_sum, steps_q, nullptr, 0, n, cap, key_bits);
+    const float* L_q = EW == kBatchEntryWords26 ? ant_L + (size_t)q * colony_max : nullptr;
+    const int src = rank_sort_chunk(kbuf, vbuf, whist, warp_sum, steps_q, L_q, 0, n, cap, key_bits);
     const uint32_t* keys = kbuf[src];
     const uint16_t* vals = vbuf[src];
     const float lambda = b.lambda;
     if (threadIdx.x == 0) {
         s_elig = 0; s_changed = 0; s_old_n = b.best_n;
-        if (n > 0) {
+        if (n > 0 && L_q) {
+            const float L0 = __uint_as_float(keys[0]);
+            if (L0 < b.best_L) {   // agentK.L < best.L  (:263) on the float lengths
+                b.best_steps = steps_q[vals[0]]; b.best_L = L0; b.best_changed = 1; b.best_ant = (int)vals[0];
+                s_changed = 1;
+            }
+        } else if (n > 0) {
             const int s = (int)keys[0];
             if (s <= cap && s < b.best_steps) {   // agentK.L < best.L  (:263); ties keep the earlier best, the first of equal ants wins
                 b.best_steps = s; b.best_L = Ltab[s]; b.best_changed = 1; b.best_ant = (int)vals[0];
@@ -712,24 +742,25 @@ __global__ void __launch_bounds__(kRankSmallThreads) k_batch_rank(IterState* st,
         const uint32_t key = keys[r];
         ranked_keys[(size_t)q * colony_max + r] = key;
         ranked_vals[(size_t)q * colony_max + r] = vals[r];
-        local += ((int)key <= cap && !((float)(r + 1) > __fsub_rn(lambda, 1.0f))) ? 1 : 0;   // :200
+        const bool arrived = L_q ? key != 0x7F800000u : (int)key <= cap;
+        local += (arrived && !((float)(r + 1) > __fsub_rn(lambda, 1.0f))) ? 1 : 0;   // :200
     }
     if (local) atomicAdd(&s_elig, local);
     __syncthreads();
     if (threadIdx.x == 0) {
         b.n_eligible = s_elig;
         unsigned long long recs = 0;
-        for (int r = 0; r < s_elig; r++) recs += keys[r];   // eligible ranks are a prefix of the sorted colony
+        for (int r = 0; r < s_elig; r++) recs += L_q ? (unsigned long long)steps_q[vals[r]] : keys[r];   // eligible ranks are a prefix of the sorted colony
         atomicAdd(&st->cnt[7], recs);
     }
     if (!s_changed) return;   // CTA-uniform
     // best = agentK (:264): the old path's nodes lose their membership flag, the new path's get it (entries are created for
-    // nodes that have none: their six slots stay sentinels, i.e. worth the scalar)
+    // nodes that have none: their slots stay sentinels, i.e. worth the scalar)
     uint32_t* bi = best_ids + (size_t)q * (cap + 1);
     uint8_t* bd = best_dirs + (size_t)q * (cap + 1);
     for (int i = threadIdx.x; i < s_old_n; i += kRankSmallThreads) {
-        const uint32_t h = batch_find(tab, bi[i], q);
-        if (h != 0xFFFFFFFFu) atomicAnd(reinterpret_cast<unsigned long long*>(tab.ent + (size_t)h * kBatchEntryWords), ~kBatchFlagBit);
+        const uint32_t h = batch_find<EW>(tab, bi[i], q);
+        if (h != 0xFFFFFFFFu) atomicAnd(reinterpret_cast<unsigned long long*>(tab.ent + (size_t)h * EW), ~kBatchFlagBit);
     }
     __syncthreads();
     const int steps = b.best_steps;
@@ -738,32 +769,40 @@ __global__ void __launch_bounds__(kRankSmallThreads) k_batch_rank(IterState* st,
         const uint32_t id = i < steps ? path_ids[off + i] : (uint32_t)b.goal;
         bi[i] = id;
         if (i < steps) bd[i] = path_dirs[off + i];
-        const uint32_t h = batch_find_or_insert(tab, id, q);
-        if (h != 0xFFFFFFFFu) atomicOr(reinterpret_cast<unsigned long long*>(tab.ent + (size_t)h * kBatchEntryWords), kBatchFlagBit);
+        const uint32_t h = batch_find_or_insert<EW>(tab, id, q);
+        if (h != 0xFFFFFFFFu) atomicOr(reinterpret_cast<unsigned long long*>(tab.ent + (size_t)h * EW), kBatchFlagBit);
     }
     if (threadIdx.x == 0) b.best_n = steps + 1;
 }
 
+template <int EW>
 __global__ void __launch_bounds__(256) k_batch_evaporate(BatchTable t, float rho)
 {   // :268-272 for every slot that ever received a deposit (sentinels are -0: unchanged by the product)
     const uint32_t n = min(t.count[0], t.limit);
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        uint32_t* e = t.ent + (size_t)t.list[i] * kBatchEntryWords;
+        uint32_t* e = t.ent + (size_t)t.list[i] * EW;
+        constexpr int end = EW == kBatchEntryWords26 ? 2 + 26 : 2 + 6;   // slots are words [2, end): two, then groups of four
         float2 a = *reinterpret_cast<float2*>(e + 2);
-        float4 b = *reinterpret_cast<float4*>(e + 4);
         a.x = __fmul_rn(a.x, rho); a.y = __fmul_rn(a.y, rho);
-        b.x = __fmul_rn(b.x, rho); b.y = __fmul_rn(b.y, rho); b.z = __fmul_rn(b.z, rho); b.w = __fmul_rn(b.w, rho);
         *reinterpret_cast<float2*>(e + 2) = a;
-        *reinterpret_cast<float4*>(e + 4) = b;
+#pragma unroll
+        for (int j = 4; j < end; j += 4) {
+            float4 b = *reinterpret_cast<float4*>(e + j);
+            b.x = __fmul_rn(b.x, rho); b.y = __fmul_rn(b.y, rho); b.z = __fmul_rn(b.z, rho); b.w = __fmul_rn(b.w, rho);
+            *reinterpret_cast<float4*>(e + j) = b;
+        }
     }
 }
 
 // update_pheromone (:198-215) of every query; value = (lambda - order)*Q/L_ant + float(onBest)*lambda*Q/L_best (:210-211)
+// EW = kBatchEntryWords26 (K = 26): ranked_keys hold the bits of the ant's L, its step count is steps26[query][ant] (unused
+// for K = 6)
 constexpr int kBatchDepThreads = 256;
+template <int EW>
 __global__ void __launch_bounds__(kBatchDepThreads) k_batch_deposit(const IterState* st, const BatchQuery* __restrict__ qs, BatchTable tab,
                                                                      const uint32_t* __restrict__ ranked_keys, const uint16_t* __restrict__ ranked_vals, int colony_max,
                                                                      const uint32_t* __restrict__ path_ids, const uint8_t* __restrict__ path_dirs, int cap,
-                                                                     const float* __restrict__ Ltab, float rho)
+                                                                     const float* __restrict__ Ltab, float rho, const int* __restrict__ steps26 = nullptr)
 {
     __shared__ uint8_t s_flag[kBatchDepThreads + 1];
     const uint32_t q = blockIdx.x;
@@ -776,8 +815,11 @@ __global__ void __launch_bounds__(kBatchDepThreads) k_batch_deposit(const IterSt
     const uint32_t goal = (uint32_t)b.goal;
     for (int r = 0; r < n; r++) {
         const int ant = (int)ranked_vals[(size_t)q * colony_max + r];
-        const int steps = (int)ranked_keys[(size_t)q * colony_max + r];
-        const float base = __fdiv_rn(__fmul_rn(__fsub_rn(lambda, (float)(r + 1)), Q), Ltab[steps]);
+        const uint32_t key = ranked_keys[(size_t)q * colony_max + r];
+        constexpr bool k26 = EW == kBatchEntryWords26;
+        const int steps = k26 ? steps26[(size_t)q * colony_max + ant] : (int)key;
+        const float L_ant = k26 ? __uint_as_float(key) : Ltab[steps];
+        const float base = __fdiv_rn(__fmul_rn(__fsub_rn(lambda, (float)(r + 1)), Q), L_ant);
         const float with_elite = __fadd_rn(base, elite), without = __fadd_rn(base, 0.0f);
         const size_t off = ((size_t)q * colony_max + (size_t)ant) * cap;
         for (int i0 = 0; i0 < steps; i0 += kBatchDepThreads) {   // CTA-uniform trips
@@ -785,16 +827,16 @@ __global__ void __launch_bounds__(kBatchDepThreads) k_batch_deposit(const IterSt
             uint32_t h = 0xFFFFFFFFu;
             bool f = false;
             if (i < steps) {
-                h = batch_find_or_insert(tab, path_ids[off + i], q);
-                if (h != 0xFFFFFFFFu) f = (tab.ent[(size_t)h * kBatchEntryWords + 1] >> 31) != 0u;
+                h = batch_find_or_insert<EW>(tab, path_ids[off + i], q);
+                if (h != 0xFFFFFFFFu) f = (tab.ent[(size_t)h * EW + 1] >> 31) != 0u;
             }
             s_flag[threadIdx.x] = f ? 1 : 0;
             if (threadIdx.x == 0) {   // membership of the node that follows this trip's last step
                 const int j = i0 + kBatchDepThreads;
                 bool fn = false;
                 if (j <= steps) {
-                    const uint32_t hn = batch_find(tab, j < steps ? path_ids[off + j] : goal, q);
-                    fn = hn != 0xFFFFFFFFu && (tab.ent[(size_t)hn * kBatchEntryWords + 1] >> 31) != 0u;
+                    const uint32_t hn = batch_find<EW>(tab, j < steps ? path_ids[off + j] : goal, q);
+                    fn = hn != 0xFFFFFFFFu && (tab.ent[(size_t)hn * EW + 1] >> 31) != 0u;
                 }
                 s_flag[kBatchDepThreads] = fn ? 1 : 0;
             }
@@ -804,10 +846,10 @@ __global__ void __launch_bounds__(kBatchDepThreads) k_batch_deposit(const IterSt
                 if (i + 1 < i0 + kBatchDepThreads && i + 1 < steps) next_on = s_flag[threadIdx.x + 1] != 0;
                 else if (i + 1 == i0 + kBatchDepThreads) next_on = s_flag[kBatchDepThreads] != 0;
                 else {   // i + 1 == steps: the goal
-                    const uint32_t hn = batch_find(tab, goal, q);
-                    next_on = hn != 0xFFFFFFFFu && (tab.ent[(size_t)hn * kBatchEntryWords + 1] >> 31) != 0u;
+                    const uint32_t hn = batch_find<EW>(tab, goal, q);
+                    next_on = hn != 0xFFFFFFFFu && (tab.ent[(size_t)hn * EW + 1] >> 31) != 0u;
                 }
-                float* slot = reinterpret_cast<float*>(tab.ent + (size_t)h * kBatchEntryWords + 2) + path_dirs[off + i];
+                float* slot = reinterpret_cast<float*>(tab.ent + (size_t)h * EW + 2) + path_dirs[off + i];   // direction 0..5 or 0..25
                 *slot = __fadd_rn(tau_or_base(*slot, base_new), (f && next_on) ? with_elite : without);
             }
             __syncthreads();   // the next ant (or trip) may touch the same node's entry

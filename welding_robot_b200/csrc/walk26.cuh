@@ -47,6 +47,19 @@ __global__ void __launch_bounds__(256) k_tau_init26(float* tau, int rx, int ry, 
 
 // selectNext :137, :151-154 with a general vector_b (up to three non-zero components): the reference's expressions,
 // left to right, no contraction: norm = sqrt((x*x + y*y) + z*z) (model_grid_map.hpp:51-54), dot = (ax*bx + ay*by) + az*bz.
+// c*: coordinates of the node, g*: of the goal, n*: of the neighbour.  k_heuristic26 tabulates it, k_walk_batch26 (batch26.cuh)
+// evaluates it per step: one function, so the two cannot drift apart.
+__device__ __forceinline__ float heur26(float cx, float cy, float cz, float gx, float gy, float gz, float nx, float ny, float nz, float beta)
+{
+    const float ax = __fsub_rn(gx, cx), ay = __fsub_rn(gy, cy), az = __fsub_rn(gz, cz);
+    const float bx = __fsub_rn(nx, cx), by = __fsub_rn(ny, cy), bz = __fsub_rn(nz, cz);
+    const float na = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay)), __fmul_rn(az, az)));
+    const float nb = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by)), __fmul_rn(bz, bz)));
+    const float dot = __fadd_rn(__fadd_rn(__fmul_rn(ax, bx), __fmul_rn(ay, by)), __fmul_rn(az, bz));
+    const float cosv = __fdiv_rn(dot, __fmul_rn(na, nb));
+    return __fadd_rn(1.0f, __fmul_rn(beta, cosv));
+}
+
 __global__ void __launch_bounds__(256) k_heuristic26(float* __restrict__ heur, const float* __restrict__ coords, const uint32_t* __restrict__ occ_bits,
                                                       int rx, int ry, int rz, unsigned long long N, int goal, float beta)
 {
@@ -67,16 +80,7 @@ __global__ void __launch_bounds__(256) k_heuristic26(float* __restrict__ heur, c
     float v = kClosedSlot;
     if (inb) {
         const unsigned long long nid = ((unsigned long long)nz * ry + ny) * rx + nx;
-        if (!((occ_bits[nid >> 5] >> (nid & 31)) & 1u)) {
-            const float cx = xs[x], cy = ys[y], cz = zs[z];
-            const float ax = __fsub_rn(xs[gx], cx), ay = __fsub_rn(ys[gy], cy), az = __fsub_rn(zs[gz], cz);
-            const float bx = __fsub_rn(xs[nx], cx), by = __fsub_rn(ys[ny], cy), bz = __fsub_rn(zs[nz], cz);
-            const float na = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay)), __fmul_rn(az, az)));
-            const float nb = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by)), __fmul_rn(bz, bz)));
-            const float dot = __fadd_rn(__fadd_rn(__fmul_rn(ax, bx), __fmul_rn(ay, by)), __fmul_rn(az, bz));
-            const float cosv = __fdiv_rn(dot, __fmul_rn(na, nb));
-            v = __fadd_rn(1.0f, __fmul_rn(beta, cosv));
-        }
+        if (!((occ_bits[nid >> 5] >> (nid & 31)) & 1u)) v = heur26(xs[x], ys[y], zs[z], xs[gx], ys[gy], zs[gz], xs[nx], ys[ny], zs[nz], beta);
     }
     heur[idx] = v;
 }
