@@ -27,6 +27,7 @@
 #include <fstream>
 #include <functional>
 #include <iostream>
+#include <memory>
 #include <set>
 #include <stdexcept>
 #include <type_traits>
@@ -568,6 +569,7 @@ class ACS_GTSP {
 public:
     std::vector<float> g_path_x, g_path_y, g_path_z;
     uint64_t seed = 0;   // addition
+    int colonies = 1;    // addition: colonies setDistanceMatrix creates; computeSolution keeps the best one's tour
 
     ~ACS_GTSP() { if (g_) wr_gtsp_destroy(g_); }
 
@@ -593,23 +595,24 @@ public:
         if (g_) wr_gtsp_destroy(g_);
         g_ = nullptr;
         city_num = n;
-        wr::check(wr_gtsp_create(dis.data(), n, cnt, 1, 0, seed, &g_));
+        wr::check(wr_gtsp_create(dis.data(), n, cnt, colonies, 0, seed, &g_));
+        batch_ = colonies;
         init_flag = true;
         best_L = 0x3f3f3f3f;
         return true;
     }
     bool computeSolution()
-    {   // :255-284
+    {   // :255-284, every colony on the device with its own stopping rule
         if (!init_flag) return false;
-        double last = 0x3f3f3f3f;
-        int bad_times = 0;
-        for (int index_itera = 0; index_itera < city_num * city_num; index_itera++) {
-            if (bad_times > city_num) break;
-            wr::check(wr_gtsp_iterate(g_, 1));
-            fetch();
-            printf("iteration %d:Best so far = %.2lf\n", index_itera, best_L);
-            if (last > best_L) { last = best_L; bad_times = 0; } else bad_times++;
-        }
+        const int cap = city_num * city_num;
+        std::vector<int> ran(batch_);
+        // left uninitialised: only the pages up to each colony's iteration count are ever touched
+        std::unique_ptr<double[]> hist(new double[(size_t)batch_ * cap]);
+        int b = 0;
+        wr::check(wr_gtsp_solve(g_, cap, ran.data(), hist.get(), &b));
+        for (int index_itera = 0; index_itera < ran[b]; index_itera++)
+            printf("iteration %d:Best so far = %.2lf\n", index_itera, hist[(size_t)b * cap + index_itera]);
+        fetch(b);
         printf("Best in all = %.2lf\n", best_L);
         for (size_t i = 0; i < best_path.size(); i++) printf("%d->", best_path[i].first + 1);
         if (!best_path.empty()) printf("%d\n", best_path.back().second + 1);
@@ -636,14 +639,15 @@ public:
 private:
     wr_gtsp* g_ = nullptr;
     int city_num = 0;
+    int batch_ = 0;
     bool init_flag = false;
     std::vector<std::pair<int, int>> best_path;
     double best_L = 0x3f3f3f3f;
-    void fetch()
+    void fetch(int colony)
     {
         std::vector<int> t((size_t)2 * city_num);
         int ne = 0;
-        wr::check(wr_gtsp_best(g_, 0, t.data(), &ne, &best_L));
+        wr::check(wr_gtsp_best(g_, colony, t.data(), &ne, &best_L));
         best_path.resize(ne);
         for (int i = 0; i < ne; i++) best_path[i] = std::make_pair(t[2 * i], t[2 * i + 1]);
     }

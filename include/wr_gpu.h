@@ -240,6 +240,14 @@ int wr_acs_peer_set_pointers(wr_acs* a, void* const* all_raw_pointers);
 int wr_gtsp_create(const double* dis, int n, int cnt, int batch, int colony_first, uint64_t seed, wr_gtsp** out);
 int wr_gtsp_destroy(wr_gtsp* g);
 int wr_gtsp_iterate(wr_gtsp* g, int iterations);   /* loop body of computeSolution :261-276, no early stop */
+/* computeSolution :255-284 for EVERY colony of the handle, on the device.  Colony b repeats the loop body until it has run
+ * max_iterations iterations (0: the reference's MAX_itera = n*n) or until more than n consecutive iterations did not
+ * lower its best (bad_times > city_num, :263-275; `last` and bad_times start afresh with every call, like the reference's
+ * locals) -- each colony on its own.  iterations[b] (optional): iterations colony b ran in this call.
+ * best_L_history (optional, [batch][max_iterations or n*n]): colony b's best L after each of its iterations (what the facade
+ * prints); entries past iterations[b] are not written.  *best_colony (optional): the colony with the lowest best L, lowest
+ * index on ties.  Later wr_gtsp_iterate / wr_gtsp_solve calls continue every colony from its own iteration count. */
+int wr_gtsp_solve(wr_gtsp* g, int max_iterations, int* iterations, double* best_L_history, int* best_colony);
 int wr_gtsp_sync(wr_gtsp* g);
 /* best tour of colony b: 2 ints per edge (r, s), n edges (closing edge last); L excludes the
  * closing edge (ACS_Tour::calc :36-44). */

@@ -38,7 +38,7 @@ wr_acs_default_params wr_acs_create wr_acs_destroy wr_acs_set_points wr_acs_set_
 wr_acs_iterate wr_acs_sync wr_acs_reset wr_acs_best wr_acs_download_pheromone wr_acs_upload_pheromone
 wr_acs_last_colony wr_acs_last_ant wr_acs_counters wr_acs_kernel_ms wr_acs_update_stats wr_acs_field_stats wr_acs_stream_kernel_ms wr_acs_set_timing wr_acs_bench_kernel wr_acs_set_stream
 wr_comm_unique_id wr_acs_comm_init wr_acs_set_shard wr_acs_peer_export wr_acs_peer_import wr_acs_peer_set_pointers
-wr_gtsp_create wr_gtsp_destroy wr_gtsp_iterate wr_gtsp_sync wr_gtsp_best wr_gtsp_download_pheromone wr_gtsp_tau0
+wr_gtsp_create wr_gtsp_destroy wr_gtsp_iterate wr_gtsp_solve wr_gtsp_sync wr_gtsp_best wr_gtsp_download_pheromone wr_gtsp_tau0
 wr_gtsp_kernel_ms wr_bspline_eval""".split()
 
 
@@ -81,7 +81,7 @@ def lib():
         "wr_acs_set_timing": [vp, i32], "wr_acs_bench_kernel": [vp, i32, i32, vp], "wr_acs_set_stream": [vp, vp], "wr_acs_set_shard": [vp, i32, i32],
         "wr_comm_unique_id": [vp], "wr_acs_comm_init": [vp, vp, i32, i32],
         "wr_acs_peer_export": [vp, vp, vp], "wr_acs_peer_import": [vp, vp], "wr_acs_peer_set_pointers": [vp, vp],
-        "wr_gtsp_create": [vp, i32, i32, i32, i32, u64, vp], "wr_gtsp_destroy": [vp], "wr_gtsp_iterate": [vp, i32],
+        "wr_gtsp_create": [vp, i32, i32, i32, i32, u64, vp], "wr_gtsp_destroy": [vp], "wr_gtsp_iterate": [vp, i32], "wr_gtsp_solve": [vp, i32, vp, vp, vp],
         "wr_gtsp_sync": [vp], "wr_gtsp_best": [vp, i32, vp, vp, vp], "wr_gtsp_download_pheromone": [vp, i32, vp],
         "wr_gtsp_tau0": [vp, vp], "wr_gtsp_kernel_ms": [vp, vp],
         "wr_bspline_eval": [i32, i32, i32, vp, vp, vp, i32, i32, f32, vp, i32, vp, vp, vp, vp],

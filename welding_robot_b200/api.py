@@ -530,10 +530,13 @@ class ACS_Rank(GridMap):
 class ACS_GTSP:
     """ACS_GTSP (core/ACS_GTSP.hpp:82-328): ant-colony ordering of the weld seams (a symmetric TSP
     over the pair-length matrix), on the GPU.  `computeBatch` is the batched entry point the
-    reference lacks: B independent colonies on the same matrix, one CTA each."""
+    reference lacks: B independent colonies on the same matrix, one CTA each.  `colonies` (an
+    addition) is the batch setDistanceMatrix creates: computeSolution then runs them all, each to
+    the reference's stopping rule, and keeps the best colony's tour (multi-start)."""
 
-    def __init__(self, seed=0):
+    def __init__(self, seed=0, colonies=1):
         self.seed = seed
+        self.colonies = colonies
         self.city_num = 0
         self.dis = None
         self.cnt = 0
@@ -566,7 +569,7 @@ class ACS_GTSP:
         self.city_num = dis.shape[0]
         self.dis = dis
         self.cnt = self.city_num * (self.city_num - 1) // 2 if cnt is None else cnt
-        self._create(1)
+        self._create(self.colonies)
         self.init_flag = True
         return True
 
@@ -603,25 +606,29 @@ class ACS_GTSP:
         check(lib().wr_gtsp_kernel_ms(self._g, ptr(out)))
         return dict(info=float(out[0]), construct=float(out[1]), update=float(out[2]))
 
+    def solve(self, max_iterations=0):
+        """wr_gtsp_solve: every colony iterates until max_iterations (0: N^2) or more than N
+        iterations without improvement.  Returns (iterations per colony, [B][cap] best L after each
+        iteration (valid up to that colony's count), the colony with the lowest best L)."""
+        cap = max_iterations if max_iterations > 0 else self.city_num * self.city_num
+        ran = np.zeros(self._batch, np.int32)
+        # np.empty: only the pages up to each colony's iteration count are ever touched
+        hist = np.empty((self._batch, cap), np.float64)
+        bc = C.c_int()
+        check(lib().wr_gtsp_solve(self._g, max_iterations, ptr(ran), ptr(hist), C.byref(bc)))
+        return ran, hist, bc.value
+
     def computeSolution(self, max_iterations=None):
         """ACS_GTSP.hpp:255-284: iterate until MAX_itera = N^2 or more than N iterations without
-        improvement."""
+        improvement, on the device for every colony; report the best colony."""
         if not self.init_flag:
             return False
-        last = float(0x3f3f3f3f)
-        bad_times = 0
         max_it = self.city_num * self.city_num if max_iterations is None else max_iterations
-        for index_itera in range(max_it):
-            if bad_times > self.city_num:
-                break
-            self.iterate(1)
-            self.best_path, self.best_L = self.best(0)
-            print("iteration %d:Best so far = %.2f" % (index_itera, self.best_L))
-            if last > self.best_L:
-                last = self.best_L
-                bad_times = 0
-            else:
-                bad_times += 1
+        if max_it > 0:
+            ran, hist, b = self.solve(max_it)
+            for index_itera in range(ran[b]):
+                print("iteration %d:Best so far = %.2f" % (index_itera, hist[b, index_itera]))
+            self.best_path, self.best_L = self.best(b)
         print("Best in all = %.2f" % self.best_L)
         if len(self.best_path):
             print("->".join(str(r + 1) for r, _ in self.best_path) + "->%d" % (self.best_path[-1][1] + 1))

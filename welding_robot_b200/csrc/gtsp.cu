@@ -34,11 +34,26 @@ constexpr int kGtspMaxStages = 4; // TMA ring depth is a template parameter of t
 constexpr int kGtspIv = 16;      // check-point interval (cities)
 constexpr double kGtspInf = 1061109567.0;   // INF 0x3f3f3f3f (ACS_GTSP.hpp:19), ACS_Tour::clean :29-34
 
+// computeSolution's locals (:258-259) for one colony during one wr_gtsp_solve call
+struct GtspSolve {
+    double last;                 // lowest best L seen in this call
+    int bad_times;               // consecutive iterations that did not lower it
+    int ran;                     // iterations run in this call
+};
+
+// the stopping rule of computeSolution (:262-264), with the iteration cap of the call
+__device__ __forceinline__ bool gtsp_stopped(const GtspSolve& s, int n, int cap) { return s.bad_times > n || s.ran >= cap; }
+
 struct GtspArgs {
     int n, npad;                 // cities; row stride of every matrix (multiple of 2 doubles = 16 B)
     int stages;                  // TMA ring depth
     size_t mat_stride;           // doubles between consecutive colonies' matrices
-    int iterations, iter0;
+    int iterations;              // per colony in this launch (a solve launch: at most this many)
+    int* iter;                   // [B] iterations each colony has run so far: the Philox iteration index of its next one
+    GtspSolve* solve;            // [B] stopping-rule state of a wr_gtsp_solve launch; nullptr: wr_gtsp_iterate, no stopping rule
+    int cap;                     // solve: iterations per colony in the whole call
+    double* hist;                // solve (nullable): [B][iterations] best L after each iteration of this launch
+    int* running;                // solve: incremented by every colony that has not stopped at the end of the launch
     int colony_first;
     uint32_t seed_lo, seed_hi;
     double evap;                 // 1 - alpha (:177), computed in double on the host
@@ -77,7 +92,7 @@ __global__ void k_gtsp_iterate(GtspArgs a)
     double* redL = reinterpret_cast<double*>(vis + (size_t)nwords * nthreads);    // [32]
     int* redK = reinterpret_cast<int*>(redL + 32);                            // [32]
     uint64_t* bar = reinterpret_cast<uint64_t*>(redK + 32);                   // [kGtspStages]
-    int* bcast = reinterpret_cast<int*>(bar + kGtspMaxStages);                // [4]
+    int* bcast = reinterpret_cast<int*>(bar + kGtspMaxStages);                // [4]: winner, improved, stopped, first iteration
 
     const size_t mat = (size_t)n * npad;
     const int colony = blockIdx.x;
@@ -89,6 +104,8 @@ __global__ void k_gtsp_iterate(GtspArgs a)
     if (k == 0) {
         for (int s = 0; s < kGtspStages; s++) tma::mbar_init(&bar[s], 1);
         tma::fence_barrier_init();
+        bcast[2] = a.solve ? gtsp_stopped(a.solve[colony], n, a.cap) : 0;   // a colony that stopped in an earlier launch returns at once
+        bcast[3] = a.iter[colony];
     }
     __syncthreads();
     unsigned phase_bits = 0;   // bit s: parity of the next wait on bar[s]
@@ -103,8 +120,12 @@ __global__ void k_gtsp_iterate(GtspArgs a)
     };
     unsigned long long t_info = 0, t_cons = 0, t_upd = 0;
 
-    for (int it = 0; it < a.iterations; it++) {
-        const uint32_t iter = (uint32_t)(a.iter0 + it);
+    // bcast[2] is set by thread 0 before the barrier that ends an iteration and read by all threads after it, so the stop
+    // is uniform over the CTA.  Leaving between iterations is safe for the TMA ring: an iteration issues and waits for
+    // exactly `total` chunks, so no bulk copy is in flight into shared memory there.
+    int it = 0;
+    for (; it < a.iterations && !bcast[2]; it++) {
+        const uint32_t iter = (uint32_t)(bcast[3] + it);
         unsigned long long t0 = gtimer();
         // ---- reset(): info = pheromone^1 * heuristic^6 (:114-119) --------------------------------
         for (size_t i = k; i < mat; i += nthreads) info[i] = __dmul_rn(__dmul_rn(1.0, ph[i]), a.h6[i]);
@@ -219,6 +240,15 @@ __global__ void k_gtsp_iterate(GtspArgs a)
                 redL[0] = bl; bcast[0] = have ? bk : -1;
                 bcast[1] = (have && bl < a.best_L[colony]) ? 1 : 0;   // now_best < best (:171-174)
                 if (bcast[1]) { a.best_L[colony] = bl; a.best_start[colony] = bk; }
+                if (a.solve) {   // computeSolution :266-275
+                    GtspSolve s = a.solve[colony];
+                    const double best = a.best_L[colony];
+                    if (s.last > best) { s.last = best; s.bad_times = 0; } else s.bad_times++;
+                    if (a.hist) a.hist[(size_t)colony * a.iterations + it] = best;
+                    s.ran++;
+                    a.solve[colony] = s;
+                    bcast[2] = gtsp_stopped(s, n, a.cap);
+                }
             }
         }
         __syncthreads();
@@ -246,6 +276,8 @@ __global__ void k_gtsp_iterate(GtspArgs a)
     }
     if (k == 0) {
         atomicAdd(&a.phase_ns[0], t_info); atomicAdd(&a.phase_ns[1], t_cons); atomicAdd(&a.phase_ns[2], t_upd);
+        a.iter[colony] = bcast[3] + it;
+        if (a.solve && !bcast[2]) atomicAdd(a.running, 1);
     }
 }
 
@@ -255,12 +287,16 @@ using namespace wr;
 
 struct wr_gtsp {
     int device = 0;
-    int n = 0, npad = 0, batch = 0, colony_first = 0, iter = 0;
+    int n = 0, npad = 0, batch = 0, colony_first = 0;
     uint64_t seed = 0;
     double tau0 = 0;
     double *d_dis = nullptr, *d_h6 = nullptr, *d_ph = nullptr, *d_info = nullptr, *d_best_L = nullptr;
     uint16_t *d_tours = nullptr, *d_best_tour = nullptr;
     int* d_best_start = nullptr;
+    int* d_iter = nullptr;                 // [batch] iterations run per colony
+    GtspSolve* d_solve = nullptr;          // [batch], allocated by the first wr_gtsp_solve
+    double* d_hist = nullptr;              // [batch][kGtspSolveSlice]
+    int* d_running = nullptr;
     unsigned long long* d_phase = nullptr;
     cudaStream_t stream = nullptr;
     float ms_total = 0;
@@ -283,6 +319,7 @@ extern "C" int wr_gtsp_destroy(wr_gtsp* g)
     if (g->stream) { cudaStreamSynchronize(g->stream); cudaStreamDestroy(g->stream); }
     cudaFree(g->d_dis); cudaFree(g->d_h6); cudaFree(g->d_ph); cudaFree(g->d_info); cudaFree(g->d_best_L);
     cudaFree(g->d_tours); cudaFree(g->d_best_tour); cudaFree(g->d_best_start); cudaFree(g->d_phase);
+    cudaFree(g->d_iter); cudaFree(g->d_solve); cudaFree(g->d_hist); cudaFree(g->d_running);
     delete g;
     return WR_OK;
 }
@@ -352,6 +389,8 @@ extern "C" int wr_gtsp_create(const double* dis, int n, int cnt, int batch, int 
     WR_CUDA_G(cudaMalloc(&g->d_best_L, batch * sizeof(double)));
     WR_CUDA_G(cudaMalloc(&g->d_phase, 3 * sizeof(unsigned long long)));
     WR_CUDA_G(cudaMemset(g->d_phase, 0, 3 * sizeof(unsigned long long)));
+    WR_CUDA_G(cudaMalloc(&g->d_iter, batch * sizeof(int)));
+    WR_CUDA_G(cudaMemset(g->d_iter, 0, batch * sizeof(int)));
     WR_CUDA_G(cudaMemcpy(g->d_dis, hd.data(), mat * sizeof(double), cudaMemcpyHostToDevice));
     WR_CUDA_G(cudaMemcpy(g->d_h6, hh.data(), mat * sizeof(double), cudaMemcpyHostToDevice));
     {
@@ -372,18 +411,21 @@ extern "C" int wr_gtsp_create(const double* dis, int n, int cnt, int batch, int 
     return WR_OK;
 }
 
-// the loop body of computeSolution :261-276, `iterations` times per colony, without the early stop
-extern "C" int wr_gtsp_iterate(wr_gtsp* g, int iterations)
+static GtspArgs gtsp_args(const wr_gtsp* g, int iterations)
 {
-    WR_REQUIRE(g && iterations >= 0, WR_ERR_INVALID, "wr_gtsp_iterate: bad argument");
-    if (iterations == 0) return WR_OK;
-    WR_CUDA(cudaSetDevice(g->device));
     GtspArgs a;
-    a.n = g->n; a.npad = g->npad; a.stages = g->stages; a.mat_stride = g->mat_stride; a.iterations = iterations; a.iter0 = g->iter; a.colony_first = g->colony_first;
+    a.n = g->n; a.npad = g->npad; a.stages = g->stages; a.mat_stride = g->mat_stride; a.iterations = iterations; a.iter = g->d_iter;
+    a.solve = nullptr; a.cap = 0; a.hist = nullptr; a.running = nullptr; a.colony_first = g->colony_first;
     a.seed_lo = (uint32_t)g->seed; a.seed_hi = (uint32_t)(g->seed >> 32);
     a.evap = 1 - 0.1;   // (1 - alpha), alpha = 0.1 (:189)
     a.dis = g->d_dis; a.h6 = g->d_h6; a.ph = g->d_ph; a.info = g->d_info; a.tours = g->d_tours; a.best_tour = g->d_best_tour;
     a.best_start = g->d_best_start; a.best_L = g->d_best_L; a.phase_ns = g->d_phase;
+    return a;
+}
+
+// one launch of k_gtsp_iterate over every colony, event-timed into wr_gtsp_kernel_ms; returns after it has finished
+static int gtsp_launch(wr_gtsp* g, const GtspArgs& a)
+{
     cudaEvent_t e0, e1;
     WR_CUDA(cudaEventCreate(&e0));
     WR_CUDA(cudaEventCreate(&e1));
@@ -398,7 +440,67 @@ extern "C" int wr_gtsp_iterate(wr_gtsp* g, int iterations)
     WR_CUDA(cudaEventElapsedTime(&ms, e0, e1));
     cudaEventDestroy(e0); cudaEventDestroy(e1);
     g->ms_total += ms;
-    g->iter += iterations;
+    return WR_OK;
+}
+
+// the loop body of computeSolution :261-276, `iterations` times per colony, without the early stop
+extern "C" int wr_gtsp_iterate(wr_gtsp* g, int iterations)
+{
+    WR_REQUIRE(g && iterations >= 0, WR_ERR_INVALID, "wr_gtsp_iterate: bad argument");
+    if (iterations == 0) return WR_OK;
+    WR_CUDA(cudaSetDevice(g->device));
+    return gtsp_launch(g, gtsp_args(g, iterations));
+}
+
+// Iterations per wr_gtsp_solve launch.  One iteration takes milliseconds at a few hundred cities, and the cap (n*n) reaches
+// 215 296 at 464 cities: the solve is a sequence of bounded launches, with one word (colonies still running) read back after
+// each.  The history goes through a [batch][kGtspSolveSlice] device buffer copied out after each launch.
+constexpr int kGtspSolveSlice = 32;
+
+// computeSolution :255-284 for every colony, each stopping by its own rule
+extern "C" int wr_gtsp_solve(wr_gtsp* g, int max_iterations, int* iterations, double* best_L_history, int* best_colony)
+{
+    WR_REQUIRE(g && max_iterations >= 0, WR_ERR_INVALID, "wr_gtsp_solve: bad argument");
+    WR_CUDA(cudaSetDevice(g->device));
+    const int cap = max_iterations > 0 ? max_iterations : g->n * g->n;   // MAX_itera (:257)
+    const int B = g->batch;
+    if (!g->d_solve) {
+        WR_CUDA(cudaMalloc(&g->d_solve, B * sizeof(GtspSolve)));
+        WR_CUDA(cudaMalloc(&g->d_hist, (size_t)B * kGtspSolveSlice * sizeof(double)));
+        WR_CUDA(cudaMalloc(&g->d_running, sizeof(int)));
+    }
+    std::vector<GtspSolve> st(B, GtspSolve{kGtspInf, 0, 0});   // last = INF, bad_times = 0 (:258-259), afresh with every call
+    WR_CUDA(cudaMemcpyAsync(g->d_solve, st.data(), B * sizeof(GtspSolve), cudaMemcpyHostToDevice, g->stream));
+    GtspArgs a = gtsp_args(g, kGtspSolveSlice);
+    a.solve = g->d_solve; a.cap = cap; a.hist = best_L_history ? g->d_hist : nullptr; a.running = g->d_running;
+    std::vector<double> h(best_L_history ? (size_t)B * kGtspSolveSlice : 0);
+    for (int start = 0;; start += kGtspSolveSlice) {
+        WR_CUDA(cudaMemsetAsync(g->d_running, 0, sizeof(int), g->stream));
+        const int rc = gtsp_launch(g, a);
+        if (rc != WR_OK) return rc;
+        int running = 0;
+        WR_CUDA(cudaMemcpyAsync(&running, g->d_running, sizeof(int), cudaMemcpyDeviceToHost, g->stream));
+        if (best_L_history) {
+            WR_CUDA(cudaMemcpyAsync(st.data(), g->d_solve, B * sizeof(GtspSolve), cudaMemcpyDeviceToHost, g->stream));
+            WR_CUDA(cudaMemcpyAsync(h.data(), g->d_hist, h.size() * sizeof(double), cudaMemcpyDeviceToHost, g->stream));
+        }
+        WR_CUDA(cudaStreamSynchronize(g->stream));
+        // a colony that ran in this launch had run exactly `start` iterations before it (it never stopped earlier)
+        for (int b = 0; best_L_history && b < B; b++)
+            for (int j = 0; j < st[b].ran - start; j++) best_L_history[(size_t)b * cap + start + j] = h[(size_t)b * kGtspSolveSlice + j];
+        if (!running) break;
+    }
+    if (iterations) {
+        WR_CUDA(cudaMemcpy(st.data(), g->d_solve, B * sizeof(GtspSolve), cudaMemcpyDeviceToHost));
+        for (int b = 0; b < B; b++) iterations[b] = st[b].ran;
+    }
+    if (best_colony) {
+        std::vector<double> L(B);
+        WR_CUDA(cudaMemcpy(L.data(), g->d_best_L, B * sizeof(double), cudaMemcpyDeviceToHost));
+        int bc = 0;
+        for (int b = 1; b < B; b++) if (L[b] < L[bc]) bc = b;
+        *best_colony = bc;
+    }
     return WR_OK;
 }
 
@@ -443,7 +545,7 @@ extern "C" int wr_gtsp_tau0(wr_gtsp* g, double* tau0)
     return WR_OK;
 }
 
-// event-timed total of all wr_gtsp_iterate calls, split by the CTAs' own phase clocks
+// event-timed total of all wr_gtsp_iterate and wr_gtsp_solve launches, split by the CTAs' own phase clocks
 extern "C" int wr_gtsp_kernel_ms(wr_gtsp* g, float out[3])
 {
     WR_REQUIRE(g && out, WR_ERR_INVALID, "wr_gtsp_kernel_ms: null");
