@@ -1,5 +1,5 @@
-"""Short concurrent-search run for ncu captures of k_walk_batch and the per-query kernels: C5-shaped queries on a synthetic
-obstacle grid (256^3 by default), 256 ants each.
+"""Short concurrent-search run for ncu captures of the batch walk (k_walk_batch3, pass 2 k_walk2<Batch6>) and the per-query
+kernels: C5-shaped queries on a synthetic obstacle grid (256^3 by default), 256 ants each.
 
     ncu --set full --clock-control none --import-source on -k regex:k_walk_batch -s 4 -c 2 -o gpurun_out/wb python scripts/profile_batch.py 256 512 6
 """

@@ -124,7 +124,7 @@ def test_queries_on_an_obstacle_grid_k26(wr):
 
 
 def test_axis_beyond_1024_k26(wr, oracle):
-    """A 1100 x 6 x 5 corridor with scattered obstacles: k_walk_batch26 uses unpacked coordinates, so an axis beyond 1024
+    """A 1100 x 6 x 5 corridor with scattered obstacles: k_walk26<Batch26> uses unpacked coordinates, so an axis beyond 1024
     nodes batches like any other grid."""
     dims = (1100, 6, 5)
     rx, ry, rz = dims

@@ -104,7 +104,7 @@ def test_ranking_step_caps_beyond_16_bit_keys(wr, oracle, meshes, step_cap, upda
 # ---------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("alpha", [2, 0])
 def test_k6_resume_pass_with_alpha(wr, oracle, meshes, alpha):
-    """16-slot visited tables: ants park in k_walk3 and finish in k_walk2<false> (the alpha != 1 resume pass)."""
+    """16-slot visited tables: ants park in k_walk3 and finish in k_walk2<Dense6, false> (the alpha != 1 resume pass)."""
     A, g = piece_pair(wr, oracle, meshes, seed=7, fixed_colony=512, step_cap=300, walk_table_log2=4, alpha=alpha)
     for _ in range(4):
         A.iterate(1); g.iterate(1)
@@ -132,7 +132,7 @@ def test_k6_predicted_gathers_with_alpha(wr, oracle, meshes, monkeypatch):
 @pytest.mark.parametrize("alpha,beta,rho,tau0", [(2, 0.9, 0.7, 0.5), (3, 0.3, 0.93, 2.5), (0, 0.6, 0.8, 1.0)])
 def test_k26_non_default_parameters(wr, oracle, meshes, alpha, beta, rho, tau0, update_mode, table_log2):
     """K = 26 away from the defaults: k_walk26p's alpha branch, k_heuristic26 with beta != 0.6, evaporation and initial
-    pheromone away from 0.8 / 1; with 16-slot tables the ants park and finish in k_walk26<true> with alpha != 1."""
+    pheromone away from 0.8 / 1; with 16-slot tables the ants park and finish in k_walk26<Dense26, true> with alpha != 1."""
     A, g = piece_pair(wr, oracle, meshes, seed=11, fixed_colony=384, step_cap=200, K=26, walk_table_log2=table_log2,
                       alpha=alpha, beta=beta, rho=rho, tau0=tau0, update_mode=update_mode)
     for it in range(3):
@@ -149,7 +149,7 @@ def test_k26_non_default_parameters(wr, oracle, meshes, alpha, beta, rho, tau0, 
 
 def test_k26_axis_beyond_1024(wr, oracle):
     """A 1100 x 6 x 5 corridor with scattered obstacles, endpoints at both ends: an axis beyond the 10-bit packed
-    coordinates, so K = 26 walks with k_walk26<false> instead of k_walk26p."""
+    coordinates, so K = 26 walks with k_walk26<Dense26, false> instead of k_walk26p."""
     dims = (1100, 6, 5)
     rx, ry, rz = dims
     free = np.ones((rz, ry, rx), np.uint8)
@@ -222,7 +222,7 @@ def batch_vs_sequential(wr, oracle, meshes, nq, iters, oracle_queries, **params)
 
 
 def test_batch_alpha2_parked_ants(wr, oracle, meshes, monkeypatch):
-    """16-entry batch visited tables with alpha = 2: the parked ants finish in k_walk_batch<false>."""
+    """16-entry batch visited tables with alpha = 2: the parked ants finish in k_walk2<Batch6, false>."""
     monkeypatch.setenv("WR_BATCH_TABLE", "16")
     g2 = batch_vs_sequential(wr, oracle, meshes, 16, 10, (0, 15), fixed_colony=150, step_cap=400, alpha=2, beta=0.9, rho=0.7, tau0=0.5)
     st = g2.batchStats()
@@ -276,7 +276,7 @@ def test_gtsp_city_limit(wr):
 # ---------------------------------------------------------------------------------------------
 # 5. debug switches that must give identical bits (DESIGN.md §6)
 # ---------------------------------------------------------------------------------------------
-# WR_WALK_PREFETCH, WR_STREAM_CS, WR_GRAPH and WR_WALK_WARM are read once per process: each setting runs in a child process
+# WR_WALK_PREFETCH, WR_STREAM_CS and WR_GRAPH are read once per process: each setting runs in a child process
 # of its own.  The child runs the C1 adaptive scenario, records which kernels ran (torch.profiler) and saves the best path,
 # the counters and the final field.
 _CHILD = r"""
@@ -316,8 +316,7 @@ def _has(kernels, pattern):
     return any(re.search(pattern, k) for k in kernels)
 
 
-@pytest.mark.parametrize("var,value", [("WR_WALK_PREFETCH", "0"), ("WR_WALK_PREFETCH", "1"), ("WR_STREAM_CS", "0"), ("WR_GRAPH", "0"),
-                                       ("WR_WALK_WARM", "1")])
+@pytest.mark.parametrize("var,value", [("WR_WALK_PREFETCH", "0"), ("WR_WALK_PREFETCH", "1"), ("WR_STREAM_CS", "0"), ("WR_GRAPH", "0")])
 def test_debug_switch_gives_identical_bits(c1_oracle_30, tmp_path, var, value):
     out = tmp_path / "run.npz"
     env = dict(os.environ)
@@ -339,12 +338,9 @@ def test_debug_switch_gives_identical_bits(c1_oracle_30, tmp_path, var, value):
     if var == "WR_WALK_PREFETCH":
         assert not _has(kernels, r"k_walk3<true, ?%d>" % (1 - int(value))), kernels
         assert _has(kernels, r"k_walk3<true, ?%s>" % value), kernels
-    elif var == "WR_WALK_WARM":
-        assert _has(kernels, r"k_path_warm|k_rankset_warm"), kernels
-    else:   # the defaults: prefetching walks on record iterations, plain ones on rank-set iterations; no warm-up kernels
+    else:   # the defaults: prefetching walks on record iterations, plain ones on rank-set iterations
         assert _has(kernels, r"k_walk3<true, ?1>"), kernels
         assert _has(kernels, r"k_walk3<true, ?0>") == _has(kernels, r"k_rankset_apply"), kernels
-        assert not _has(kernels, r"k_path_warm|k_rankset_warm"), kernels
 
 
 @pytest.mark.parametrize("update_mode", [0, 4])

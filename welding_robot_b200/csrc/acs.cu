@@ -134,7 +134,6 @@ struct wr_acs {
     bool in_process_peers = false;   // the peers are handles of THIS process (wr_acs_peer_set_pointers; tests): one plain stream per shard, see there
     int* d_nq = nullptr;              // records in this rank's slot slice
     unsigned parity = 0;              // flips at every wr_acs_walk of a sharded handle
-    bool warm_by_pull = false;        // the last iteration ended with k_pull_finals (which doubles as the L2 warm-up)
 
     float* d_tau = nullptr;
     float* d_heur = nullptr;          // [N][6] heuristic factor for the current goal
@@ -285,7 +284,7 @@ static void feedback_release(uint32_t* h)
 // stream-ordered pool whose blocks are tied to the allocating handle's stream.
 static void rankset_release_buffers(RankSet& rs, cudaStream_t)
 {
-    cudaFree(rs.key); cudaFree(rs.rows); cudaFree(rs.list); cudaFree(rs.touched); cudaFree(rs.count); cudaFree(rs.vtab);
+    cudaFree(rs.key); cudaFree(rs.rows); cudaFree(rs.list); cudaFree(rs.count); cudaFree(rs.vtab);
     rs = RankSet{};
 }
 
@@ -444,7 +443,6 @@ static int alloc_colony_buffers(wr_acs* a, int colony_max)
             WR_CUDA(cudaMemsetAsync(a->rs.key, 0, R * sizeof(unsigned long long), s));
             WR_CUDA(cudaMemsetAsync(a->rs.rows, 0, R * kRsRowWords * sizeof(uint32_t), s));
             WR_CUDA(cudaMalloc(&a->rs.list, ((size_t)limit + 1) * sizeof(uint32_t)));
-            WR_CUDA(cudaMalloc(&a->rs.touched, ((size_t)limit + 1) * sizeof(uint32_t)));
             WR_CUDA(cudaMalloc(&a->rs.count, 8 * sizeof(uint32_t)));
             WR_CUDA(cudaMalloc(&a->rs.vtab, (size_t)2 * (a->w_max + 1) * sizeof(float)));
         }
@@ -484,14 +482,6 @@ static int walk_prefetch()
 static int stream_cs()
 {
     static const int env = [] { const char* e = getenv("WR_STREAM_CS"); return e ? atoi(e) : 1; }();   // evict-first streaming of the tiles without deposits (default on)
-    return env;
-}
-static int walk_warm()
-{
-    // The L2 warm-up of the rows under the last deposits (k_path_warm / k_rankset_warm) paid in round 1, when every step's gather
-    // was a demand load; with the gathers predicted a trip ahead (converged colony) or prefetched a step ahead (wandering colony)
-    // it no longer does: off, value 7.42 -> 7.46e9, converged iteration 0.3185 -> 0.3154 ms, e2e 3.27 -> 3.31e9.  WR_WALK_WARM=1 restores it.
-    static const int env = [] { const char* e = getenv("WR_WALK_WARM"); return e ? atoi(e) : 0; }();
     return env;
 }
 static size_t walk_smem(const wr_acs* a)
@@ -643,7 +633,7 @@ extern "C" int wr_acs_create(wr_grid* g, const wr_acs_params* p, wr_acs** out)
         const size_t ws = walk_smem(a);
         if (ws > 227 * 1024) { set_error("wr_acs_create: walk shared memory %zu B exceeds 227 KB", ws); wr_acs_destroy(a); return WR_ERR_INVALID; }
         if (a->K == kK26) {
-            WR_CUDA_A(cudaFuncSetAttribute(k_walk26<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws));
+            WR_CUDA_A(cudaFuncSetAttribute(k_walk26<Dense26, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws));
             WR_CUDA_A(cudaFuncSetAttribute(k_walk26p, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ws));
         }
         else {
@@ -808,19 +798,6 @@ extern "C" int wr_acs_begin(wr_acs* a, float predict)
     return WR_OK;
 }
 
-// before k_iter_begin: pull the rows under last iteration's deposits into L2 (see k_path_warm)
-static void launch_warm(wr_acs* a, bool prev_rankset)
-{
-    if (!walk_warm() || a->p.update_mode == WR_UPDATE_ATOMIC || a->K != 6) return;
-    if (a->rankset && a->rs_enqueued > 0 && prev_rankset) {   // the previous iteration's deposits went through rank sets
-        k_rankset_warm<<<kNumSMs, 256, 0, a->stream>>>(a->rs.touched, a->rs.count, a->d_tau, a->d_heur, a->d_state);
-        return;
-    }
-    if (a->warm_by_pull) return;   // owner-computes update: k_pull_finals has just touched the rows under the deposits
-    const uint32_t* ck = a->recs_in_b ? a->sort_recs.keys_b : a->sort_recs.keys_a;
-    k_path_warm<<<kNumSMs, 256, 0, a->stream>>>(a->d_state, ck, a->d_tau, a->d_heur);
-}
-
 static int launch_walk(wr_acs* a)
 {
     const wr_grid* g = a->g;
@@ -836,16 +813,15 @@ static int launch_walk(wr_acs* a)
     w.ant_steps = a->d_local_steps;
     w.path_ids = a->d_path_ids; w.path_dirs = a->d_path_dirs;
     w.table_log2 = a->table_log2; w.table_entries = a->table_entries; w.overflow_list = a->d_overflow;
-    w.gkeys = a->d_gkeys; w.gmasks = a->d_gmasks; w.gtab = a->d_gmasks; w.gtable_log2 = a->gtable_log2; w.resume = a->d_resume;
+    w.gkeys = a->d_gkeys; w.gtab = a->d_gmasks; w.gtable_log2 = a->gtable_log2; w.resume = a->d_resume;
     w.precision = g->precision; w.ant_L = a->d_ant_L; w.best_ids = a->d_best_ids;
     if (a->K == kK26) {
         const size_t smem = walk_smem(a);
         const int per_sm = std::max(1, std::min((int)((227 * 1024) / (smem + 1024)), 16));
         const int blocks = std::max(1, std::min((a->chunk + kWalk26Ants - 1) / kWalk26Ants, kNumSMs * per_sm));
         if (g->rx <= 1024 && g->ry <= 1024 && g->rz <= 1024) k_walk26p<<<blocks, kWalk26Threads, smem, a->stream>>>(w);
-        else k_walk26<false><<<blocks, kWalk26Threads, smem, a->stream>>>(w);
-        w.table_log2 = a->gtable_log2;
-        k_walk26<true><<<std::max(1, std::min((a->chunk + kWalk26Ants - 1) / kWalk26Ants, kNumSMs * 4)), kWalk26Threads, 0, a->stream>>>(w);
+        else k_walk26<Dense26, false><<<blocks, kWalk26Threads, smem, a->stream>>>(w);
+        k_walk26<Dense26, true><<<std::max(1, std::min((a->chunk + kWalk26Ants - 1) / kWalk26Ants, kNumSMs * 4)), kWalk26Threads, 0, a->stream>>>(w);
         WR_CUDA(cudaGetLastError());
         return WR_OK;
     }
@@ -864,8 +840,8 @@ static int launch_walk(wr_acs* a)
     else k_walk3<true, 0><<<blocks1, kWalkThreads, smem1, a->stream>>>(w);
     // pass 2: resume the ants that parked on a full shared-memory table (usually none: the kernel exits at once)
     w.table_log2 = a->gtable_log2;
-    if (alpha1) k_walk2<true><<<a->walk2_blocks, kWalkThreads, kWalk2Lut, a->stream>>>(w);
-    else k_walk2<false><<<a->walk2_blocks, kWalkThreads, kWalk2Lut, a->stream>>>(w);
+    if (alpha1) k_walk2<Dense6, true><<<a->walk2_blocks, kWalkThreads, kWalk2Lut, a->stream>>>(w);
+    else k_walk2<Dense6, false><<<a->walk2_blocks, kWalkThreads, kWalk2Lut, a->stream>>>(w);
     WR_CUDA(cudaGetLastError());
     return WR_OK;
 }
@@ -1027,8 +1003,8 @@ static int launch_record_update_sharded(wr_acs* a)
     WR_CUDA(cudaMemsetAsync(fin, 0, 4 * sizeof(uint32_t), s));
     st = launch_fused(a, ck, cv, a->d_nq, fin);
     if (st != WR_OK) return st;
-    k_pull_finals<<<barrier_grid(a, kNumSMs * 2), 256, 0, s>>>(barrier_args(a), a->d_state, a->d_tau, walk_warm() ? a->d_heur : nullptr,
-                                              reinterpret_cast<const uint32_t* const*>(a->tab(2, a->parity)), a->nranks, a->rank, a->d_dirty, a->d_upd_q);
+    k_pull_finals<<<barrier_grid(a, kNumSMs * 2), 256, 0, s>>>(barrier_args(a), a->d_state, a->d_tau, reinterpret_cast<const uint32_t* const*>(a->tab(2, a->parity)),
+                                                                a->nranks, a->rank, a->d_dirty, a->d_upd_q);
     WR_CUDA(cudaGetLastError());
     return WR_OK;
 }
@@ -1094,7 +1070,7 @@ static int launch_construct_and_rank(wr_acs* a, bool rankset_iteration)
 }
 
 // One rank-set iteration whose predecessor was a rank-set iteration too, captured from the very launch sequence of
-// wr_acs_iterate (k_iter_end of the predecessor folded into k_iter_begin): L2 warm-up, iteration parameters, walk pass 1 + 2,
+// wr_acs_iterate (k_iter_end of the predecessor folded into k_iter_begin): iteration parameters, walk pass 1 + 2,
 // ranking, best copy, rank-set build, evaporation of the dirty tiles, ordered chains.  Every argument is fixed for the search
 // (sharded handles alternate between two trail buffers, hence one graph per parity).
 static int capture_steady_iteration(wr_acs* a, cudaGraphExec_t* out)
@@ -1102,7 +1078,6 @@ static int capture_steady_iteration(wr_acs* a, cudaGraphExec_t* out)
     cudaStream_t s = a->stream;
     if (s == nullptr || s == cudaStreamLegacy || s == cudaStreamPerThread) return WR_ERR_STATE;   // the default streams cannot be captured
     WR_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    launch_warm(a, true);
     k_iter_begin<<<1, 1, 0, s>>>(a->d_state, a->p.fixed_colony, a->colony_max, a->g->precision, a->p.tau0, 1, a->d_upd_q, a->rs.count, 1, a->d_feedback,
                                  a->rs_generation, a->p.rho);
     int st = launch_construct_and_rank(a, true);
@@ -1151,7 +1126,7 @@ extern "C" int wr_acs_iterate(wr_acs* a, int n)
     if (n > 0) a->field_clean = false;
     for (int it = 0; it < n; it++) {
         if (a->timer.enabled) cudaEventRecord(a->timer.next(), s);
-        const bool rs_prev = a->rankset && a->rs_choice;   // path of the previous iteration (what the L2 warm-up reads)
+        const bool rs_prev = a->rankset && a->rs_choice;   // path of the previous iteration
         if (a->rankset) { int rc = choose_deposit_path(a); if (rc != WR_OK) return rc; }
         const bool rs_now = a->rankset && a->rs_choice;
         if (sharded) {   // trails and step counts are double-buffered: a peer may still be reading the previous iteration's
@@ -1171,20 +1146,18 @@ extern "C" int wr_acs_iterate(wr_acs* a, int n)
                 continue;
             }
         }
-        launch_warm(a, rs_prev);
         k_iter_begin<<<1, 1, 0, s>>>(a->d_state, a->p.fixed_colony, a->colony_max, a->g->precision, a->p.tau0, it > 0 ? 1 : 0, a->d_upd_q,
                                      a->rankset ? a->rs.count : nullptr, rs_now ? 1 : 0, a->d_feedback, a->rs_generation, a->p.rho);
         a->upd_q_zeroed = true;
         int st = launch_construct_and_rank(a, rs_now);
         if (st != WR_OK) return st;
         if (rs_now) st = launch_rankset_update(a);   // rank sets instead of sorted records (rankset.cuh)
-        else if (sharded) { st = launch_record_update_sharded(a); a->warm_by_pull = true; }
+        else if (sharded) st = launch_record_update_sharded(a);
         else {
             st = launch_deposit_gen(a);
             if (st == WR_OK) st = launch_update(a);
         }
         if (st != WR_OK) return st;
-        if (rs_now) a->warm_by_pull = false;
         if (a->rankset) { WR_CUDA(cudaEventRecord(a->rs_ev[a->rs_enqueued % wr_acs::kRsAhead], s)); a->rs_enqueued++; }
         a->upd_q_zeroed = false;
         if (it == n - 1) k_iter_end<<<1, 1, 0, s>>>(a->d_state, a->p.rho);   // otherwise folded into the next k_iter_begin
@@ -1423,7 +1396,7 @@ static int alloc_batch(wr_acs* a, int want_q, int cm, int* qc_out)
     WR_CUDA(cudaMalloc(&b->res_n, nq * sizeof(int)));
     if (k26) WR_CUDA(cudaMalloc(&b->ant_L, nq * cm * sizeof(float)));
     // HBM visited tables for ants whose shared-memory table fills up: a pool (2 GB at most), handed out on demand.  K = 6:
-    // k_walk_batch's 64-bit key|mask entries; K = 26: k_walk26's format, u32 tile keys + u64 masks
+    // k_walk2's 64-bit key|mask entries; K = 26: k_walk26's format, u32 tile keys + u64 masks
     const size_t Eg = (size_t)1 << a->gtable_log2_for_cap();
     const size_t gbytes = k26 ? 12 : 8;
     size_t pool = std::min<size_t>(nq * cm, std::max<size_t>(16, ((size_t)2 << 30) / (Eg * gbytes)));
@@ -1478,7 +1451,7 @@ extern "C" int wr_acs_search_batch(wr_acs* a, const int64_t* start_ids, const in
     const int maxn = (std::max(cm, 32) + 31) / 32 * 32;
     const size_t rank_smem = (size_t)12 * maxn + 32 * 256 * sizeof(uint32_t);
     if (k26) {
-        WR_CUDA(cudaFuncSetAttribute(k_walk_batch26<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+        WR_CUDA(cudaFuncSetAttribute(k_walk26<Batch26, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
     } else {
         WR_CUDA(cudaFuncSetAttribute(k_walk_batch3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
         WR_CUDA(cudaFuncSetAttribute(k_walk_batch3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
@@ -1512,14 +1485,14 @@ extern "C" int wr_acs_search_batch(wr_acs* a, const int64_t* start_ids, const in
         for (int it = 0; it < n_iterations; it++) {
             k_batch_iter_begin<<<(n + 255) / 256, 256, 0, s>>>(a->d_state, b->qs, n, a->p.fixed_colony, cm, a->g->precision, a->p.tau0, it > 0 ? 1 : 0, a->p.rho);
             if (k26) {
-                k_walk_batch26<false><<<blocks1, kWalk26Threads, smem1, s>>>(w);
-                k_walk_batch26<true><<<blocks2, kWalk26Threads, 0, s>>>(w);
+                k_walk26<Batch26, false><<<blocks1, kWalk26Threads, smem1, s>>>(w);
+                k_walk26<Batch26, true><<<blocks2, kWalk26Threads, 0, s>>>(w);
             } else if (alpha1) {
                 k_walk_batch3<true><<<blocks1, kWalkThreads, smem1, s>>>(w);
-                k_walk_batch<true><<<blocks2, kWalkThreads, kWalk2Lut, s>>>(w);
+                k_walk2<Batch6, true><<<blocks2, kWalkThreads, kWalk2Lut, s>>>(w);
             } else {
                 k_walk_batch3<false><<<blocks1, kWalkThreads, smem1, s>>>(w);
-                k_walk_batch<false><<<blocks2, kWalkThreads, kWalk2Lut, s>>>(w);
+                k_walk2<Batch6, false><<<blocks2, kWalkThreads, kWalk2Lut, s>>>(w);
             }
             if (k26) batch_rank_update<kBatchEntryWords26>(a, b, n, maxn, rank_smem, s);
             else batch_rank_update<kBatchEntryWords>(a, b, n, maxn, rank_smem, s);
@@ -1574,9 +1547,9 @@ static int preload_iteration_kernels()
     WR_PRELOAD(k_rank_finish_prefix); WR_PRELOAD(k_best_copy_peer); WR_PRELOAD(k_best_copy); WR_PRELOAD(k_rankset_gen); WR_PRELOAD(k_rankset_publish);
     WR_PRELOAD(k_rankset_merge); WR_PRELOAD(k_evaporate_tiles); WR_PRELOAD(k_rankset_apply); WR_PRELOAD(k_rankset_clear); WR_PRELOAD(k_deposit_serial);
     WR_PRELOAD((k_deposit_gen<false, true>)); WR_PRELOAD(k_tile_offsets); WR_PRELOAD(k_update_fused<true>); WR_PRELOAD(k_update_fused<false>);
-    WR_PRELOAD(k_pull_finals); WR_PRELOAD(k_iter_begin); WR_PRELOAD(k_iter_end); WR_PRELOAD(k_path_warm); WR_PRELOAD(k_rankset_warm);
+    WR_PRELOAD(k_pull_finals); WR_PRELOAD(k_iter_begin); WR_PRELOAD(k_iter_end);
     WR_PRELOAD((k_walk3<true, 0>)); WR_PRELOAD((k_walk3<true, 1>)); WR_PRELOAD((k_walk3<false, 0>)); WR_PRELOAD((k_walk3<false, 1>));
-    WR_PRELOAD((k_walk2<true>)); WR_PRELOAD((k_walk2<false>));
+    WR_PRELOAD((k_walk2<Dense6, true>)); WR_PRELOAD((k_walk2<Dense6, false>));
 #undef WR_PRELOAD
     int rc = sort_preload();
     if (rc != WR_OK) return rc;

@@ -55,12 +55,11 @@ struct WalkArgs {
     int* ant_steps;          // [chunk]  steps, -1 dead, -2 pending (table overflow -> pass 2)
     uint32_t* path_ids;      // [chunk][cap]   node the ant stood on before step i
     uint8_t* path_dirs;      // [chunk][cap]   slot chosen at step i
-    int table_log2;          // k_walk26: shared-memory (pass 1) or global (pass 2) visited-tile table size
+    int table_log2;          // K = 26: shared-memory visited-tile table size of pass 1 (pass 2's HBM tables have 1 << gtable_log2)
     int table_entries;       // k_walk2: shared-memory visited-tile entries per ant (any size; the HBM tables of pass 2 have 1 << gtable_log2)
     uint32_t* overflow_list; // [chunk]
-    uint32_t* gkeys;         // HBM visited tables, one per overflowed ant: [chunk][1 << gtable_log2]
-    unsigned long long* gmasks;
-    unsigned long long* gtab;   // k_walk2: HBM visited tables of 64-bit entries (aliases gmasks)
+    uint32_t* gkeys;         // K = 26: tile keys of the HBM visited tables, one per overflowed ant: [chunk][1 << gtable_log2]
+    unsigned long long* gtab;   // HBM visited tables: K = 6 64-bit key|mask entries, K = 26 the masks beside gkeys
     int gtable_log2;
     int4* resume;            // [chunk] state of an overflowed ant: {cur, steps, ntiles, bits of L (K = 26)}
     float precision;         // K = 26 (walk26.cuh): step lengths precision, precision*1.414f, precision*1.732f
@@ -201,6 +200,17 @@ __device__ __noinline__ float slow_norm1(float d) { return __fsqrt_rn(__fmul_rn(
 
 constexpr float kClosedSlot = -1.0f;   // heur value of a slot whose neighbour is out of bounds or occupied (a real factor is >= 1 - beta or NaN)
 
+// The factor of one slot: ac = the goal vector's component along the slot's axis, d = neighbour minus node on that axis,
+// na = |goal - node|.  k_heuristic tabulates it, Batch6 (batch.cuh) evaluates it per step: one function, so the two
+// cannot drift apart.
+__device__ __forceinline__ float heur6(float ac, float d, float na, float beta)
+{
+    float nb = fabsf(d);
+    if (!(nb >= 1e-18f && nb <= 1e18f) && nb != 0.0f) nb = slow_norm1(d);
+    const float cosv = __fdiv_rn(__fmul_rn(ac, d), __fmul_rn(na, nb));
+    return __fadd_rn(1.0f, __fmul_rn(beta, cosv));
+}
+
 __global__ void __launch_bounds__(256) k_heuristic(float* __restrict__ heur, const float* __restrict__ coords, const uint32_t* __restrict__ occ_bits,
                                                     int rx, int ry, int rz, unsigned long long N, int goal, float beta)
 {
@@ -228,10 +238,7 @@ __global__ void __launch_bounds__(256) k_heuristic(float* __restrict__ heur, con
         if (open) {
             const float ac = dx ? ax : (dy ? ay : az);
             const float d = dx ? __fsub_rn(xs[nx], cx) : (dy ? __fsub_rn(ys[ny], cy) : __fsub_rn(zs[nz], cz));
-            float nb = fabsf(d);
-            if (!(nb >= 1e-18f && nb <= 1e18f) && nb != 0.0f) nb = slow_norm1(d);
-            const float cosv = __fdiv_rn(__fmul_rn(ac, d), __fmul_rn(na, nb));
-            v = __fadd_rn(1.0f, __fmul_rn(beta, cosv));
+            v = heur6(ac, d, na, beta);
         }
         h[k] = v;
     }
@@ -644,10 +651,10 @@ __global__ void k_save_result(const IterState* st, const int* __restrict__ best_
 // Sharded colonies, owner-computes: rank r applied the deposits of its slot slice and listed the final values
 // (k_update_fused<true>); every other rank pulls that list straight out of r's HBM over NVLink (peer pointers) and
 // overwrites its own, so far only evaporated, copy.  bufs[p]: word 0 = count, records (slot, value bits) from word 4.
-// The same pass is the next walk's L2 warm-up (cf. k_path_warm): the slots that just received deposits are where the
-// colony walks next, so the tau lines are left dirty in L2 by the writes and the heuristic rows are touched here.
-__global__ void __launch_bounds__(256) k_pull_finals(PeerBarrier pb, const IterState* st, float* tau, const float* __restrict__ heur,
-                                                      const uint32_t* const* __restrict__ bufs, int npeers, int me, uint8_t* dirty, uint32_t* upd_q)
+// The same pass is the next walk's L2 warm-up: the slots that just received deposits are where the colony walks next, so
+// the tau lines are left in L2 — the other ranks' by the writes, this rank's own slice by a touch.
+__global__ void __launch_bounds__(256) k_pull_finals(PeerBarrier pb, const IterState* st, float* tau, const uint32_t* const* __restrict__ bufs, int npeers,
+                                                      int me, uint8_t* dirty, uint32_t* upd_q)
 {
     peer_barrier(pb, st, 2u);   // every rank's list of final values is complete
     uint32_t acc = 0;
@@ -664,7 +671,6 @@ __global__ void __launch_bounds__(256) k_pull_finals(PeerBarrier pb, const IterS
             const uint2 r = __ldcg(rec + i);
             if (p != me) { tau[r.x] = __uint_as_float(r.y); dirty[r.x / (uint32_t)kUpdTile] = 1; }
             else acc ^= __ldcg(reinterpret_cast<const uint32_t*>(tau) + r.x);
-            if (heur) acc ^= __ldcg(reinterpret_cast<const uint32_t*>(heur) + r.x);
         }
     }
     if (acc == 0x9E3779B9u && npeers < 0) tau[0] = 0.0f;   // keeps the warm-up loads alive; never true

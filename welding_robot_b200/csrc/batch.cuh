@@ -4,14 +4,15 @@
 // thousands of searches advance in lockstep, one launch per phase covering every (query, ant):
 //
 //   k_batch_iter_begin   colony size, lambda, Q of every query (:247-249)
-//   k_walk_batch         K2 over (query, 4-ant group) work items — the walk of walk2.cuh with two differences forced by
-//                        memory: 1024 dense pheromone + heuristic fields would need 800 MB (256^3) to 6.4 GB (512^3) EACH, so
+//   k_walk_batch3        K2 over (query, 4-ant group) work items, pass 1; pass 2 (parked ants) is k_walk2<Batch6>.  The step
+//                        is walk2.cuh's with two differences forced by memory — 1024 dense pheromone + heuristic fields would
+//                        need 800 MB (256^3) to 6.4 GB (512^3) EACH — both behind the input type Batch6:
 //                          * pheromone lives in ONE hash table for the whole batch, keyed by (query, node): an entry holds the
 //                            node's six directed slots (32 B = one sector, read by the ant's six lanes in one request); a node
 //                            without an entry has never received a deposit and is worth the scalar `base` — the clean-tile
 //                            argument of acs_kernels.cuh at node granularity, bit-exact for the same reason;
-//                          * the geometric factor 1 + beta*cos is computed per step from the three axis tables (the same
-//                            expressions, in the same order, as k_heuristic) while the pheromone gather is in flight, and
+//                          * the geometric factor 1 + beta*cos is computed per step from the three axis tables (heur6, the
+//                            function k_heuristic tabulates) while the pheromone gather is in flight, and
 //                            the open-neighbour mask comes from the grid's one byte per node (grid.cu k_open6);
 //   k_batch_rank         one CTA per query: stable sort by (steps, ant), best decision (:263-264), eligibility (:200), new
 //                        best path and its node-membership flags (isOnBestPath, :209)
@@ -22,7 +23,7 @@
 // Every query draws from its own Philox search index (wr_common.cuh), so a batch equals the same searches run one after
 // the other through wr_acs_search_pairs bit for bit — and those equal the oracle's.
 // K = 26 (batch26.cuh) shares the table code — templated on the entry's words EW, so the K = 6 kernels keep a constant
-// stride — with a 128-byte entry, ranking by the bits of L and deposits with the ant's own L; only the walk is its own kernel.
+// stride — with a 128-byte entry, ranking by the bits of L and deposits with the ant's own L; its walk is k_walk26<Batch26>.
 #pragma once
 #include "rank_small.cuh"
 #include "walk2.cuh"
@@ -129,6 +130,104 @@ struct BatchArgs {
     float* ant_L;             // [nq][colony_max] length of every ant, +inf if it died
 };
 
+// Inputs of a K = 6 walk over a batch: k_walk_batch3 (pass 1) and k_walk2<Batch6> (pass 2, the parked ants).
+//   * tau: the node's (query, node) entry, or the scalar if it has none;
+//   * the geometric factor: heur6 from the three axis tables, per step;
+//   * open: the grid's one byte per node (grid.cu k_open6).
+// issue() sends the loads of a step (first probe of the entry, open byte, coordinates) out as soon as the node is known,
+// resolve() finishes them when the step needs them.
+struct Batch6 {
+    using Args = BatchArgs;
+    // this lane
+    int k, kk6;
+    int axis_k, dk, axis_len;         // axis of the slot: 0 = x (slots 2, 3), 1 = y (slots 1, 4), 2 = z (slots 0, 5); -1 / +1 along it (0 for the idle lanes)
+    const float *xs, *ys, *zs, *axis_tab;
+    const uint32_t* ent;
+    const uint8_t* open6;
+    int shift;
+    uint32_t tmask;
+    float beta;
+    int rx, rxy;
+    // the bound query and ant
+    uint32_t qi, qhash;
+    float gxv, gyv, gzv;              // goal coordinates (vector_a = goal - node, :151)
+    int start, goal;
+    uint32_t ant, stream_word, block_hi;
+    size_t row;
+    // the current step
+    uint32_t want0, eh, etau, omask;
+    uint2 ekey;
+    float cxv, cyv, czv, nbv;
+
+    __device__ __forceinline__ Batch6(const BatchArgs& a, int k_)
+        : k(k_), kk6(k_ < 6 ? k_ : 5), ent(a.tab.ent), open6(a.open6), shift(a.tab.shift), tmask(a.tab.tmask), beta(a.beta), rx(a.rx), rxy(a.rx * a.ry)
+    {
+        const int dxk = (k == 3) - (k == 2), dyk = (k == 4) - (k == 1), dzk = (k == 5) - (k == 0);
+        axis_k = (k == 2 || k == 3) ? 0 : ((k == 1 || k == 4) ? 1 : 2);
+        dk = dxk + dyk + dzk;
+        xs = a.coords;
+        ys = xs + a.rx;
+        zs = ys + a.ry;
+        axis_tab = axis_k == 0 ? xs : (axis_k == 1 ? ys : zs);
+        axis_len = axis_k == 0 ? a.rx : (axis_k == 1 ? a.ry : a.rz);
+    }
+    __device__ __forceinline__ const BatchQuery& query(const BatchArgs& a, uint32_t q)
+    {
+        qi = q;
+        qhash = q * 0x85EBCA6Bu + (q << 13);
+        const BatchQuery& bq = a.qs[q];
+        const int g = bq.goal;
+        gxv = __ldg(xs + g % rx); gyv = __ldg(ys + (g % rxy) / rx); gzv = __ldg(zs + g / rxy);
+        return bq;
+    }
+    // entry q of the parked-ant list (has = false: no ant, the group idles)
+    __device__ __forceinline__ void bind(const BatchArgs& a, unsigned q, bool has)
+    {
+        const uint32_t ga = has ? a.overflow_list[q] : 0u;   // query * colony_max + ant
+        const uint32_t qq = ga / (uint32_t)a.colony_max;
+        ant = ga - qq * (uint32_t)a.colony_max;
+        const BatchQuery& bq = query(a, qq);
+        start = bq.start; goal = bq.goal;
+        stream_word = bq.stream_word; block_hi = bq.block_hi;
+        row = (size_t)qq * a.colony_max + ant;
+    }
+    __device__ __forceinline__ void issue(int cur, uint32_t P)
+    {
+        want0 = (uint32_t)cur + 1u;
+        eh = (((uint32_t)cur * 2654435761u) ^ qhash) >> shift;
+        const uint32_t* e = ent + (size_t)eh * kBatchEntryWords;
+        ekey = __ldg(reinterpret_cast<const uint2*>(e));
+        etau = __ldg(e + 2 + kk6);
+        omask = (uint32_t)__ldg(open6 + cur);
+        const int x = (int)(P & 1023u), y = (int)((P >> 10) & 1023u), z = (int)((P >> 20) & 1023u);   // bits 30-31 may carry a key tag
+        cxv = __ldg(xs + x); cyv = __ldg(ys + y); czv = __ldg(zs + z);
+        const int ci = (axis_k == 0 ? x : (axis_k == 1 ? y : z)) + dk;
+        nbv = __ldg(axis_tab + min(max(ci, 0), axis_len - 1));
+    }
+    __device__ __forceinline__ Slot6 resolve()
+    {
+        Slot6 s;
+        s.open = k < 6 && ((omask >> k) & 1u);
+        // ---- geometric factor of slot k, k_heuristic's expressions ----
+        const float ax = __fsub_rn(gxv, cxv), ay = __fsub_rn(gyv, cyv), az = __fsub_rn(gzv, czv);
+        const float na = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay)), __fmul_rn(az, az)));
+        const float cc = axis_k == 0 ? cxv : (axis_k == 1 ? cyv : czv);
+        const float ac = axis_k == 0 ? ax : (axis_k == 1 ? ay : az);
+        s.heur = heur6(ac, __fsub_rn(nbv, cc), na, beta);
+        // ---- pheromone of slot k: the node's entry, or the scalar if it has none ----
+        uint32_t probes = 0;
+        while ((ekey.x != want0 || (ekey.y & 0x7FFFFFFFu) != qi) && (ekey.x | ekey.y) != 0u) {   // rare: linear probing at load <= 1/2
+            if (++probes > tmask) { ekey = make_uint2(0u, 0u); break; }   // a full table: only in a batch that has already failed and will be re-run
+            eh = (eh + 1) & tmask;
+            const uint32_t* e = ent + (size_t)eh * kBatchEntryWords;
+            ekey = __ldg(reinterpret_cast<const uint2*>(e));
+            etau = __ldg(e + 2 + kk6);
+        }
+        s.tau = (ekey.x | ekey.y) != 0u ? __uint_as_float(etau) : __uint_as_float(kSentinelBits);
+        return s;
+    }
+};
+
 template <int EW>
 __global__ void k_batch_fill(uint4* __restrict__ ent4, size_t n_entries)
 {   // keys 0, every slot (and the unused words of a K = 26 entry) the sentinel
@@ -192,223 +291,12 @@ __global__ void k_batch_iter_begin(IterState* st, BatchQuery* qs, int nq, int fi
 }
 
 // ------------------------------------------------------------------------------------------
-// K2 over a batch, pass 2: the ants that pass 1 (k_walk_batch3 below) parked on a full shared-memory table, resumed with their
-// HBM tables from the pool.  See walk2.cuh for the step itself; differences are marked BATCH.
-// ------------------------------------------------------------------------------------------
-template <bool ALPHA1>
-__global__ void __launch_bounds__(kWalkThreads) k_walk_batch(BatchArgs a)
-{
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    int4* move_lut = reinterpret_cast<int4*>(smem_raw);
-    if (threadIdx.x < 64) {
-        const int pbv = threadIdx.x;
-        const int c = pbv ? 31 - __clz(pbv) : 0;
-        const int dx = (c == 3) - (c == 2), dy = (c == 4) - (c == 1), dz = (c == 5) - (c == 0);
-        move_lut[pbv] = pbv ? make_int4(dx + dy * a.rx + dz * a.rx * a.ry, dx + dy * 1024 + dz * 1048576, c, 0) : make_int4(0, 0, 0, 0);
-    }
-    __syncthreads();
-
-    constexpr unsigned FULL = 0xffffffffu;
-    const int lane = threadIdx.x & 31;
-    const int gbase = lane & 24;
-    const int k = lane & 7;
-    const int E = 1 << a.gtable_log2;
-    uint32_t lut_sa = (uint32_t)__cvta_generic_to_shared(move_lut);
-    TabRef<true> tab;
-    tab.gp = a.gtab;
-    tab.sa = 0;
-    asm volatile("" : "+r"(lut_sa));
-
-    const int rx = a.rx, rxy = a.rx * a.ry;
-    const int dxk = (k == 3) - (k == 2), dyk = (k == 4) - (k == 1), dzk = (k == 5) - (k == 0);
-    const uint32_t dPk = (uint32_t)(dxk + dyk * 1024 + dzk * 1048576);
-    const int kk6 = k < 6 ? k : 5;
-    // BATCH: this lane's axis for the geometric factor: 0 = x (slots 2, 3), 1 = y (slots 1, 4), 2 = z (slots 0, 5)
-    const int axis_k = (k == 2 || k == 3) ? 0 : ((k == 1 || k == 4) ? 1 : 2);
-    const int dk = dxk + dyk + dzk;   // -1 / +1 along that axis (0 for the idle lanes)
-    const float* xs = a.coords;
-    const float* ys = xs + a.rx;
-    const float* zs = ys + a.ry;
-    const float* axis_tab = axis_k == 0 ? xs : (axis_k == 1 ? ys : zs);
-    const int axis_len = axis_k == 0 ? a.rx : (axis_k == 1 ? a.ry : a.rz);
-    uint32_t m4 = k <= 4 ? ~0u : 0u, m3 = k <= 3 ? ~0u : 0u, m2 = k <= 2 ? ~0u : 0u, m1 = k <= 1 ? ~0u : 0u, m0 = k <= 0 ? ~0u : 0u;
-    asm volatile("" : "+r"(m4), "+r"(m3), "+r"(m2), "+r"(m1), "+r"(m0));
-
-    IterState* st = a.st;
-    const uint32_t iter = (uint32_t)st->iter;
-    const float base_now = st->base;
-    const float beta = a.beta;
-    const unsigned n_items = st->overflow_n;   // the ants pass 1 parked
-    const int cap = a.cap;
-    const uint32_t* ent = a.tab.ent;
-
-    unsigned long long c_steps = 0, c_ants = 0, c_arrived = 0, c_nocand = 0, c_fall = 0, c_cap = 0;
-
-    while (true) {
-        unsigned q0 = 0;
-        if (lane == 0) q0 = atomicAdd(&st->queue2, 4u);
-        q0 = __shfl_sync(FULL, q0, 0);
-        if (q0 >= n_items) break;                                    // warp-uniform
-        // BATCH: four parked ants of any queries
-        const unsigned slot_o = q0 + (unsigned)(lane >> 3);
-        const bool has = slot_o < n_items;
-        const uint32_t ga = has ? a.overflow_list[slot_o] : 0u;
-        const uint32_t qi = ga / (uint32_t)a.colony_max;
-        const int ant = (int)(ga - qi * (uint32_t)a.colony_max);
-        const BatchQuery& bq = a.qs[qi];
-        const int start = bq.start, goal = bq.goal;
-        const uint32_t stream_word = bq.stream_word, block_hi = bq.block_hi;
-        const uint32_t qhash = qi * 0x85EBCA6Bu + (qi << 13);
-        // goal coordinates (vector_a = goal - node, :151)
-        const float gxv = __ldg(xs + goal % rx), gyv = __ldg(ys + (goal % rxy) / rx), gzv = __ldg(zs + goal / rxy);
-
-        int cur = start, steps = 0;
-        uint32_t P = pack_xyz(start % rx, (start % rxy) / rx, start / rxy);
-        float u0 = 0.f, u1 = 0.f, u2 = 0.f, u3 = 0.f;
-        auto draw4 = [&](uint32_t block) {
-            uint32_t w0, w1, w2, w3;
-            philox4(iter, (uint32_t)ant, block | block_hi, stream_word, a.seed_lo, a.seed_hi, w0, w1, w2, w3);
-            u0 = __fmul_rn(__int2float_rn((int)(w0 >> 1)), 4.656612873077392578125e-10f);
-            u1 = __fmul_rn(__int2float_rn((int)(w1 >> 1)), 4.656612873077392578125e-10f);
-            u2 = __fmul_rn(__int2float_rn((int)(w2 >> 1)), 4.656612873077392578125e-10f);
-            u3 = __fmul_rn(__int2float_rn((int)(w3 >> 1)), 4.656612873077392578125e-10f);
-        };
-        tab.gp = a.gtab + (size_t)(has ? slot_o : 0) * E;
-        if (has) {   // resume: the visited set already lives in HBM table slot_o
-            const int4 r = a.resume[slot_o];
-            cur = r.x; steps = r.y;
-            P = pack_xyz(cur % rx, (cur % rxy) / rx, cur / rxy);
-            draw4((uint32_t)steps >> 2);
-        }
-        __syncwarp();
-
-        bool live = has;
-        int result = -1, reason = 0;
-        if (live && steps >= cap) { live = false; reason = 3; }
-        const size_t ant_row = ((size_t)qi * a.colony_max + (size_t)(has ? ant : 0)) * cap;
-        uint32_t* pid = a.path_ids + ant_row;
-        uint8_t* pdir = a.path_dirs + ant_row;
-
-        // BATCH: the loads of a step — pheromone entry (first probe), open mask, coordinates — go out as soon as the node is known
-        uint32_t want0, eh; uint2 ekey; uint32_t etau; uint32_t omask; float cxv, cyv, czv, nbv;
-        auto issue_loads = [&]() {
-            want0 = (uint32_t)cur + 1u;
-            eh = (((uint32_t)cur * 2654435761u) ^ qhash) >> a.tab.shift;
-            const uint32_t* e = ent + (size_t)eh * kBatchEntryWords;
-            ekey = __ldg(reinterpret_cast<const uint2*>(e));
-            etau = __ldg(e + 2 + kk6);
-            omask = (uint32_t)__ldg(a.open6 + cur);
-            const int x = (int)(P & 1023u), y = (int)((P >> 10) & 1023u), z = (int)(P >> 20);
-            cxv = __ldg(xs + x); cyv = __ldg(ys + y); czv = __ldg(zs + z);
-            const int ci = (axis_k == 0 ? x : (axis_k == 1 ? y : z)) + dk;
-            nbv = __ldg(axis_tab + min(max(ci, 0), axis_len - 1));
-        };
-        issue_loads();
-
-        auto step = [&]() {
-            if (live && (steps & 3) == 0) draw4((uint32_t)steps >> 2);
-            const float u = (steps & 2) ? ((steps & 1) ? u3 : u2) : ((steps & 1) ? u1 : u0);
-            // ---- BATCH: geometric factor of slot k, k_heuristic's expressions ----------------------------------------
-            const bool open_k = k < 6 && ((omask >> k) & 1u);
-            const float ax = __fsub_rn(gxv, cxv), ay = __fsub_rn(gyv, cyv), az = __fsub_rn(gzv, czv);
-            const float na = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay)), __fmul_rn(az, az)));
-            const float cc = axis_k == 0 ? cxv : (axis_k == 1 ? cyv : czv);
-            const float ac = axis_k == 0 ? ax : (axis_k == 1 ? ay : az);
-            const float d = __fsub_rn(nbv, cc);
-            float nb = fabsf(d);
-            if (!(nb >= 1e-18f && nb <= 1e18f) && nb != 0.0f) nb = slow_norm1(d);
-            const float heur_v = __fadd_rn(1.0f, __fmul_rn(beta, __fdiv_rn(__fmul_rn(ac, d), __fmul_rn(na, nb))));
-            // ---- BATCH: pheromone of slot k: the node's entry, or the scalar if it has none ---------------------------
-            uint32_t probes = 0;
-            while ((ekey.x != want0 || (ekey.y & 0x7FFFFFFFu) != qi) && (ekey.x | ekey.y) != 0u) {   // rare: linear probing at load <= 1/2
-                if (++probes > a.tab.tmask) { ekey = make_uint2(0u, 0u); break; }   // a full table: only in a batch that has already failed and will be re-run
-                eh = (eh + 1) & a.tab.tmask;
-                const uint32_t* e = ent + (size_t)eh * kBatchEntryWords;
-                ekey = __ldg(reinterpret_cast<const uint2*>(e));
-                etau = __ldg(e + 2 + kk6);
-            }
-            const float tau_v = (ekey.x | ekey.y) != 0u ? __uint_as_float(etau) : __uint_as_float(kSentinelBits);
-            // ---- neighbour k: tabu probe ------------------------------------------------------------------------------
-            const uint32_t Pk = P + dPk;
-            const uint32_t key = (Pk & kPackKey) | kKeyTag;
-            const uint32_t bitm = 1u << ((((Pk & kPackLow) * kPackMul) >> 20) & 31u);
-            unsigned slot = tile_hash(key, (uint32_t)E);
-            unsigned long long e = tab.load(slot);
-            while (open_k && (uint32_t)(e >> 32) != key && (uint32_t)(e >> 32) != 0u) {
-                slot = slot + 1 < (unsigned)E ? slot + 1 : 0u;
-                e = tab.load(slot);
-            }
-            const bool found = (uint32_t)(e >> 32) == key;
-            const uint32_t emask = found ? (uint32_t)e : 0u;
-            const bool cand = live && open_k && !(emask & bitm);
-            const float tau_now = tau_or_base(tau_v, base_now);
-            const float tpow = ALPHA1 ? tau_now : pow_int(tau_now, a.alpha);
-            const float info = cand ? __fmul_rn(tpow, heur_v) : 0.0f;
-            // ---- roulette in the reference's order (:155, :172-181) --------------------------------------------------
-            const unsigned cb = (__ballot_sync(FULL, cand) >> gbase) & 0x3Fu;
-            const float v0 = __shfl_sync(FULL, info, 0, 8), v1 = __shfl_sync(FULL, info, 1, 8), v2 = __shfl_sync(FULL, info, 2, 8);
-            const float v3 = __shfl_sync(FULL, info, 3, 8), v4 = __shfl_sync(FULL, info, 4, 8), v5 = __shfl_sync(FULL, info, 5, 8);
-            const float total = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(0.0f, v0), v1), v2), v3), v4), v5);
-            const float rnd = __fmul_rn(u, total);
-            float mine = __fadd_rn(0.0f, v5);
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v4) & m4));
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v3) & m3));
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v2) & m2));
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v1) & m1));
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v0) & m0));
-            const bool pick = cand && (mine >= rnd);
-            const unsigned pb = (__ballot_sync(FULL, pick) >> gbase) & 0x3Fu;
-            int4 mv;
-            asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(mv.x), "=r"(mv.y), "=r"(mv.z), "=r"(mv.w) : "r"(lut_sa + pb * 16u) : "memory");
-            const int c = mv.z;
-            const bool stepok = live && pb != 0;
-            const int prev = cur, at = steps;
-            if (stepok) { cur += mv.x; P += (uint32_t)mv.y; steps++; }
-            issue_loads();
-            if (live && !stepok) reason = cb == 0 ? 1 : 2;
-            if (stepok && k == c) {
-                tab.store(slot, ((unsigned long long)key << 32) | (unsigned long long)(emask | bitm));
-                pid[at] = (uint32_t)prev;
-                pdir[at] = (uint8_t)c;
-            }
-            const bool arrived = stepok && cur == goal;
-            const bool capped = stepok && !arrived && steps >= cap;
-            result = arrived ? steps : result;
-            reason = capped ? 3 : reason;
-            live = stepok && !arrived && !capped;
-            __syncwarp();
-        };
-        while (__any_sync(FULL, live)) {
-            step();
-            step();
-        }
-        if (has) {
-            c_arrived += result >= 0 ? 1 : 0;
-            c_nocand += (result < 0 && reason == 1) ? 1 : 0;
-            c_fall += (result < 0 && reason == 2) ? 1 : 0;
-            c_cap += (result < 0 && reason == 3) ? 1 : 0;
-            c_steps += (unsigned long long)steps; c_ants++;
-            if (k == 0) a.ant_steps[(size_t)qi * a.colony_max + ant] = result;
-        }
-        __syncwarp();
-    }
-    if (k == 0) {
-        if (c_steps) atomicAdd(&st->cnt[0], c_steps);
-        if (c_ants) atomicAdd(&st->cnt[1], c_ants);
-        if (c_arrived) atomicAdd(&st->cnt[2], c_arrived);
-        if (c_nocand) atomicAdd(&st->cnt[3], c_nocand);
-        if (c_fall) atomicAdd(&st->cnt[4], c_fall);
-        if (c_cap) atomicAdd(&st->cnt[5], c_cap);
-    }
-}
-
-// ------------------------------------------------------------------------------------------
 // Pass 1 of K2 over a batch, restructured like k_walk3 (walk3.cuh): the four ants of a warp are at the same step index, so
 // four steps per trip with the draw chosen at compile time, Philox for the next four steps computed in slices beside them, the
 // trail kept in registers and written eight steps at a time, the visited insert a predicated store by the lane whose pick is
-// the highest, the tile count fed by one vote, outcomes reconstructed after the loop.  The step's arithmetic — pheromone entry
-// or scalar, geometric factor, roulette — is k_walk_batch's, so every ant is bit-identical; pass 2 (parked ants) stays
-// k_walk_batch<GLOBAL = true>.  This kernel is issue-bound once a few hundred queries are in flight (60 % of the issue
+// the highest, the tile count fed by one vote, outcomes reconstructed after the loop.  Its inputs — pheromone entry or scalar,
+// geometric factor, open mask — come from Batch6, as in pass 2 (k_walk2<Batch6>, parked ants), so every ant is bit-identical.
+// This kernel is issue-bound once a few hundred queries are in flight (60 % of the issue
 // slots), so the shorter instruction stream is throughput.
 // ------------------------------------------------------------------------------------------
 // Register allocation bounded for five CTAs per SM (102 registers): measured best on C5 — 2027 queries/s, against 1934 with six
@@ -444,14 +332,7 @@ __global__ void __launch_bounds__(kWalkThreads, 5) k_walk_batch3(BatchArgs a)
     const int rx = a.rx, rxy = a.rx * a.ry;
     const int dxk = (k == 3) - (k == 2), dyk = (k == 4) - (k == 1), dzk = (k == 5) - (k == 0);
     const uint32_t dPk = (uint32_t)(dxk + dyk * 1024 + dzk * 1048576);
-    const int kk6 = k < 6 ? k : 5;
-    const int axis_k = (k == 2 || k == 3) ? 0 : ((k == 1 || k == 4) ? 1 : 2);
-    const int dk = dxk + dyk + dzk;
-    const float* xs = a.coords;
-    const float* ys = xs + a.rx;
-    const float* zs = ys + a.ry;
-    const float* axis_tab = axis_k == 0 ? xs : (axis_k == 1 ? ys : zs);
-    const int axis_len = axis_k == 0 ? a.rx : (axis_k == 1 ? a.ry : a.rz);
+    Batch6 in(a, k);
     uint32_t m4 = k <= 4 ? ~0u : 0u, m3 = k <= 3 ? ~0u : 0u, m2 = k <= 2 ? ~0u : 0u, m1 = k <= 1 ? ~0u : 0u, m0 = k <= 0 ? ~0u : 0u;
     asm volatile("" : "+r"(m4), "+r"(m3), "+r"(m2), "+r"(m1), "+r"(m0));
     constexpr uint32_t kKeyMask = kPackKey | kKeyTag;
@@ -459,13 +340,11 @@ __global__ void __launch_bounds__(kWalkThreads, 5) k_walk_batch3(BatchArgs a)
     IterState* st = a.st;
     const uint32_t iter = (uint32_t)st->iter;
     const float base_now = st->base;
-    const float beta = a.beta;
     const unsigned n_items = (unsigned)(a.nq * a.items_per_query);
     const uint32_t limit = (uint32_t)((E >> 2) * 3);
     const int cap = a.cap;
     int cap_k = k < 6 ? cap : 0;   // the two idle lanes of a group are never alive
     asm volatile("" : "+r"(cap_k));
-    const uint32_t* ent = a.tab.ent;
 
     unsigned long long c_steps = 0, c_ants = 0, c_arrived = 0, c_nocand = 0, c_fall = 0, c_cap = 0, c_over = 0;
 
@@ -476,12 +355,10 @@ __global__ void __launch_bounds__(kWalkThreads, 5) k_walk_batch3(BatchArgs a)
         if (q0 >= n_items) break;                                    // warp-uniform
         const uint32_t qi = q0 / (unsigned)a.items_per_query;        // work item = (query, group of four ants)
         const int ant = (int)(q0 - qi * (unsigned)a.items_per_query) * 4 + (lane >> 3);
-        const BatchQuery& bq = a.qs[qi];
+        const BatchQuery& bq = in.query(a, qi);
         const bool has = ant < bq.colony;
         const int start = bq.start, goal = bq.goal;
         const uint32_t stream_word = bq.stream_word, block_hi = bq.block_hi;
-        const uint32_t qhash = qi * 0x85EBCA6Bu + (qi << 13);
-        const float gxv = __ldg(xs + goal % rx), gyv = __ldg(ys + (goal % rxy) / rx), gzv = __ldg(zs + goal / rxy);
 
         const uint32_t Pstart = pack_xyz(start % rx, (start % rxy) / rx, start / rxy) | kKeyTag;   // bit 31: the key tag rides along
         for (int i = k; i < E; i += kGroup) tab.store(i, 0ull);
@@ -516,43 +393,12 @@ __global__ void __launch_bounds__(kWalkThreads, 5) k_walk_batch3(BatchArgs a)
         uint32_t pc0 = 0, pc1 = 0, pc2 = 0, pc3 = 0;
         auto rounds = [&](auto r0, auto r1) { philox_rounds<decltype(r0)::value, decltype(r1)::value>(pc0, pc1, pc2, pc3, a.seed_lo, a.seed_hi); };
 
-        // the loads of a step — pheromone entry (first probe), open mask, coordinates — go out as soon as the node is known
-        uint32_t want0, eh; uint2 ekey; uint32_t etau; uint32_t omask; float cxv, cyv, czv, nbv;
-        auto issue_loads = [&]() {
-            want0 = (uint32_t)cur + 1u;
-            eh = (((uint32_t)cur * 2654435761u) ^ qhash) >> a.tab.shift;
-            const uint32_t* e = ent + (size_t)eh * kBatchEntryWords;
-            ekey = __ldg(reinterpret_cast<const uint2*>(e));
-            etau = __ldg(e + 2 + kk6);
-            omask = (uint32_t)__ldg(a.open6 + cur);
-            const int x = (int)(P & 1023u), y = (int)((P >> 10) & 1023u), z = (int)((P >> 20) & 1023u);
-            cxv = __ldg(xs + x); cyv = __ldg(ys + y); czv = __ldg(zs + z);
-            const int ci = (axis_k == 0 ? x : (axis_k == 1 ? y : z)) + dk;
-            nbv = __ldg(axis_tab + min(max(ci, 0), axis_len - 1));
-        };
-        issue_loads();
+        in.issue(cur, P);   // the loads of a step go out as soon as the node is known
 
         auto step = [&](const uint32_t J, const float u) {
-            // ---- geometric factor of slot k, k_heuristic's expressions -------------------------------------------------
-            const bool open_k = k < 6 && ((omask >> k) & 1u);
-            const float ax = __fsub_rn(gxv, cxv), ay = __fsub_rn(gyv, cyv), az = __fsub_rn(gzv, czv);
-            const float na = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay)), __fmul_rn(az, az)));
-            const float cc = axis_k == 0 ? cxv : (axis_k == 1 ? cyv : czv);
-            const float ac = axis_k == 0 ? ax : (axis_k == 1 ? ay : az);
-            const float d = __fsub_rn(nbv, cc);
-            float nb = fabsf(d);
-            if (!(nb >= 1e-18f && nb <= 1e18f) && nb != 0.0f) nb = slow_norm1(d);
-            const float heur_v = __fadd_rn(1.0f, __fmul_rn(beta, __fdiv_rn(__fmul_rn(ac, d), __fmul_rn(na, nb))));
-            // ---- pheromone of slot k: the node's entry, or the scalar if it has none -----------------------------------
-            uint32_t probes = 0;
-            while ((ekey.x != want0 || (ekey.y & 0x7FFFFFFFu) != qi) && (ekey.x | ekey.y) != 0u) {   // rare: linear probing at load <= 1/2
-                if (++probes > a.tab.tmask) { ekey = make_uint2(0u, 0u); break; }
-                eh = (eh + 1) & a.tab.tmask;
-                const uint32_t* e = ent + (size_t)eh * kBatchEntryWords;
-                ekey = __ldg(reinterpret_cast<const uint2*>(e));
-                etau = __ldg(e + 2 + kk6);
-            }
-            const float tau_v = (ekey.x | ekey.y) != 0u ? __uint_as_float(etau) : __uint_as_float(kSentinelBits);
+            // ---- open, factor and pheromone of slot k ------------------------------------------------------------------
+            const Slot6 sl = in.resolve();
+            const bool open_k = sl.open;
             // ---- neighbour k: tabu probe -------------------------------------------------------------------------------
             const uint32_t Pk = P + dPk;
             const uint32_t key = Pk & kKeyMask;
@@ -566,9 +412,9 @@ __global__ void __launch_bounds__(kWalkThreads, 5) k_walk_batch3(BatchArgs a)
             const bool found = (uint32_t)(e >> 32) == key;
             const uint32_t emask = found ? (uint32_t)e : 0u;
             const bool cand = live && open_k && !(emask & bitm);
-            const float tau_now = tau_or_base(tau_v, base_now);
+            const float tau_now = tau_or_base(sl.tau, base_now);
             const float tpow = ALPHA1 ? tau_now : pow_int(tau_now, a.alpha);
-            const float info = cand ? __fmul_rn(tpow, heur_v) : 0.0f;
+            const float info = cand ? __fmul_rn(tpow, sl.heur) : 0.0f;
             // ---- roulette in the reference's order (:155, :172-181) ---------------------------------------------------
             const unsigned cb = __ballot_sync(FULL, cand) & gmask;
             const float v0 = __shfl_sync(FULL, info, 0, 8), v1 = __shfl_sync(FULL, info, 1, 8), v2 = __shfl_sync(FULL, info, 2, 8);
@@ -589,7 +435,7 @@ __global__ void __launch_bounds__(kWalkThreads, 5) k_walk_batch3(BatchArgs a)
             const uint32_t prev = (uint32_t)cur;
             cur += mv.x;
             P += (uint32_t)mv.y;
-            issue_loads();
+            in.issue(cur, P);
             // ---- side effects, all predicated --------------------------------------------------------------------------
             const bool stepok = pb != 0u;
             const bool win = pick && (pb >> k) == 1u;
@@ -632,7 +478,7 @@ __global__ void __launch_bounds__(kWalkThreads, 5) k_walk_batch3(BatchArgs a)
         int reason = 0;
         if (result == -1) reason = steps >= cap ? 3 : (lastcb == 0u ? 1 : 2);
 
-        {   // park the ants whose shared-memory table filled up (see k_walk_batch); HBM tables come from a pool
+        {   // park the ants whose shared-memory table filled up (k_walk2<Batch6> resumes them); HBM tables come from a pool
             const bool pk = has && parked && !arrived;
             const unsigned pm = __ballot_sync(FULL, pk && k == 0);
             if (pm) {

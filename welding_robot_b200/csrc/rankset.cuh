@@ -39,9 +39,8 @@ struct RankSet {
     unsigned long long* key;   // [R]  slot+1 | group << 32 | onbest << 63; 0 = free
     uint32_t* rows;            // [R][32]
     uint32_t* list;            // [limit+1] blocks claimed (or merged in) this iteration
-    uint32_t* touched;         // [limit+1] their slots (written by apply, read by the next walk's L2 warm-up)
     uint32_t* count;           // [0] blocks in `list` [1] blocks of the previous rank-set iteration (0xFFFFFFFF: it overflowed) [2] always 0
-                               // [3] overflow flag [4] entries in `touched`
+                               // [3] overflow flag
     float* vtab;               // [w_max][2]  d(r, s) without / with the elitist term
     uint32_t rmask;            // R - 1
     int shift;                 // 32 - log2(R)
@@ -291,15 +290,14 @@ __global__ void __launch_bounds__(256) k_rankset_apply(const IterState* st, floa
             if (lane == 0) { tau[ss] = x; dirty[ss / (uint32_t)kUpdTile] = 1; }
         }
         __syncwarp();
-        if (has && wipe_here) {   // leave the table empty for the next iteration; remember the slot for the walk's L2 warm-up
+        if (has && wipe_here) {   // leave the table empty for the next iteration
 #pragma unroll
             for (int j = 0; j < 8; j++) reinterpret_cast<uint4*>(row)[j] = make_uint4(0u, 0u, 0u, 0u);
             rs.key[h] = 0ull;
-            if (!overflow) rs.touched[e] = slot;   // after an overflow the sweep below races with this loop: a key may already read 0
         }
     }
     if (!wipe_here) return;
-    if (blockIdx.x == 0 && threadIdx.x == 0) { rs.count[1] = overflow ? 0xFFFFFFFFu : n; rs.count[4] = overflow ? 0u : n; }   // no warm-up list after an overflow
+    if (blockIdx.x == 0 && threadIdx.x == 0) rs.count[1] = overflow ? 0xFFFFFFFFu : n;
     if (overflow) {   // blocks claimed beyond the list (their indices were dropped): a sweep of the whole table finds them
         const size_t R = (size_t)rs.rmask + 1;
         for (size_t h = (size_t)blockIdx.x * blockDim.x + threadIdx.x; h < R; h += (size_t)gridDim.x * blockDim.x) {
@@ -323,15 +321,11 @@ __global__ void __launch_bounds__(256) k_rankset_clear(const IterState* st, Rank
     const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
     for (uint32_t e = warp; e < n; e += nwarps) {   // warp per block: one coalesced 128-byte store
         const uint32_t h = rs.list[e];
-        const unsigned long long k = rs.key[h];
         rs.rows[(size_t)h * kRsRowWords + lane] = 0u;
         __syncwarp();
-        if (lane == 0) {
-            if (!overflow) rs.touched[e] = (uint32_t)k - 1u;   // after an overflow the sweep below races with this loop: k may already read 0
-            rs.key[h] = 0ull;
-        }
+        if (lane == 0) rs.key[h] = 0ull;
     }
-    if (blockIdx.x == 0 && threadIdx.x == 0) { rs.count[1] = overflow ? 0xFFFFFFFFu : n; rs.count[4] = overflow ? 0u : n; }   // no warm-up list after an overflow
+    if (blockIdx.x == 0 && threadIdx.x == 0) rs.count[1] = overflow ? 0xFFFFFFFFu : n;
     if (overflow) {
         const size_t R = (size_t)rs.rmask + 1;
         for (size_t h = (size_t)blockIdx.x * blockDim.x + threadIdx.x; h < R; h += (size_t)gridDim.x * blockDim.x) {
@@ -377,22 +371,6 @@ __global__ void __launch_bounds__(1024) k_deposit_serial(const IterState* st, co
         }
         __syncthreads();
     }
-}
-
-// L2 warm-up for the next walk from the slots that just received deposits (cf. k_path_warm, which reads the sorted records).
-__global__ void __launch_bounds__(256) k_rankset_warm(const uint32_t* __restrict__ touched, const uint32_t* __restrict__ count, const float* tau, const float* heur,
-                                                       IterState* st)
-{
-    if (!st->use_rankset) return;   // runs before k_iter_begin: the flag still describes the iteration that just ended
-    const uint32_t n = count[4];
-    uint32_t acc = 0;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const uint32_t node = touched[i] / 6u;
-        const uint32_t* pt = reinterpret_cast<const uint32_t*>(tau) + (size_t)node * 6;
-        const uint32_t* ph = reinterpret_cast<const uint32_t*>(heur) + (size_t)node * 6;
-        acc ^= __ldcg(pt) ^ __ldcg(pt + 5) ^ __ldcg(ph) ^ __ldcg(ph + 5);
-    }
-    if (acc == 0x9E3779B9u && n == 0xFFFFFFFFu) st->cnt[8] = 0;   // keeps the loads alive; never true
 }
 
 }  // namespace wr

@@ -15,7 +15,9 @@
 // ant whose shared-memory table reaches 3/4 moves its visited set to a table in HBM sized for the step cap, parks {node, steps}
 // and is RESUMED by the kernel below, k_walk2, from the very step it stopped at — exact, because its draws are a pure function
 // of (search, iteration, ant, step).  Two launches keep shared-memory addressing on the common path (a run-time switch cost
-// 8-13 % per step); pass 2 usually finds nothing to do and exits at once.
+// 8-13 % per step); pass 2 usually finds nothing to do and exits at once.  One k_walk2 serves both: its input type says where
+// tau, the factor, the open mask and the ant's identity come from — Dense6 (below) for one search, Batch6 (batch.cuh) for
+// concurrent searches.
 // (Round 1-2 history: k_walk2 also was pass 1 until k_walk3 replaced it — 164 -> 127 instructions per warp-step, see
 // profiles/r2_walk3_*; that generic form, its L1/L2 prefetch modes and the register look-ahead experiment are gone.)
 #pragma once
@@ -52,29 +54,50 @@ template <bool GLOBAL> struct TabRef {
     }
 };
 
-// L2 warm-up for the walk.  The fused update has just streamed the whole pheromone field through L2, so the rows the
-// colony is about to read are back in HBM — and a converging colony advances in lockstep over a small family of paths,
-// so every step would wait for somebody's DRAM miss.  Where the colony will walk is known: the slot-sorted deposit
-// records of the previous iteration name every node the top-ranked ants crossed.  Pull the tau and heuristic rows of
-// those nodes (each distinct node once) into L2 before the ants start: a few hundred KB, microseconds.
-// Must run BEFORE k_iter_begin (which clears n_records).
-__global__ void __launch_bounds__(256) k_path_warm(const IterState* st, const uint32_t* __restrict__ rec_keys, const float* tau, const float* heur)
-{
-    const int n = st->n_records_sort;   // 0 when the last iteration's deposits went through rank sets (k_rankset_warm covers it)
-    uint32_t acc = 0;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const uint32_t node = rec_keys[i] / 6u;
-        if (i > 0 && rec_keys[i - 1] / 6u == node) continue;
-        const uint32_t* pt = reinterpret_cast<const uint32_t*>(tau) + (size_t)node * 6;
-        const uint32_t* ph = reinterpret_cast<const uint32_t*>(heur) + (size_t)node * 6;
-        // a 24-byte row touches one or two 32-byte sectors: its first and last word cover it
-        acc ^= __ldcg(pt) ^ __ldcg(pt + 5) ^ __ldcg(ph) ^ __ldcg(ph + 5);
-    }
-    if (acc == 0x9E3779B9u && n < 0) const_cast<IterState*>(st)->cnt[8] = 0;   // keeps the loads alive; never true
-}
+// What a lane of the resume pass needs about its neighbour slot at the current node
+struct Slot6 {
+    float tau;    // as stored: the sentinel stands for the clean-field scalar
+    float heur;   // 1 + beta*cos
+    bool open;    // in bounds, free, and one of the six neighbour lanes
+};
 
-template <bool ALPHA1>
-__global__ void __launch_bounds__(kWalkThreads) k_walk2(WalkArgs a)
+// Inputs of k_walk2 for one search (WalkArgs): tau and the tabulated factor from the dense [N][6] rows
+struct Dense6 {
+    using Args = WalkArgs;
+    const float* tau_k;    // this lane's column of the tau rows; idle lanes (k = 6, 7) re-read slot 5 (same sector)
+    const float* heur_k;   // ... of the factor rows; idle lanes read a constant "closed" marker with a zero row stride, so
+    int heur_row;          //     `open` is one compare for every lane
+    int start, goal;
+    uint32_t ant, stream_word, block_hi;   // Philox counter words of the bound ant
+    size_t row;            // its row of path_ids / path_dirs / ant_steps
+    float tau_v, heur_v;   // this lane's slot of the current row
+
+    __device__ __forceinline__ Dense6(const WalkArgs& a, int k)
+        : tau_k(a.tau + (k < 6 ? k : 5)), heur_k(k < 6 ? a.heur + k : a.closed_marker), heur_row(k < 6 ? 6 : 0), start(a.start), goal(a.goal),
+          stream_word(a.stream_word), block_hi(a.block_hi)
+    {
+    }
+    // entry q of the parked-ant list (has = false: no ant, the group idles)
+    __device__ __forceinline__ void bind(const WalkArgs& a, unsigned q, bool has)
+    {
+        const int ant_local = has ? (int)a.overflow_list[q] : 0;
+        ant = (uint32_t)(a.shard_first + ant_local);
+        row = (size_t)ant_local;
+    }
+    // reloaded as soon as the next node is known, ahead of the move's side effects
+    __device__ __forceinline__ void issue(int cur, uint32_t)
+    {
+        tau_v = __ldg(tau_k + (size_t)cur * 6);
+        heur_v = __ldg(heur_k + (size_t)cur * heur_row);
+    }
+    // NaN (duplicate plane) stays open, as in the reference
+    __device__ __forceinline__ Slot6 resolve() const { return {tau_v, heur_v, heur_v != kClosedSlot}; }
+};
+
+// Pass 2: resume the ants pass 1 parked, with their visited sets in HBM tables.  In = Dense6 (one search) or Batch6
+// (concurrent searches, batch.cuh) says where tau, the factor, the open mask and the ant's identity come from.
+template <class In, bool ALPHA1>
+__global__ void __launch_bounds__(kWalkThreads) k_walk2(typename In::Args a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     // [0, 1024): move table indexed by the 6-bit pick ballot: the winner is its highest set bit c (the roulette scans
@@ -103,22 +126,16 @@ __global__ void __launch_bounds__(kWalkThreads) k_walk2(WalkArgs a)
     const int rx = a.rx, rxy = a.rx * a.ry;
     const int dxk = (k == 3) - (k == 2), dyk = (k == 4) - (k == 1), dzk = (k == 5) - (k == 0);
     const uint32_t dPk = (uint32_t)(dxk + dyk * 1024 + dzk * 1048576);
-    const int kk6 = k < 6 ? k : 5;                                             // idle lanes re-read slot 5 (same sector)
-    const float* tau_k = a.tau + kk6;
-    // idle lanes (k = 6, 7) read a constant "closed" marker with a zero row stride, so `open` is one compare for every lane
-    const float* heur_k_base = k < 6 ? a.heur + k : a.closed_marker;
-    const int heur_row = k < 6 ? 6 : 0;
+    In in(a, k);
     // lane masks of the descending prefix chain: lane k adds v_j only for j >= k
     uint32_t m4 = k <= 4 ? ~0u : 0u, m3 = k <= 3 ? ~0u : 0u, m2 = k <= 2 ? ~0u : 0u, m1 = k <= 1 ? ~0u : 0u, m0 = k <= 0 ? ~0u : 0u;
     asm volatile("" : "+r"(m4), "+r"(m3), "+r"(m2), "+r"(m1), "+r"(m0));   // keep them as register masks (one LOP3 each) instead of re-derived predicates
 
-    const uint32_t Pstart = pack_xyz(a.start % rx, (a.start % rxy) / rx, a.start / rxy);
-
     IterState* st = a.st;
     const uint32_t iter = (uint32_t)st->iter;
     const float base_now = st->base;   // clean-tile field: what a slot that never received a deposit is worth this iteration
-    const int local_n = (int)st->overflow_n;   // the ants pass 1 parked
-    const int cap = a.cap, goal = a.goal;
+    const unsigned n_items = st->overflow_n;   // the ants pass 1 parked
+    const int cap = a.cap;
 
     unsigned long long c_steps = 0, c_ants = 0, c_arrived = 0, c_nocand = 0, c_fall = 0, c_cap = 0;
 
@@ -126,18 +143,17 @@ __global__ void __launch_bounds__(kWalkThreads) k_walk2(WalkArgs a)
         unsigned q0 = 0;
         if (lane == 0) q0 = atomicAdd(&st->queue2, 4u);
         q0 = __shfl_sync(FULL, q0, 0);
-        if (q0 >= (unsigned)local_n) break;                                    // warp-uniform
+        if (q0 >= n_items) break;                                              // warp-uniform
         const unsigned q = q0 + (unsigned)(lane >> 3);
-        const bool has = q < (unsigned)local_n;
-        const int ant_local = has ? (int)a.overflow_list[q] : 0;
-        const uint32_t ant_global = (uint32_t)(a.shard_first + ant_local);
+        const bool has = q < n_items;
+        in.bind(a, q, has);
 
-        int cur = a.start, steps = 0;
-        uint32_t P = Pstart;
+        int cur = in.start, steps = 0;
+        uint32_t P = pack_xyz(cur % rx, (cur % rxy) / rx, cur / rxy);
         float u0 = 0.f, u1 = 0.f, u2 = 0.f, u3 = 0.f;
         auto draw4 = [&](uint32_t block) {
             uint32_t w0, w1, w2, w3;
-            philox4(iter, ant_global, block | a.block_hi, a.stream_word, a.seed_lo, a.seed_hi, w0, w1, w2, w3);
+            philox4(iter, in.ant, block | in.block_hi, in.stream_word, a.seed_lo, a.seed_hi, w0, w1, w2, w3);
             // (float)rand()/(float)RAND_MAX (:169): (float)RAND_MAX is 2^31, so the division is an exact scaling
             u0 = __fmul_rn(__int2float_rn((int)(w0 >> 1)), 4.656612873077392578125e-10f);
             u1 = __fmul_rn(__int2float_rn((int)(w1 >> 1)), 4.656612873077392578125e-10f);
@@ -158,22 +174,20 @@ __global__ void __launch_bounds__(kWalkThreads) k_walk2(WalkArgs a)
         int result = -1;   // >= 0: steps of an ant that arrived, -1: dead, -2: parked (table 3/4 full -> pass 2)
         int reason = 0;    // why a dead ant died: 1 no candidate, 2 roulette fall-through, 3 step cap
         if (live && steps >= cap) { live = false; reason = 3; }
-        uint32_t* pid = a.path_ids + (size_t)ant_local * cap;
-        uint8_t* pdir = a.path_dirs + (size_t)ant_local * cap;
-
-        // this lane's slot of the current row; reloaded as soon as the next node is known, ahead of the move's side effects
-        float tau_v = __ldg(tau_k + (size_t)cur * 6);
-        float heur_v = __ldg(heur_k_base + (size_t)cur * heur_row);
+        uint32_t* pid = a.path_ids + in.row * cap;
+        uint8_t* pdir = a.path_dirs + in.row * cap;
+        in.issue(cur, P);
 
         auto step = [&]() {
             // ---- Philox: one call yields the draws of 4 consecutive steps (live ants of a warp are in lockstep) ----
             if (live && (steps & 3) == 0) draw4((uint32_t)steps >> 2);
             const float u = (steps & 2) ? ((steps & 1) ? u3 : u2) : ((steps & 1) ? u1 : u0);
-            // ---- neighbour k: open (in bounds + free, folded into the heuristic table), tabu probe ------------------
+            // ---- neighbour k: open, tau, factor, tabu probe -----------------------------------------------------------
+            const Slot6 sl = in.resolve();
+            const bool open_k = sl.open;
             const uint32_t Pk = P + dPk;
             const uint32_t key = (Pk & kPackKey) | kKeyTag;
             const uint32_t bitm = 1u << ((((Pk & kPackLow) * kPackMul) >> 20) & 31u);
-            const bool open_k = heur_v != kClosedSlot;   // NaN (duplicate plane) stays open, as in the reference; idle lanes read the marker
             unsigned slot = tile_hash(key, (uint32_t)E);
             unsigned long long e = tab.load(slot);
             while (open_k && (uint32_t)(e >> 32) != key && (uint32_t)(e >> 32) != 0u) {   // collisions are rare at load <= 3/4
@@ -183,10 +197,10 @@ __global__ void __launch_bounds__(kWalkThreads) k_walk2(WalkArgs a)
             const bool found = (uint32_t)(e >> 32) == key;
             const uint32_t emask = found ? (uint32_t)e : 0u;
             const bool cand = live && open_k && !(emask & bitm);
-            // ---- info = tau^alpha * (1 + beta*cos)  (:151-154; the factor is tabulated by k_heuristic) --------------
-            const float tau_now = tau_or_base(tau_v, base_now);
+            // ---- info = tau^alpha * (1 + beta*cos)  (:151-154) -------------------------------------------------------
+            const float tau_now = tau_or_base(sl.tau, base_now);
             const float tpow = ALPHA1 ? tau_now : pow_int(tau_now, a.alpha);
-            const float info = cand ? __fmul_rn(tpow, heur_v) : 0.0f;
+            const float info = cand ? __fmul_rn(tpow, sl.heur) : 0.0f;
             // ---- roulette in the reference's order (:155, :172-181) ------------------------------
             const unsigned cb = (__ballot_sync(FULL, cand) >> gbase) & 0x3Fu;
             const float v0 = __shfl_sync(FULL, info, 0, 8), v1 = __shfl_sync(FULL, info, 1, 8), v2 = __shfl_sync(FULL, info, 2, 8);
@@ -209,8 +223,7 @@ __global__ void __launch_bounds__(kWalkThreads) k_walk2(WalkArgs a)
             const bool stepok = live && pb != 0;
             const int prev = cur, at = steps;
             if (stepok) { cur += mv.x; P += (uint32_t)mv.y; steps++; }
-            tau_v = __ldg(tau_k + (size_t)cur * 6);
-            heur_v = __ldg(heur_k_base + (size_t)cur * heur_row);
+            in.issue(cur, P);
             // ---- outcome -------------------------------------------------------------------------
             if (live && !stepok) reason = cb == 0 ? 1 : 2;              // :162-166 / fall-through :191-192
             if (stepok && k == c) {   // the winning lane performs the move's side effects: tabu insert + addNextNode (:73-79)
@@ -218,7 +231,7 @@ __global__ void __launch_bounds__(kWalkThreads) k_walk2(WalkArgs a)
                 pid[at] = (uint32_t)prev;
                 pdir[at] = (uint8_t)c;
             }
-            const bool arrived = stepok && cur == goal;              // :182-186
+            const bool arrived = stepok && cur == in.goal;           // :182-186
             const bool capped = stepok && !arrived && steps >= cap;   // a deviation the oracle mirrors; the reference is unbounded
             result = arrived ? steps : result;
             reason = capped ? 3 : reason;
@@ -235,7 +248,7 @@ __global__ void __launch_bounds__(kWalkThreads) k_walk2(WalkArgs a)
             c_fall += (result < 0 && reason == 2) ? 1 : 0;
             c_cap += (result < 0 && reason == 3) ? 1 : 0;
             c_steps += (unsigned long long)steps; c_ants++;
-            if (k == 0) a.ant_steps[ant_local] = result;
+            if (k == 0) a.ant_steps[in.row] = result;
         }
         __syncwarp();
     }

@@ -9,7 +9,9 @@
 //   k_heuristic26    1 + beta*cos(theta) per (node, slot, goal); closed slots carry the sentinel
 //   k_walk26         one ant per WARP: lane s < 26 owns slot s — the node's 26 pheromone values (104 contiguous bytes) and
 //                    its 26 heuristic factors are one coalesced request each; the roulette re-adds the 26 scores in the
-//                    reference's order (ascending total, descending prob_sum) from values exchanged by shuffle
+//                    reference's order (ascending total, descending prob_sum) from values exchanged by shuffle.  Pass 2 of
+//                    every search and pass 1 where an axis exceeds 1024 nodes (k_walk26p below is pass 1 otherwise);
+//                    k_walk26<Batch26> (batch26.cuh) is the same walk for concurrent searches
 //   ranking          an ant's length is no longer a function of its step count (three step lengths, float sums in path
 //                    order), so the colony is ranked by the bits of L (non-negative floats order like their bit patterns;
 //                    +inf for a dead ant): rank_small.cuh with ant_L != nullptr
@@ -47,7 +49,7 @@ __global__ void __launch_bounds__(256) k_tau_init26(float* tau, int rx, int ry, 
 
 // selectNext :137, :151-154 with a general vector_b (up to three non-zero components): the reference's expressions,
 // left to right, no contraction: norm = sqrt((x*x + y*y) + z*z) (model_grid_map.hpp:51-54), dot = (ax*bx + ay*by) + az*bz.
-// c*: coordinates of the node, g*: of the goal, n*: of the neighbour.  k_heuristic26 tabulates it, k_walk_batch26 (batch26.cuh)
+// c*: coordinates of the node, g*: of the goal, n*: of the neighbour.  k_heuristic26 tabulates it, Batch26 (batch26.cuh)
 // evaluates it per step: one function, so the two cannot drift apart.
 __device__ __forceinline__ float heur26(float cx, float cy, float cz, float gx, float gy, float gz, float nx, float ny, float nz, float beta)
 {
@@ -85,28 +87,77 @@ __global__ void __launch_bounds__(256) k_heuristic26(float* __restrict__ heur, c
     heur[idx] = v;
 }
 
+// Inputs of k_walk26 for one search (WalkArgs): tau and the tabulated factor from the dense [N][26] rows
+struct Dense26 {
+    using Args = WalkArgs;
+    const float* tau_k;    // this lane's column of the tau rows
+    const float* heur_k;   // ... of the factor rows
+    bool active;           // one of the 26 slot lanes
+    int start, sx, sy, sz, goal;
+    uint32_t ant, stream_word, block_hi;   // Philox counter words of the bound ant
+    uint32_t row;          // its row of path_ids / path_dirs / ant_steps / ant_L
+    float heur_v;
+
+    __device__ __forceinline__ Dense26(const WalkArgs& a, int kk, bool active_, int)
+        : tau_k(a.tau + kk), heur_k(a.heur + kk), active(active_), start(a.start), sx(a.start % a.rx), sy((a.start % (a.rx * a.ry)) / a.rx),
+          sz(a.start / (a.rx * a.ry)), goal(a.goal), stream_word(a.stream_word), block_hi(a.block_hi)
+    {
+    }
+    __device__ __forceinline__ unsigned items(const WalkArgs& a, const IterState* st, bool resumed) const
+    {
+        return resumed ? st->overflow_n : (unsigned)min(max(st->colony - a.shard_first, 0), a.shard_chunk);
+    }
+    // item = the ant's index in this rank's chunk
+    __device__ __forceinline__ bool bind(const WalkArgs& a, uint32_t item, bool)
+    {
+        ant = (uint32_t)a.shard_first + item;
+        row = item;
+        return true;
+    }
+    // tau of this lane's slot at node cur, as stored; the factor row goes out with it
+    __device__ __forceinline__ float tau(int cur)
+    {
+        const float t = __ldg(tau_k + (size_t)cur * kK26);
+        heur_v = __ldg(heur_k + (size_t)cur * kK26);
+        return t;
+    }
+    // whether this lane's neighbour (nx, ny, nz) is open, and the factor of its slot
+    __device__ __forceinline__ bool open(int, int, int, int, int, int, int, float& heur) const
+    {
+        heur = heur_v;
+        return active && heur_v != kClosedSlot;   // NaN (duplicate plane) stays open, as in the reference
+    }
+    // whether the ant may move its visited set to HBM table o
+    __device__ __forceinline__ bool park(const WalkArgs& a, int, int lane) const
+    {
+        if (lane == 0) a.ant_steps[row] = -2;
+        return true;
+    }
+};
+
 // ------------------------------------------------------------------------------------------
 // K2 for K = 26: one ant per warp, persistent warps pulling ants from the device queue.  Everything in a step is
 // warp-uniform (one ant), so there is no predication on liveness: an ant that arrives, dies or parks leaves the loop.
 // Visited set: the same open-addressed hash of 4x4x4-node tiles (u32 key + u64 mask per entry) in shared
 // memory, one table per warp; an ant that fills it to 3/4 moves the set to its table in HBM, parks {node, steps, tiles,
-// L} and is resumed by pass 2 (GLOBAL) — exact, its draws are a pure function of (iteration, ant, step).
+// L} and is resumed by pass 2 (GLOBAL) — exact, its draws are a pure function of (iteration, ant, step).  Coordinates are
+// unpacked, so no axis limit.  In = Dense26 (one search) or Batch26 (concurrent searches, batch26.cuh) says where tau, the
+// factor, the open neighbours and the ant's identity come from.
 // ------------------------------------------------------------------------------------------
-template <bool GLOBAL>
-__global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
+template <class In, bool GLOBAL>
+__global__ void __launch_bounds__(kWalk26Threads) k_walk26(typename In::Args a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31;
     const int w = threadIdx.x >> 5;
-    const int E = 1 << a.table_log2;
-    const int hshift = 32 - a.table_log2;
+    const int tlog2 = GLOBAL ? a.gtable_log2 : a.table_log2;
+    const int E = 1 << tlog2;
+    const int hshift = 32 - tlog2;
 
-    unsigned long long* masks;
-    uint32_t* keys;
-    if (GLOBAL) {
-        keys = a.gkeys; masks = a.gmasks;   // re-pointed per ant below
-    } else {
+    unsigned long long* masks = nullptr;   // GLOBAL: pointed at the ant's HBM table below
+    uint32_t* keys = nullptr;
+    if (!GLOBAL) {
         unsigned long long* mbase = reinterpret_cast<unsigned long long*>(smem_raw);
         masks = mbase + (size_t)w * E;
         keys = reinterpret_cast<uint32_t*>(mbase + (size_t)kWalk26Ants * E) + (size_t)w * E;
@@ -123,16 +174,14 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
     const int type_k = (dxk != 0) + (dyk != 0) + (dzk != 0);
     // per-slot step length, initFromGridMap :375-385 with the commented-out lengths enabled
     const float dist_k = type_k == 1 ? a.precision : (type_k == 2 ? __fmul_rn(a.precision, 1.414f) : __fmul_rn(a.precision, 1.732f));
-
-    const int sz = a.start / rxy, sy = (a.start % rxy) / rx, sx = a.start % rx;
+    In in(a, kk, active, stride_k);
     const bool alpha1 = a.alpha == 1;
+    const int cap = a.cap;
 
     IterState* st = a.st;
-    const int colony = st->colony;
     const uint32_t iter = (uint32_t)st->iter;
     const float base_now = st->base;
-    int local_n = min(max(colony - a.shard_first, 0), a.shard_chunk);
-    if (GLOBAL) local_n = (int)st->overflow_n;
+    const unsigned n_items = in.items(a, st, GLOBAL);
     const int limit = (E >> 2) * 3;
 
     unsigned long long c_steps = 0, c_ants = 0, c_arrived = 0, c_nocand = 0, c_fall = 0, c_cap = 0, c_over = 0;
@@ -141,20 +190,19 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
         unsigned q = 0;
         if (lane == 0) q = atomicAdd(GLOBAL ? &st->queue2 : &st->queue, 1u);
         q = __shfl_sync(FULL, q, 0);
-        if (q >= (unsigned)local_n) break;
-        const int ant_local = GLOBAL ? (int)a.overflow_list[q] : (int)q;
-        const uint32_t ant_global = (uint32_t)(a.shard_first + ant_local);
+        if (q >= n_items) break;                                         // warp-uniform
+        if (!in.bind(a, GLOBAL ? a.overflow_list[q] : q, GLOBAL)) continue;
 
-        int cur = a.start, x = sx, y = sy, z = sz, steps = 0, ntiles = 1;
+        int cur = in.start, x = in.sx, y = in.sy, z = in.sz, steps = 0, ntiles = 1;
         float L = 0.0f;                                   // addStartNode :81-86
         uint32_t rw0 = 0, rw1 = 0, rw2 = 0, rw3 = 0;
         if (GLOBAL) {   // resume a parked ant: its visited set already lives in HBM table q
             keys = a.gkeys + (size_t)q * E;
-            masks = a.gmasks + (size_t)q * E;
+            masks = a.gtab + (size_t)q * E;
             const int4 r = a.resume[q];
             cur = r.x; steps = r.y; ntiles = r.z; L = __int_as_float(r.w);
             z = cur / rxy; y = (cur % rxy) / rx; x = cur % rx;
-            philox4(iter, ant_global, ((uint32_t)steps >> 2) | a.block_hi, a.stream_word, a.seed_lo, a.seed_hi, rw0, rw1, rw2, rw3);
+            philox4(iter, in.ant, ((uint32_t)steps >> 2) | in.block_hi, in.stream_word, a.seed_lo, a.seed_hi, rw0, rw1, rw2, rw3);
         } else {
             for (int i = lane; i < E; i += 32) keys[i] = kEmptyKey;
             __syncwarp();
@@ -169,19 +217,19 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
 
         int result = -1;   // >= 0: steps of an ant that arrived, -1: dead, -2: parked (table overflow -> pass 2)
         int reason = 0;    // 1 no candidate, 2 roulette fall-through, 3 step cap
-        uint32_t* pid = a.path_ids + (size_t)ant_local * a.cap;
-        uint8_t* pdir = a.path_dirs + (size_t)ant_local * a.cap;
+        uint32_t* pid = a.path_ids + (size_t)in.row * cap;
+        uint8_t* pdir = a.path_dirs + (size_t)in.row * cap;
 
         while (true) {
-            if (steps >= a.cap) { reason = 3; break; }   // step cap (a deviation the oracle mirrors)
-            const float tau_k = tau_or_base(__ldg(a.tau + (size_t)cur * kK26 + kk), base_now);
-            const float heur_k = __ldg(a.heur + (size_t)cur * kK26 + kk);
-            if ((steps & 3) == 0) philox4(iter, ant_global, ((uint32_t)steps >> 2) | a.block_hi, a.stream_word, a.seed_lo, a.seed_hi, rw0, rw1, rw2, rw3);
+            if (steps >= cap) { reason = 3; break; }   // step cap (a deviation the oracle mirrors)
+            const float tau_k = tau_or_base(in.tau(cur), base_now);
+            if ((steps & 3) == 0) philox4(iter, in.ant, ((uint32_t)steps >> 2) | in.block_hi, in.stream_word, a.seed_lo, a.seed_hi, rw0, rw1, rw2, rw3);
             const uint32_t rsel = (steps & 2) ? ((steps & 1) ? rw3 : rw2) : ((steps & 1) ? rw1 : rw0);
             const float u = __fmul_rn(__int2float_rn((int)(rsel >> 1)), 4.656612873077392578125e-10f);   // (float)rand()/(float)RAND_MAX :169
-            // ---- neighbour of this lane: open (in bounds and free, folded into the table), tabu probe ----
+            // ---- neighbour of this lane: open (in bounds and free), geometric factor, tabu probe ----
             const int nx = x + dxk, ny = y + dyk, nz = z + dzk;
-            const bool open_k = active && heur_k != kClosedSlot;   // NaN (duplicate plane) stays open, as in the reference
+            float heur_k;
+            const bool open_k = in.open(cur, x, y, z, nx, ny, nz, heur_k);
             const uint32_t tile = (uint32_t)(((nz >> 2) * TY + (ny >> 2)) * TX + (nx >> 2));
             const unsigned bit = ((nz & 3) << 4) | ((ny & 3) << 2) | (nx & 3);
             unsigned slot = (tile * 2654435761u) >> hshift;
@@ -225,14 +273,15 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
             steps++;
             ntiles += newtile;
             __syncwarp();
-            if (cur == a.goal) { result = steps; break; }       // :182-186
+            if (cur == in.goal) { result = steps; break; }      // :182-186
             if (!GLOBAL && newtile && ntiles > limit) {          // rare: shared-memory table 3/4 full -> park for pass 2
                 int o = 0;
                 if (lane == 0) o = (int)atomicAdd(&st->overflow_n, 1u);
                 o = __shfl_sync(FULL, o, 0);
+                if (!in.park(a, o, lane)) break;
                 const int Eg = 1 << a.gtable_log2, gsh = 32 - a.gtable_log2;
                 uint32_t* nkeys = a.gkeys + (size_t)o * Eg;
-                unsigned long long* nmasks = a.gmasks + (size_t)o * Eg;
+                unsigned long long* nmasks = a.gtab + (size_t)o * Eg;
                 for (int i = lane; i < Eg; i += 32) nkeys[i] = kEmptyKey;
                 __syncwarp();
                 for (int i = lane; i < E; i += 32) {
@@ -244,8 +293,7 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
                 }
                 if (lane == 0) {
                     a.resume[o] = make_int4(cur, steps, ntiles, __float_as_int(L));
-                    a.overflow_list[o] = (uint32_t)ant_local;
-                    a.ant_steps[ant_local] = -2;
+                    a.overflow_list[o] = in.row;
                 }
                 result = -2;
                 break;
@@ -256,8 +304,8 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
             c_over++;   // its steps are counted by pass 2
         } else {
             if (lane == 0) {
-                a.ant_steps[ant_local] = result;
-                a.ant_L[ant_local] = result >= 0 ? L : INFINITY;   // setDeadEnd :88-91
+                a.ant_steps[in.row] = result;
+                a.ant_L[in.row] = result >= 0 ? L : INFINITY;   // setDeadEnd :88-91
             }
             c_steps += (unsigned long long)steps; c_ants++;
             c_arrived += result >= 0 ? 1 : 0;
@@ -278,7 +326,6 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
     }
 }
 
-
 // ------------------------------------------------------------------------------------------
 // K2 for K = 26, pass 1, second generation (round 2): the step of k_walk26 with the instruction stream cut from ~340 to ~170
 // per step, by the means that worked for K = 6 (walk3.cuh) plus two that are specific to 26 slots:
@@ -288,7 +335,7 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26(WalkArgs a)
 //   * packed coordinates z<<20 | y<<10 | x (one add per move, tile key = one AND, bit index = one multiply);
 //   * the move (node stride, packed delta, step length) is one LDS.128 from a 26-entry table instead of five shuffles;
 //   * Philox for steps T+4..T+7 in four slices beside steps T..T+3; the trail in registers, 32 steps per coalesced store.
-// Grids with an axis above 1024 nodes keep k_walk26<false>; parked ants are resumed by k_walk26<true> either way (the visited set
+// Grids with an axis above 1024 nodes keep k_walk26<Dense26, false>; parked ants are resumed by k_walk26<Dense26, true> either way (the visited set
 // is re-keyed to its tile indices when it moves to HBM).
 // ------------------------------------------------------------------------------------------
 constexpr uint32_t kLow26 = 0x00300C03u;                       // x, y, z bits 0-1: position inside a 4x4x4 tile
@@ -474,7 +521,7 @@ __global__ void __launch_bounds__(kWalk26Threads) k_walk26p(WalkArgs a)
             o = __shfl_sync(FULL, o, 0);
             const int Eg = 1 << a.gtable_log2, gsh = 32 - a.gtable_log2;
             uint32_t* nkeys = a.gkeys + (size_t)o * Eg;
-            unsigned long long* nmasks = a.gmasks + (size_t)o * Eg;
+            unsigned long long* nmasks = a.gtab + (size_t)o * Eg;
             for (int i = lane; i < Eg; i += 32) nkeys[i] = kEmptyKey;
             __syncwarp();
             for (int i = lane; i < E; i += 32) {
