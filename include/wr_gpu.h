@@ -175,6 +175,9 @@ int wr_acs_set_timing(wr_acs* a, int enabled);
 /* WR_UPDATE_RANKSET: [0] the last iteration took the rank-set path, [1] pheromone tiles that received deposits in the last
  * record-path iteration, [2] distinct slots in the last rank-set iteration, [3] rank-set iterations since begin */
 int wr_acs_update_stats(wr_acs* a, uint32_t out[4]);
+/* Converged iterations check the best path against roulette thresholds instead of walking it (WR_WALK_VERIFY, default on):
+ * [0] ants completed by that check alone, [1] ant-steps it decided, both cumulative since the handle was created */
+int wr_acs_walk_stats(wr_acs* a, uint64_t out[2]);
 /* Clean-tile pheromone field (FUSED / RANKSET handles): [0] 16 KB tiles that hold at least one slot that ever received a
  * deposit since init/reset() — the only tiles the evaporation pass reads and writes — [1] tiles of the field.  Slots that
  * never received a deposit all hold the same value (tau0 * rho per iteration, kept as one scalar); downloads materialise it. */

@@ -495,6 +495,13 @@ class ACS_Rank(GridMap):
         check(lib().wr_acs_update_stats(self._need(), ptr(out)))
         return dict(rankset_last=int(out[0]), deposit_tiles=int(out[1]), distinct_slots=int(out[2]), rankset_iterations=int(out[3]))
 
+    def walkStats(self):
+        """Converged iterations: ants completed by checking the best path against roulette thresholds, and the ant-steps that
+        check decided (cumulative since the handle was created)."""
+        out = np.zeros(2, np.uint64)
+        check(lib().wr_acs_walk_stats(self._need(), ptr(out)))
+        return dict(verified_ants=int(out[0]), verified_steps=int(out[1]))
+
     def streamKernelMs(self):
         """(cumulative device ms, launches) of the kernel that streams the pheromone field, timed inside the loop."""
         ms = C.c_float(); n = C.c_int()

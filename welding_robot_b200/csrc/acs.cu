@@ -15,6 +15,7 @@
 #include "walk2.cuh"
 #include "walk26.cuh"
 #include "walk3.cuh"
+#include "path_verify.cuh"
 #include "rank_small.cuh"
 #include "rankset.cuh"
 #include "batch.cuh"
@@ -145,6 +146,12 @@ struct wr_acs {
     int* d_best_n = nullptr;
     uint32_t* d_best_ids = nullptr;
     uint8_t* d_best_dirs = nullptr;
+    // path verification of converged iterations (path_verify.cuh): thresholds [cap + 1], node / tile -> position maps, {D, full}
+    float4* d_thr = nullptr;
+    uint2* d_pmap = nullptr;
+    uint32_t pmap_entries = 0;
+    int2* d_pv = nullptr;
+    int* d_vdev = nullptr;           // [chunk] steps each ant followed the best path
     // per-colony buffers (sized at begin)
     int* d_ant_steps = nullptr;      // global colony order (ranking input)
     int* d_local_steps = nullptr;    // this rank's chunk (== d_ant_steps when nranks == 1)
@@ -330,6 +337,7 @@ static void free_colony_buffers(wr_acs* a)
     drop_steady_graph(a);
     free_rankset(a);
     pool_free(a->d_ant_steps, s); pool_free(a->d_overflow, s); pool_free(a->d_ant_L, s); a->d_ant_L = nullptr;
+    pool_free(a->d_vdev, s); a->d_vdev = nullptr;
     if (!a->d_slab) { pool_free(a->d_path_ids, s); pool_free(a->d_path_dirs, s); }
     pool_free(a->d_gkeys, s); pool_free(a->d_gmasks, s); pool_free(a->d_resume, s); a->d_resume = nullptr; pool_free(a->d_rec_off, s); pool_free(a->d_order, s);
     a->d_local_steps = nullptr;   // aliases d_ant_steps (one GPU) or lives in the slab (sharded)
@@ -406,6 +414,7 @@ static int alloc_colony_buffers(wr_acs* a, int colony_max)
     }
     WR_CUDA(dmalloc(&a->d_overflow, chunk * sizeof(uint32_t), a->stream));
     if (a->K == kK26) WR_CUDA(dmalloc(&a->d_ant_L, chunk * sizeof(float), a->stream));
+    else WR_CUDA(dmalloc(&a->d_vdev, chunk * sizeof(int), a->stream));
     WR_CUDA(dmalloc(&a->d_rec_off, cm * sizeof(uint32_t), a->stream));
     WR_CUDA(dmalloc(&a->d_order, cm * sizeof(int), a->stream));
     WR_CUDA(cudaMemsetAsync(a->d_order, 0, cm * sizeof(int), a->stream));
@@ -479,6 +488,11 @@ static int walk_prefetch()
     static const int env = [] { const char* e = getenv("WR_WALK_PREFETCH"); return e ? atoi(e) : -1; }();   // -1: chosen per iteration (launch_walk)
     return env;
 }
+static bool walk_verify()
+{
+    static const bool on = [] { const char* e = getenv("WR_WALK_VERIFY"); return !e || atoi(e) != 0; }();   // 0: converged ants walk the whole path
+    return on;
+}
 static int stream_cs()
 {
     static const int env = [] { const char* e = getenv("WR_STREAM_CS"); return e ? atoi(e) : 1; }();   // evict-first streaming of the tiles without deposits (default on)
@@ -535,6 +549,7 @@ extern "C" int wr_acs_destroy(wr_acs* a)
     pool_free(a->d_tau, s); pool_free(a->d_heur, s); pool_free(a->d_state, s); pool_free(a->d_onbest, s); pool_free(a->d_Ltab, s);
     pool_free(a->d_best_n, s); pool_free(a->d_best_ids, s); pool_free(a->d_best_dirs, s); pool_free(a->d_tile_off, s); pool_free(a->d_dep_list, s);
     pool_free(a->d_upd_q, s); pool_free(a->d_dirty, s);
+    pool_free(a->d_thr, s); pool_free(a->d_pmap, s); pool_free(a->d_pv, s);
     if (a->stream) cudaStreamSynchronize(a->stream);
     feedback_release(a->h_feedback);
     for (cudaEvent_t e : a->sk_ev) cudaEventDestroy(e);
@@ -623,6 +638,13 @@ extern "C" int wr_acs_create(wr_grid* g, const wr_acs_params* p, wr_acs** out)
     WR_CUDA_A(dmalloc(&a->d_best_ids, ((size_t)a->cap + 16) * sizeof(uint32_t), a->stream));   // k_walk3 reads ids up to 7 positions past the walk: every entry must be a node id
     WR_CUDA_A(cudaMemsetAsync(a->d_best_ids, 0, ((size_t)a->cap + 16) * sizeof(uint32_t), a->stream));
     WR_CUDA_A(dmalloc(&a->d_best_dirs, (size_t)a->cap + 2, a->stream));
+    if (a->K == 6) {
+        a->pmap_entries = 2;
+        while (a->pmap_entries < 2u * ((uint32_t)a->cap + 1)) a->pmap_entries <<= 1;
+        WR_CUDA_A(dmalloc(&a->d_thr, ((size_t)a->cap + 1) * sizeof(float4), a->stream));
+        WR_CUDA_A(dmalloc(&a->d_pmap, 2 * (size_t)a->pmap_entries * sizeof(uint2), a->stream));
+        WR_CUDA_A(dmalloc(&a->d_pv, sizeof(int2), a->stream));
+    }
     WR_CUDA_A(dmalloc(&a->d_tile_off, ((size_t)a->ntiles + 2) * sizeof(uint32_t), a->stream));
     WR_CUDA_A(dmalloc(&a->d_dep_list, ((size_t)a->ntiles + 2) * sizeof(uint32_t), a->stream));
     WR_CUDA_A(dmalloc(&a->d_upd_q, 4 * sizeof(uint32_t), a->stream));
@@ -834,6 +856,17 @@ static int launch_walk(wr_acs* a)
     // instructions per step are pure issue cost (converged walk 0.346 -> 0.317 ms without them)
     int pf = walk_prefetch();
     if (pf < 0) pf = (a->rankset && a->rs_choice) ? 0 : 2;
+    // predicted gathers (a converged colony): most ants follow the best path, which is checked for all of them at once
+    w.verify_dev = nullptr; w.verify_n = a->d_pv;
+    if (!pf && walk_verify()) {
+        k_path_thresholds<<<1, kPathThreads, 0, a->stream>>>(a->d_state, a->d_best_n, a->d_best_ids, a->d_best_dirs, a->d_tau, a->d_heur, a->p.alpha, g->rx, g->ry,
+                                                            g->rz, (int)a->start, (int)a->goal, a->cap, (uint32_t)((a->table_entries >> 2) * 3), a->d_pmap,
+                                                            a->pmap_entries, a->d_thr, a->d_pv);
+        k_path_verify<<<(unsigned)((a->chunk + kVerifyThreads / 32 - 1) / (kVerifyThreads / 32)), kVerifyThreads, 0, a->stream>>>(
+            a->d_state, a->d_pv, a->d_thr, a->d_best_ids, a->d_best_dirs, w.seed_lo, w.seed_hi, w.stream_word, w.block_hi, w.shard_first, w.shard_chunk, a->cap,
+            a->d_vdev, a->d_path_ids, a->d_path_dirs);
+        w.verify_dev = a->d_vdev;
+    }
     if (!alpha1 && pf) k_walk3<false, 1><<<blocks1, kWalkThreads, smem1, a->stream>>>(w);
     else if (!alpha1) k_walk3<false, 0><<<blocks1, kWalkThreads, smem1, a->stream>>>(w);
     else if (pf) k_walk3<true, 1><<<blocks1, kWalkThreads, smem1, a->stream>>>(w);
@@ -1549,7 +1582,7 @@ static int preload_iteration_kernels()
     WR_PRELOAD((k_deposit_gen<false, true>)); WR_PRELOAD(k_tile_offsets); WR_PRELOAD(k_update_fused<true>); WR_PRELOAD(k_update_fused<false>);
     WR_PRELOAD(k_pull_finals); WR_PRELOAD(k_iter_begin); WR_PRELOAD(k_iter_end);
     WR_PRELOAD((k_walk3<true, 0>)); WR_PRELOAD((k_walk3<true, 1>)); WR_PRELOAD((k_walk3<false, 0>)); WR_PRELOAD((k_walk3<false, 1>));
-    WR_PRELOAD((k_walk2<Dense6, true>)); WR_PRELOAD((k_walk2<Dense6, false>));
+    WR_PRELOAD((k_walk2<Dense6, true>)); WR_PRELOAD((k_walk2<Dense6, false>)); WR_PRELOAD(k_path_thresholds); WR_PRELOAD(k_path_verify);
 #undef WR_PRELOAD
     int rc = sort_preload();
     if (rc != WR_OK) return rc;
@@ -1782,6 +1815,16 @@ extern "C" int wr_acs_counters(wr_acs* a, uint64_t out[9])
     IterState st;
     WR_CUDA(cudaMemcpy(&st, a->d_state, sizeof st, cudaMemcpyDeviceToHost));
     for (int i = 0; i < 9; i++) out[i] = st.cnt[i];
+    return WR_OK;
+}
+
+extern "C" int wr_acs_walk_stats(wr_acs* a, uint64_t out[2])
+{
+    WR_REQUIRE(a && out, WR_ERR_INVALID, "wr_acs_walk_stats: null");
+    WR_CUDA(cudaStreamSynchronize(a->stream));
+    IterState st;
+    WR_CUDA(cudaMemcpy(&st, a->d_state, sizeof st, cudaMemcpyDeviceToHost));
+    out[0] = st.verified[0]; out[1] = st.verified[1];
     return WR_OK;
 }
 

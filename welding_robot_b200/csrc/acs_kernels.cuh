@@ -65,6 +65,8 @@ struct WalkArgs {
     float precision;         // K = 26 (walk26.cuh): step lengths precision, precision*1.414f, precision*1.732f
     float* ant_L;            // K = 26: [chunk] length of the finished ant, +inf if it died (for K = 6 L is a function of steps)
     const uint32_t* best_ids;   // k_walk3: nodes of the best path so far, [cap + 16], every entry a valid node id (gather prediction)
+    const int* verify_dev;   // k_walk3<*, 0>: [chunk] steps each ant followed the best path (k_path_verify), nullptr: walk from the start
+    const int2* verify_n;    // {verifiable prefix D, best_n - 1 if the whole path verified else -1} (k_path_thresholds)
 };
 
 __device__ __forceinline__ float pow_int(float x, int y)

@@ -47,6 +47,31 @@ __device__ __forceinline__ void philox_rounds(uint32_t& c0, uint32_t& c1, uint32
     }
 }
 
+// The roulette arithmetic of one step, shared with k_path_thresholds (path_verify.cuh), which must reproduce it bit for bit.
+// Score of a slot (:151-154): tau^alpha * (1 + beta*cos), 0 for a slot that is no candidate.
+template <bool ALPHA1>
+__device__ __forceinline__ float slot_score(bool cand, float tau_v, float heur_v, float base, int alpha)
+{
+    const float tau_now = tau_or_base(tau_v, base);
+    const float tpow = ALPHA1 ? tau_now : pow_int(tau_now, alpha);
+    return cand ? __fmul_rn(tpow, heur_v) : 0.0f;
+}
+// the roulette total (:155) and the suffix sum v5 + ... + v_k that slot k compares with the draw (:172-181); m_j = k <= j ? ~0 : 0
+__device__ __forceinline__ float roulette_total(float v0, float v1, float v2, float v3, float v4, float v5)
+{
+    return __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(0.0f, v0), v1), v2), v3), v4), v5);
+}
+__device__ __forceinline__ float roulette_suffix(float v0, float v1, float v2, float v3, float v4, float v5, uint32_t m4, uint32_t m3, uint32_t m2,
+                                                 uint32_t m1, uint32_t m0)
+{
+    float mine = __fadd_rn(0.0f, v5);
+    mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v4) & m4));
+    mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v3) & m3));
+    mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v2) & m2));
+    mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v1) & m1));
+    return __fadd_rn(mine, __uint_as_float(__float_as_uint(v0) & m0));
+}
+
 template <bool ALPHA1, int PREFETCH>
 __global__ void __launch_bounds__(kWalkThreads, 2) k_walk3(WalkArgs a)   // two CTAs per SM (shared memory); no register squeeze
 {
@@ -63,6 +88,7 @@ __global__ void __launch_bounds__(kWalkThreads, 2) k_walk3(WalkArgs a)   // two 
     __syncthreads();
 
     constexpr unsigned FULL = 0xffffffffu;
+    constexpr bool PREDICT = PREFETCH == 0;   // 0: converged colony, predicted gathers; 1: wandering colony, neighbour rows prefetched
     const int lane = threadIdx.x & 31;
     const int gbase = lane & 24;
     const int k = lane & 7;
@@ -103,6 +129,8 @@ __global__ void __launch_bounds__(kWalkThreads, 2) k_walk3(WalkArgs a)   // two 
     asm volatile("" : "+r"(cap_k), "+r"(lut_rot));
 
     unsigned long long c_steps = 0, c_ants = 0, c_arrived = 0, c_nocand = 0, c_fall = 0, c_cap = 0, c_over = 0;
+    uint32_t c_vants = 0, c_vsteps = 0;    // ants completed by verification, steps not walked here because they were verified
+    const int vfull = (PREDICT && a.verify_dev) ? a.verify_n->y : -1;   // best_n - 1 when the whole best path verified, else -1
 
     while (true) {
         unsigned q0 = 0;
@@ -114,32 +142,68 @@ __global__ void __launch_bounds__(kWalkThreads, 2) k_walk3(WalkArgs a)   // two 
         const int ant_local = has ? (int)q : 0;
         const uint32_t ant_global = (uint32_t)(a.shard_first + ant_local);
 
-        for (int i = k; i < E; i += kGroup) tab.store(i, 0ull);
-        __syncwarp();
-        if (k == 0) {   // addStartNode :81-86
-            const uint32_t key = Pstart & kKeyMask;
-            const uint32_t bit = (((Pstart & kPackLow) * kPackMul) >> 20) & 31u;
-            tab.store(tile_hash(key, (uint32_t)E - 3u), ((unsigned long long)key << 32) | (unsigned long long)(1u << bit));
+        // Converged colony with the path verified (k_path_verify): every ant of the warp has followed the best path for at least
+        // T steps, a multiple of 8, so it stands on best[T] with visited set best[0..T], like any other such ant.  The warp
+        // resumes there; if all its ants followed the whole path, it only does their bookkeeping.
+        uint32_t T = 0;                    // step index of every live ant of the warp
+        bool done = false;
+        if (PREDICT && a.verify_dev) {
+            const int dv = has ? a.verify_dev[ant_local] : INT_MAX;
+            const bool complete = has && dv == vfull;
+            T = __reduce_min_sync(FULL, (uint32_t)(complete ? vfull : dv) & ~7u);
+            done = __all_sync(FULL, !has || complete);
+            if (done) { c_vants += has ? 1u : 0u; c_vsteps += has ? (uint32_t)vfull : 0u; }
+            else c_vsteps += has ? T : 0u;
         }
-        __syncwarp();
-
-        int cur = a.start, steps = 0;
-        uint32_t P = Pstart;
         uint32_t ntiles = 1u;
+        if (!done) {
+            for (int i = k; i < E; i += kGroup) tab.store(i, 0ull);
+            __syncwarp();
+            if (T == 0) {
+                if (k == 0) {   // addStartNode :81-86
+                    const uint32_t key = Pstart & kKeyMask;
+                    const uint32_t bit = (((Pstart & kPackLow) * kPackMul) >> 20) & 31u;
+                    tab.store(tile_hash(key, (uint32_t)E - 3u), ((unsigned long long)key << 32) | (unsigned long long)(1u << bit));
+                }
+            } else {   // the tiles of best[0..T], the group's lanes in parallel; linear probing gives the same look-ups in any insertion order
+                unsigned* tw = reinterpret_cast<unsigned*>(tab_s + (size_t)g * E);   // entry i: mask word 2i, key word 2i + 1
+                uint32_t claims = 0;
+                for (uint32_t p = (uint32_t)k; p <= T; p += kGroup) {
+                    const int node = (int)a.best_ids[p];
+                    const uint32_t Pn = pack_xyz(node % rx, (node % rxy) / rx, node / rxy) | kKeyTag;
+                    const uint32_t key = Pn & kKeyMask;
+                    const uint32_t bit = (((Pn & kPackLow) * kPackMul) >> 20) & 31u;
+                    unsigned slot = tile_hash(key, (uint32_t)E - 3u);
+                    while (true) {
+                        const unsigned old = atomicCAS(tw + 2 * slot + 1, 0u, key);
+                        if (old == 0u || old == key) { atomicOr(tw + 2 * slot, 1u << bit); claims += old == 0u ? 1u : 0u; break; }
+                        slot = slot + 1 < (unsigned)E ? slot + 1 : 0u;
+                    }
+                }
+                __syncwarp();
+                claims += __shfl_xor_sync(FULL, claims, 4);
+                claims += __shfl_xor_sync(FULL, claims, 2);
+                claims += __shfl_xor_sync(FULL, claims, 1);
+                ntiles = claims;
+            }
+            __syncwarp();
+        }
+
+        int cur = done ? goal : (T ? (int)a.best_ids[T] : a.start), steps = done ? vfull : (int)T;
+        uint32_t P = T ? pack_xyz(cur % rx, (cur % rxy) / rx, cur / rxy) | kKeyTag : Pstart;
         uint32_t lastcb = 1u;              // candidate mask of the last step the ant was alive in (why a dead ant died)
         bool parked = false;
-        bool live = has && cap_k > 0;
-        uint32_t T = 0;                    // step index of every live ant of the warp
-        uint32_t kt = (uint32_t)k;         // (k - T) & 7: the lane that keeps step T + j of the trail is the one with kt == j
+        bool live = has && cap_k > 0 && !done;
+        uint32_t kt = (uint32_t)k;         // (k - T) & 7: the lane that keeps step T + j of the trail is the one with kt == j (T % 8 == 0)
         uint32_t rec_id = 0, rec_dir = 0;
         uint32_t* pid = a.path_ids + (size_t)ant_local * cap;
         uint8_t* pdir = a.path_dirs + (size_t)ant_local * cap;
 
-        // draws of steps 0..3; the next block is produced inside the loop, one slice per step
+        // draws of steps T..T+3; the next block is produced inside the loop, one slice per step
         float u0, u1, u2, u3;
         {
             uint32_t w0, w1, w2, w3;
-            philox4(iter, ant_global, a.block_hi, a.stream_word, a.seed_lo, a.seed_hi, w0, w1, w2, w3);
+            philox4(iter, ant_global, (T >> 2) | a.block_hi, a.stream_word, a.seed_lo, a.seed_hi, w0, w1, w2, w3);
             // (float)rand()/(float)RAND_MAX (:169): (float)RAND_MAX is 2^31, so the division is an exact scaling
             u0 = __fmul_rn(__int2float_rn((int)(w0 >> 1)), 4.656612873077392578125e-10f);
             u1 = __fmul_rn(__int2float_rn((int)(w1 >> 1)), 4.656612873077392578125e-10f);
@@ -153,12 +217,11 @@ __global__ void __launch_bounds__(kWalkThreads, 2) k_walk3(WalkArgs a)   // two 
         float heur_v = __ldg(heur_k + (size_t)cur * 6);
 
         // predicted rows (PREDICT): best-path positions T+1..T+3 (c*) and T+4..T+7 (n*), this lane's slot of each
-        constexpr bool PREDICT = PREFETCH == 0;   // 0: converged colony, predicted gathers; 1: wandering colony, neighbour rows prefetched
         uint32_t c1 = 0, c2 = 0, c3 = 0, n0 = 0, n1 = 0, n2 = 0, n3 = 0;
         float ct1 = 0.f, ct2 = 0.f, ct3 = 0.f, ch1 = 0.f, ch2 = 0.f, ch3 = 0.f;
         float nt0 = 0.f, nt1 = 0.f, nt2 = 0.f, nt3 = 0.f, nh0 = 0.f, nh1 = 0.f, nh2 = 0.f, nh3 = 0.f;
         if (PREDICT) {
-            const uint4 q = __ldg(reinterpret_cast<const uint4*>(a.best_ids));
+            const uint4 q = __ldg(reinterpret_cast<const uint4*>(a.best_ids + T));
             c1 = q.y; c2 = q.z; c3 = q.w;
             ct1 = __ldg(tau_k + (size_t)c1 * 6); ch1 = __ldg(heur_k + (size_t)c1 * 6);
             ct2 = __ldg(tau_k + (size_t)c2 * 6); ch2 = __ldg(heur_k + (size_t)c2 * 6);
@@ -225,21 +288,14 @@ __global__ void __launch_bounds__(kWalkThreads, 2) k_walk3(WalkArgs a)   // two 
             }
             const bool cand = live && open_k && !(emask & bitm);
             // ---- info = tau^alpha * (1 + beta*cos)  (:151-154) ------------------------------------------------------
-            const float tau_now = tau_or_base(tau_v, base_now);
-            const float tpow = ALPHA1 ? tau_now : pow_int(tau_now, a.alpha);
-            const float info = cand ? __fmul_rn(tpow, heur_v) : 0.0f;
+            const float info = slot_score<ALPHA1>(cand, tau_v, heur_v, base_now, a.alpha);
             // ---- roulette in the reference's order (:155, :172-181) ------------------------------------------------
             const unsigned cb = __ballot_sync(FULL, cand) & gmask;
             const float v0 = __shfl_sync(FULL, info, 0, 8), v1 = __shfl_sync(FULL, info, 1, 8), v2 = __shfl_sync(FULL, info, 2, 8);
             const float v3 = __shfl_sync(FULL, info, 3, 8), v4 = __shfl_sync(FULL, info, 4, 8), v5 = __shfl_sync(FULL, info, 5, 8);
-            const float total = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(0.0f, v0), v1), v2), v3), v4), v5);
+            const float total = roulette_total(v0, v1, v2, v3, v4, v5);
             const float rnd = __fmul_rn(u, total);
-            float mine = __fadd_rn(0.0f, v5);
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v4) & m4));
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v3) & m3));
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v2) & m2));
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v1) & m1));
-            mine = __fadd_rn(mine, __uint_as_float(__float_as_uint(v0) & m0));
+            const float mine = roulette_suffix(v0, v1, v2, v3, v4, v5, m4, m3, m2, m1, m0);
             const bool pick = cand && (mine >= rnd);
             const unsigned pball = __ballot_sync(FULL, pick);
             // ---- the move: a dead or finished ant has no pick and the table's entry 0 moves nowhere --------------------
@@ -366,6 +422,8 @@ __global__ void __launch_bounds__(kWalkThreads, 2) k_walk3(WalkArgs a)   // two 
         if (c_fall) atomicAdd(&st->cnt[4], c_fall);
         if (c_cap) atomicAdd(&st->cnt[5], c_cap);
         if (c_over) atomicAdd(&st->cnt[8], c_over);
+        if (c_vants) atomicAdd(&st->verified[0], (unsigned long long)c_vants);
+        if (c_vsteps) atomicAdd(&st->verified[1], (unsigned long long)c_vsteps);
     }
 }
 

@@ -120,6 +120,7 @@ struct IterState {
     unsigned queue2;     // pass 2 (resumed ants): its own counter, so no reset launch sits between the two passes
     unsigned overflow_n; // ants whose shared-memory visited table overflowed (pass 2)
     unsigned long long cnt[9];
+    unsigned long long verified[2];   // k_walk3: ants completed by path verification, ant-steps it decided (wr_acs_walk_stats)
 };
 
 }  // namespace wr
