@@ -87,16 +87,88 @@ def _endpoints(A):
     return int(ids[10]), int(ids[-10])
 
 
-def _run_vs_oracle(A, g, iters=(1, 1, 1, 1, 12, 14)):
+def tile_of(node, rx, ry):
+    """k_walk3's visited-table key of a node: its 4 x 4 x 2 tile."""
+    x, y, z = node % rx, (node // rx) % ry, node // (rx * ry)
+    return (x >> 2, y >> 2, z >> 1)
+
+
+def expected_walk_stats(best, trails, start, goal, cap, dims, table_log2=0, colony=None, world=1, nonfinite=()):
+    """walkStats() increments of one converged iteration, from the CPU oracle alone.
+
+    best: the best path's node ids before the iteration; trails: every ant's node ids from the iteration (the oracle keeps
+    them for dead ants too); nonfinite: best-path positions whose roulette total or suffix sums are not finite.  The
+    verifiable prefix D is the first position the check cannot decide (step cap, visited table full, non-finite sums); an
+    ant's dev is the first step it leaves the best path.  Warps of four consecutive ants of a shard either book their ants
+    complete (every ant followed the whole path) or resume at the lowest floor8(dev) of their ants.
+    Returns ([{verified_ants, verified_steps} per shard], {D, n, dev, warps: [(shard, first ant, present, T, done)]})."""
+    rx, ry, _ = dims
+    n = len(best)
+    D = n - 1 if 2 <= n <= cap + 1 else 0
+    limit = ((1 << table_log2 if table_log2 > 0 else 768) >> 2) * 3
+    if D > 0:
+        assert int(best[0]) == start and int(best[-1]) == goal
+        tiles = set()
+        for t in range(D):
+            tiles.add(tile_of(int(best[t]), rx, ry))
+            if t + 1 >= cap or len(tiles) > limit or t in nonfinite:
+                D = t
+                break
+    colony = len(trails) if colony is None else colony
+    dev = np.empty(colony, np.int64)
+    for k in range(colony):
+        tr = trails[k]
+        m = min(D, len(tr) - 1)
+        diff = np.flatnonzero(np.asarray(tr[1:m + 1]) != np.asarray(best[1:m + 1]))
+        dev[k] = diff[0] if len(diff) else m
+    complete = (D == n - 1) & (dev == D)
+    chunk = (max(colony, 1) + world - 1) // world
+    counts, warps = [], []
+    for r in range(world):
+        first, last = min(r * chunk, colony), min((r + 1) * chunk, colony)
+        ants = steps = 0
+        for w0 in range(first, last, 4):
+            present = list(range(w0, min(w0 + 4, last)))
+            done = bool(all(complete[present]))
+            T = min(int(dev[k]) & ~7 for k in present)
+            if done:
+                ants += len(present); steps += len(present) * (n - 1)
+            else:
+                steps += len(present) * T
+            warps.append((r, w0, len(present), T, done))
+        counts.append({"verified_ants": ants, "verified_steps": steps})
+    return counts, {"D": D, "n": n, "dev": dev, "warps": warps}
+
+
+def oracle_step(A, start, goal, cap, dims, table_log2=0, world=1, nonfinite=()):
+    """One oracle iteration and its expected walkStats() increments per shard (expected_walk_stats)."""
+    best = A.best()[0]
+    A.iterate(1)
+    colony = A.last_colony()[0]
+    trails = [A.last_ant(k)[0] for k in range(colony)]
+    return expected_walk_stats(best, trails, start, goal, cap, dims, table_log2, colony, world, nonfinite)
+
+
+def add_stats(total, counts):
+    return [{k: t[k] + c[k] for k in t} for t, c in zip(total, counts)]
+
+
+def _run_vs_oracle(A, g, iters=(1, 1, 1, 1, 12, 14), table_log2=0):
     s, e = _endpoints(A)
     A.set_endpoints(s, e); g.setEndpoints(s, e)
     A.begin(1.0); g.begin(1.0)
+    dims = (g.rangeX, g.rangeY, g.rangeZ)
+    want = [{"verified_ants": 0, "verified_steps": 0}]
     for n in iters:
-        A.iterate(n); g.iterate(n)
+        for _ in range(n):
+            want = add_stats(want, oracle_step(A, s, e, g.stepCap(), dims, table_log2)[0])
+        g.iterate(n)
         compare_iteration(A, g)
+        assert g.walkStats() == want[0]
     oc, gc = A.counters(), g.counters()
     for key in ("ant_steps", "ants", "arrived", "dead_no_candidate", "dead_fallthrough", "dead_step_cap"):
         assert oc[key] == gc[key], key
+    assert g.updateStats()["rankset_iterations"] == sum(iters)
     return gc
 
 
@@ -115,7 +187,7 @@ def test_small_tables_fill_inside_the_verified_prefix(wr, oracle, meshes, monkey
     """16-entry visited tables (12 tiles): the verifiable prefix ends where a table would fill; the rest parks and resumes in HBM."""
     monkeypatch.setenv("WR_RANKSET_POLICY", "1")
     A, g = make_pair(wr, oracle, meshes["simplified_piece"], 0.02, 3, seed=52, fixed_colony=512, step_cap=300, update_mode=4, walk_table_log2=4)
-    gc = _run_vs_oracle(A, g)
+    gc = _run_vs_oracle(A, g, table_log2=4)
     assert gc["table_overflows"] > 0
 
 
