@@ -182,7 +182,17 @@ __global__ void k_gtsp_iterate(GtspArgs a)
                 double rnd = __ddiv_rn((double)(int)r31, 2147483647.0);   // (double)rand()/(double)RAND_MAX (:126)
                 rnd = __dmul_rn(rnd, sum);
                 int iv = -1;
-                for (int j = 0; j < nck; j++) if (ckpt[j * nthreads + k] >= rnd) { iv = j; break; }
+                if (rnd <= 0.0) {
+                    // every prefix sum is >= 0 >= rnd: the reference takes the lowest unvisited city.  The check-point search
+                    // would stop at interval 0 even when all its cities are visited (a zero draw, a zero or subnormal sum),
+                    // so the city comes from the visited words; left > 0 puts it below n.  A NaN rnd skips both branches.
+                    for (int w = 0;; w++) {
+                        const uint32_t fr = ~vis[w * nthreads + k];
+                        if (fr) { next = w * 32 + __ffs(fr) - 1; break; }
+                    }
+                } else {
+                    for (int j = 0; j < nck; j++) if (ckpt[j * nthreads + k] >= rnd) { iv = j; break; }
+                }
                 if (iv >= 0) {
                     double s = iv > 0 ? ckpt[(iv - 1) * nthreads + k] : 0.0;
                     const int c0 = iv * kGtspIv;
