@@ -1433,6 +1433,7 @@ static int alloc_batch(wr_acs* a, int want_q, int cm, int* qc_out)
     const size_t Eg = (size_t)1 << a->gtable_log2_for_cap();
     const size_t gbytes = k26 ? 12 : 8;
     size_t pool = std::min<size_t>(nq * cm, std::max<size_t>(16, ((size_t)2 << 30) / (Eg * gbytes)));
+    if (const char* e = getenv("WR_BATCH_POOL")) pool = std::min<size_t>(pool, (size_t)std::max(1, atoi(e)));
     b->pool = (uint32_t)pool;
     WR_CUDA(cudaMalloc(&b->overflow_list, pool * sizeof(uint32_t)));
     WR_CUDA(cudaMalloc(&b->gtab, pool * Eg * sizeof(unsigned long long)));

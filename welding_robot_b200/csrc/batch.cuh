@@ -180,6 +180,8 @@ struct Batch6 {
         gxv = __ldg(xs + g % rx); gyv = __ldg(ys + (g % rxy) / rx); gzv = __ldg(zs + g / rxy);
         return bq;
     }
+    // parked ants to resume: those beyond the pool got no table (the batch has failed and will be re-run), as Batch26::items
+    __device__ __forceinline__ unsigned items(const BatchArgs& a, const IterState* st) const { return min(st->overflow_n, a.pool); }
     // entry q of the parked-ant list (has = false: no ant, the group idles)
     __device__ __forceinline__ void bind(const BatchArgs& a, unsigned q, bool has)
     {

@@ -77,6 +77,8 @@ struct Dense6 {
           stream_word(a.stream_word), block_hi(a.block_hi)
     {
     }
+    // parked ants to resume: the search has an HBM table for every ant of its colony
+    __device__ __forceinline__ unsigned items(const WalkArgs&, const IterState* st) const { return st->overflow_n; }
     // entry q of the parked-ant list (has = false: no ant, the group idles)
     __device__ __forceinline__ void bind(const WalkArgs& a, unsigned q, bool has)
     {
@@ -134,7 +136,7 @@ __global__ void __launch_bounds__(kWalkThreads) k_walk2(typename In::Args a)
     IterState* st = a.st;
     const uint32_t iter = (uint32_t)st->iter;
     const float base_now = st->base;   // clean-tile field: what a slot that never received a deposit is worth this iteration
-    const unsigned n_items = st->overflow_n;   // the ants pass 1 parked
+    const unsigned n_items = in.items(a, st);   // the ants pass 1 parked (and found a table for)
     const int cap = a.cap;
 
     unsigned long long c_steps = 0, c_ants = 0, c_arrived = 0, c_nocand = 0, c_fall = 0, c_cap = 0;
