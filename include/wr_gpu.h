@@ -179,11 +179,15 @@ int wr_acs_update_stats(wr_acs* a, uint32_t out[4]);
  * [0] ants completed by that check alone, [1] ant-steps it decided, both cumulative since the handle was created */
 int wr_acs_walk_stats(wr_acs* a, uint64_t out[2]);
 /* Clean-tile pheromone field (FUSED / RANKSET handles): [0] 16 KB tiles that hold at least one slot that ever received a
- * deposit since init/reset() — the only tiles the evaporation pass reads and writes — [1] tiles of the field.  Slots that
- * never received a deposit all hold the same value (tau0 * rho per iteration, kept as one scalar); downloads materialise it. */
+ * deposit since init/reset(), [1] tiles of the field.  Slots that never received a deposit all hold the same value
+ * (tau0 * rho per iteration, kept as one scalar); downloads materialise it. */
 int wr_acs_field_stats(wr_acs* a, uint64_t out[2]);
+/* The same at the granule the evaporation pass reads and writes: [0] 128-byte lines (32 slots) that hold at least one slot
+ * that ever received a deposit since init/reset() (every line after an upload or on a materialised field), [1] lines of
+ * the field. */
+int wr_acs_field_lines(wr_acs* a, uint64_t out[2]);
 /* cumulative device ms and launch count, since begin and with timing enabled, of the kernel that streams the pheromone field
- * (k_update_fused or k_evaporate_tiles) measured by its own event pair inside the iteration loop */
+ * (k_update_fused or k_evaporate_lines) measured by its own event pair inside the iteration loop */
 int wr_acs_stream_kernel_ms(wr_acs* a, float* ms, int* launches);
 /* measurement hook: run ONE kernel of the update path `reps` times back to back on the handle's
  * stream and report the average device time per launch (CUDA events).  which: 0 = fused update

@@ -509,9 +509,15 @@ class ACS_Rank(GridMap):
         return ms.value, n.value
 
     def fieldStats(self):
-        """Clean-tile field: (tiles the evaporation pass touches, tiles of the field)."""
+        """Clean-tile field: (16 KB tiles with at least one dirty line, tiles of the field)."""
         out = np.zeros(2, np.uint64)
         check(lib().wr_acs_field_stats(self._need(), ptr(out)))
+        return int(out[0]), int(out[1])
+
+    def fieldLines(self):
+        """Clean-tile field: (128-byte lines the evaporation pass touches, lines of the field)."""
+        out = np.zeros(2, np.uint64)
+        check(lib().wr_acs_field_lines(self._need(), ptr(out)))
         return int(out[0]), int(out[1])
 
     def benchKernel(self, which, reps=20):

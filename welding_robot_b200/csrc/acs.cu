@@ -192,7 +192,7 @@ struct wr_acs {
     // CUDA graph launch: 9 kernels whose arguments do not change within a search; re-captured after wr_acs_begin
     cudaGraphExec_t rs_graph[2] = {nullptr, nullptr};   // sharded handles: one per trail-buffer parity
     bool rs_graph_failed = false;
-    // device time of the streaming kernel alone (k_update_fused / k_evaporate_tiles), inside the loop: event pairs around it
+    // device time of the streaming kernel alone (k_update_fused / k_evaporate_lines), inside the loop: event pairs around it
     std::vector<cudaEvent_t> sk_ev;
     size_t sk_used = 0;
     float sk_ms = 0;
@@ -210,8 +210,11 @@ struct wr_acs {
         }
         sk_used = 0;
     }
-    // clean-tile field (acs_kernels.cuh): per-tile dirty flags; lazy = in-bounds slots start as sentinels (FUSED / RANKSET handles)
+    // clean-tile field (acs_kernels.cuh): per-tile and per-line dirty flags; lazy = in-bounds slots start as sentinels (FUSED / RANKSET handles)
     uint8_t* d_dirty = nullptr;
+    uint8_t* d_lines = nullptr;       // [ntiles * kTileLines]
+    DirtyFlags flags() const { return DirtyFlags{d_dirty, d_lines}; }
+    size_t nlines() const { return (size_t)ntiles * kTileLines; }
     bool lazy = false;
     bool oob_zero = true;             // out-of-bounds slots still hold their initial 0 (until the first reset())
 
@@ -548,7 +551,7 @@ extern "C" int wr_acs_destroy(wr_acs* a)
     cudaStream_t s = a->stream;
     pool_free(a->d_tau, s); pool_free(a->d_heur, s); pool_free(a->d_state, s); pool_free(a->d_onbest, s); pool_free(a->d_Ltab, s);
     pool_free(a->d_best_n, s); pool_free(a->d_best_ids, s); pool_free(a->d_best_dirs, s); pool_free(a->d_tile_off, s); pool_free(a->d_dep_list, s);
-    pool_free(a->d_upd_q, s); pool_free(a->d_dirty, s);
+    pool_free(a->d_upd_q, s); pool_free(a->d_dirty, s); pool_free(a->d_lines, s);
     pool_free(a->d_thr, s); pool_free(a->d_pmap, s); pool_free(a->d_pv, s);
     if (a->stream) cudaStreamSynchronize(a->stream);
     feedback_release(a->h_feedback);
@@ -614,6 +617,8 @@ extern "C" int wr_acs_create(wr_grid* g, const wr_acs_params* p, wr_acs** out)
     }
     WR_CUDA_A(dmalloc(&a->d_dirty, (size_t)a->ntiles + 1, a->stream));
     WR_CUDA_A(cudaMemsetAsync(a->d_dirty, a->lazy ? 0 : 1, (size_t)a->ntiles + 1, a->stream));
+    WR_CUDA_A(dmalloc(&a->d_lines, a->nlines(), a->stream));
+    WR_CUDA_A(cudaMemsetAsync(a->d_lines, a->lazy ? 0 : 1, a->nlines(), a->stream));
     {
         const float init_val = a->lazy ? -0.0f : p->tau0;   // -0.0f: the sentinel (kSentinelBits)
         if (a->K == kK26) k_tau_init26<<<(unsigned)((a->n_slots + 255) / 256), 256, 0, a->stream>>>(a->d_tau, g->rx, g->ry, g->rz, a->N, init_val);
@@ -936,9 +941,9 @@ static int launch_fused(wr_acs* a, const uint32_t* ck, const uint32_t* cv, const
     k_tile_offsets<<<(a->ntiles + 1 + 255) / 256, 256, 0, s>>>(d_n ? d_n : a->dptr_nrec(), ck, a->d_tile_off, a->ntiles, a->d_dep_list, a->d_upd_q + 2);
     if (a->timer.enabled) cudaEventRecord(a->sk_next(), s);
     if (fin) k_update_fused<true><<<kNumSMs * kFusedCtasPerSm, kUpdThreads, 0, s>>>(a->d_tau, a->ntiles, a->p.rho, ck, cv, a->d_tile_off, a->d_dep_list, a->d_upd_q, fin, stream_cs(),
-                                                                                      a->d_state, a->d_dirty);
+                                                                                      a->d_state, a->flags());
     else k_update_fused<false><<<kNumSMs * kFusedCtasPerSm, kUpdThreads, 0, s>>>(a->d_tau, a->ntiles, a->p.rho, ck, cv, a->d_tile_off, a->d_dep_list, a->d_upd_q, nullptr, stream_cs(),
-                                                                                 a->d_state, a->d_dirty);
+                                                                                 a->d_state, a->flags());
     if (a->timer.enabled) cudaEventRecord(a->sk_next(), s);
     WR_CUDA(cudaGetLastError());
     return WR_OK;
@@ -1001,15 +1006,15 @@ static int launch_rankset_update(wr_acs* a)
         a->evap_forked = false;
     } else {
         if (a->timer.enabled) cudaEventRecord(a->sk_next(), s);
-        k_evaporate_tiles<<<kNumSMs * 8, 256, 0, s>>>(reinterpret_cast<float4*>(a->d_tau), a->ntiles, a->p.rho, a->d_dirty, stream_cs());
+        k_evaporate_lines<<<kNumSMs * kEvapCtasPerSm, 256, 0, s>>>(reinterpret_cast<float4*>(a->d_tau), a->ntiles, a->p.rho, a->d_lines, stream_cs());
         if (a->timer.enabled) cudaEventRecord(a->sk_next(), s);
     }
     // ordered chains (all rank groups in one launch), wipe; on overflow of the fixed-capacity table (flag raised by gen / merge)
     // the chains are skipped, the whole table is swept and k_deposit_serial applies the deposits in the reference's own loop order
-    k_rankset_apply<<<kNumSMs * 4, 256, 0, s>>>(a->d_state, a->d_tau, a->rs, a->p.rho, a->d_dirty, a->rs_groups);
+    k_rankset_apply<<<kNumSMs * 4, 256, 0, s>>>(a->d_state, a->d_tau, a->rs, a->p.rho, a->flags(), a->rs_groups);
     if (a->rs_groups > 1) k_rankset_clear<<<kNumSMs * 2, 256, 0, s>>>(a->d_state, a->rs);
     k_deposit_serial<<<1, 1024, 0, s>>>(a->d_state, rank_keys(a), rank_vals(a), a->trail_ids_tab(), a->trail_dirs_tab(), a->cap, a->chunk, (int)a->goal, a->d_Ltab,
-                                        a->d_onbest, a->rs.count + 3, a->d_tau, a->p.rho, a->d_dirty, a->K, a->K == kK26 ? a->d_ant_steps : nullptr);
+                                        a->d_onbest, a->rs.count + 3, a->d_tau, a->p.rho, a->flags(), a->K, a->K == kK26 ? a->d_ant_steps : nullptr);
     WR_CUDA(cudaGetLastError());
     return WR_OK;
 }
@@ -1037,7 +1042,7 @@ static int launch_record_update_sharded(wr_acs* a)
     st = launch_fused(a, ck, cv, a->d_nq, fin);
     if (st != WR_OK) return st;
     k_pull_finals<<<barrier_grid(a, kNumSMs * 2), 256, 0, s>>>(barrier_args(a), a->d_state, a->d_tau, reinterpret_cast<const uint32_t* const*>(a->tab(2, a->parity)),
-                                                                a->nranks, a->rank, a->d_dirty, a->d_upd_q);
+                                                                a->nranks, a->rank, a->flags(), a->d_upd_q);
     WR_CUDA(cudaGetLastError());
     return WR_OK;
 }
@@ -1080,7 +1085,7 @@ static int launch_construct_and_rank(wr_acs* a, bool rankset_iteration)
         WR_CUDA(cudaEventRecord(a->ev_fork, s));
         WR_CUDA(cudaStreamWaitEvent(a->side, a->ev_fork, 0));
         if (a->timer.enabled) cudaEventRecord(a->sk_next(), a->side);
-        k_evaporate_tiles<<<kNumSMs * 8, 256, 0, a->side>>>(reinterpret_cast<float4*>(a->d_tau), a->ntiles, a->p.rho, a->d_dirty, stream_cs());
+        k_evaporate_lines<<<kNumSMs * kEvapCtasPerSm, 256, 0, a->side>>>(reinterpret_cast<float4*>(a->d_tau), a->ntiles, a->p.rho, a->d_lines, stream_cs());
         if (a->timer.enabled) cudaEventRecord(a->sk_next(), a->side);
         WR_CUDA(cudaEventRecord(a->ev_join, a->side));
         a->evap_forked = true;
@@ -1104,7 +1109,7 @@ static int launch_construct_and_rank(wr_acs* a, bool rankset_iteration)
 
 // One rank-set iteration whose predecessor was a rank-set iteration too, captured from the very launch sequence of
 // wr_acs_iterate (k_iter_end of the predecessor folded into k_iter_begin): iteration parameters, walk pass 1 + 2,
-// ranking, best copy, rank-set build, evaporation of the dirty tiles, ordered chains.  Every argument is fixed for the search
+// ranking, best copy, rank-set build, evaporation of the dirty lines, ordered chains.  Every argument is fixed for the search
 // (sharded handles alternate between two trail buffers, hence one graph per parity).
 static int capture_steady_iteration(wr_acs* a, cudaGraphExec_t* out)
 {
@@ -1579,7 +1584,7 @@ static int preload_iteration_kernels()
 #define WR_PRELOAD(f) WR_CUDA(cudaFuncGetAttributes(&at, f))
     WR_PRELOAD(k_gather_steps); WR_PRELOAD(k_rank_small); WR_PRELOAD(k_rank_chunks); WR_PRELOAD(k_rank_merge);
     WR_PRELOAD(k_rank_finish_prefix); WR_PRELOAD(k_best_copy_peer); WR_PRELOAD(k_best_copy); WR_PRELOAD(k_rankset_gen); WR_PRELOAD(k_rankset_publish);
-    WR_PRELOAD(k_rankset_merge); WR_PRELOAD(k_evaporate_tiles); WR_PRELOAD(k_rankset_apply); WR_PRELOAD(k_rankset_clear); WR_PRELOAD(k_deposit_serial);
+    WR_PRELOAD(k_rankset_merge); WR_PRELOAD(k_evaporate_lines); WR_PRELOAD(k_rankset_apply); WR_PRELOAD(k_rankset_clear); WR_PRELOAD(k_deposit_serial);
     WR_PRELOAD((k_deposit_gen<false, true>)); WR_PRELOAD(k_tile_offsets); WR_PRELOAD(k_update_fused<true>); WR_PRELOAD(k_update_fused<false>);
     WR_PRELOAD(k_pull_finals); WR_PRELOAD(k_iter_begin); WR_PRELOAD(k_iter_end);
     WR_PRELOAD((k_walk3<true, 0>)); WR_PRELOAD((k_walk3<true, 1>)); WR_PRELOAD((k_walk3<false, 0>)); WR_PRELOAD((k_walk3<false, 1>));
@@ -1692,8 +1697,8 @@ extern "C" int wr_acs_reset(wr_acs* a)
 {   // reset() :307-315: every slot (out-of-bounds ones included) back to tau0
     WR_REQUIRE(a, WR_ERR_INVALID, "wr_acs_reset: null");
     WR_CUDA(cudaSetDevice(a->device));
-    if (a->lazy) {   // clean-tile field: back to all-sentinel with base = tau0; after the first reset only the dirty tiles need rewriting
-        k_tau_reset_tiles<<<kNumSMs * 8, 256, 0, a->stream>>>(reinterpret_cast<float4*>(a->d_tau), a->ntiles, a->d_dirty, a->oob_zero ? 1 : 0);
+    if (a->lazy) {   // clean-tile field: back to all-sentinel with base = tau0; after the first reset only the dirty lines need rewriting
+        k_tau_reset_lines<<<kNumSMs * 8, 256, 0, a->stream>>>(reinterpret_cast<float4*>(a->d_tau), a->ntiles, a->flags(), a->oob_zero ? 1 : 0);
         a->oob_zero = false;
     } else {
         k_tau_fill<<<kNumSMs * 8, 256, 0, a->stream>>>(a->d_tau, a->n_slots, a->p.tau0);
@@ -1759,7 +1764,8 @@ extern "C" int wr_acs_upload_pheromone(wr_acs* a, const float* tau, size_t n)
     } else {
         WR_CUDA(cudaMemcpy(a->d_tau, tau, a->n_slots * sizeof(float), cudaMemcpyHostToDevice));
     }
-    WR_CUDA(cudaMemset(a->d_dirty, 1, (size_t)a->ntiles + 1));   // explicit values everywhere: every tile takes part in the evaporation
+    WR_CUDA(cudaMemset(a->d_dirty, 1, (size_t)a->ntiles + 1));   // explicit values everywhere: every line takes part in the evaporation
+    WR_CUDA(cudaMemset(a->d_lines, 1, a->nlines()));
     a->field_clean = false;
     return WR_OK;
 }
@@ -1874,6 +1880,18 @@ extern "C" int wr_acs_field_stats(wr_acs* a, uint64_t out[2])
     uint64_t n = 0;
     for (uint8_t v : h) n += v ? 1 : 0;
     out[0] = n; out[1] = a->ntiles;
+    return WR_OK;
+}
+
+extern "C" int wr_acs_field_lines(wr_acs* a, uint64_t out[2])
+{
+    WR_REQUIRE(a && out, WR_ERR_INVALID, "wr_acs_field_lines: null");
+    WR_CUDA(cudaStreamSynchronize(a->stream));
+    std::vector<uint8_t> h(a->nlines());
+    WR_CUDA(cudaMemcpy(h.data(), a->d_lines, h.size(), cudaMemcpyDeviceToHost));
+    uint64_t n = 0;
+    for (uint8_t v : h) n += v ? 1 : 0;
+    out[0] = n; out[1] = h.size();
     return WR_OK;
 }
 

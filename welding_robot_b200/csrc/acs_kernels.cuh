@@ -33,9 +33,21 @@ constexpr int kUpdThreads = 256;
 // walk step); the first deposit on a slot starts its chain from the base of that iteration, exactly the value the
 // reference's slot holds at that point, and marks the tile dirty for good.  Bits are identical by construction; what is
 // saved is the traffic of every tile the colony never touched (most of a 512^3 field).
+// The same rule holds per 128-byte line (32 slots), and that is the granule the passes skip at: a wandering colony leaves
+// scattered single deposits in ~40 % of the tiles but only ~8 % of the lines, and the set stops growing once the colony
+// converges.  Every writer of a non-sentinel value marks the slot's line AND its tile (plain byte stores of 1, no
+// atomics); the tile byte is a summary (any of its lines dirty) that fieldStats() counts and the tile-level passes test.
 // ------------------------------------------------------------------------------------------
 constexpr uint32_t kSentinelBits = 0x80000000u;
 __device__ __forceinline__ float tau_or_base(float v, float base) { return __float_as_uint(v) == kSentinelBits ? base : v; }
+
+constexpr int kLineSlots = 32;                             // floats per 128-byte line
+constexpr int kTileLines = kUpdTile / kLineSlots;          // 128 lines per tile
+struct DirtyFlags {
+    uint8_t* tile;   // [ntiles + 1]     1: some line of the tile is dirty
+    uint8_t* line;   // [ntiles * 128]   1: the line holds (or held since the last reset()) a value that is not a sentinel
+    __device__ __forceinline__ void mark(uint32_t slot) const { line[slot / (uint32_t)kLineSlots] = 1; tile[slot / (uint32_t)kUpdTile] = 1; }
+};
 
 struct WalkArgs {
     IterState* st;
@@ -354,16 +366,24 @@ __global__ void __launch_bounds__(128) k_deposit_gen(const IterState* st, const 
 // EMIT (sharded colonies, owner-computes): every finished run also appends (slot, final value) to `fin` — the list the
 // other ranks pull over NVLink instead of redoing this rank's chains (fin[0] = count, records from word 4).
 // sent_val: what a slot that still holds the clean-field sentinel is worth after this iteration's evaporation (base * rho).
+// lines (clean-tile field, base = 0): the line flags.  The head of the first run in each line marks it (one byte store per
+// line, not per slot); the caller marks the tile.
 template <bool EMIT = false>
 __device__ __forceinline__ void apply_runs(float* buf, uint32_t base, const uint32_t* __restrict__ keys, const uint32_t* __restrict__ vals,
-                                           uint32_t lo, uint32_t hi, uint32_t first, uint32_t stride, uint32_t* fin = nullptr, float sent_val = 0.0f)
+                                           uint32_t lo, uint32_t hi, uint32_t first, uint32_t stride, uint32_t* fin = nullptr, float sent_val = 0.0f,
+                                           uint8_t* lines = nullptr)
 {
     const int lane = threadIdx.x & 31;
     for (uint32_t r0 = lo + first; r0 < hi; r0 += stride) {   // r0 is warp-uniform: all 32 lanes run the same trips
         const uint32_t r = r0 + lane;
         bool head = r < hi;
         uint32_t key = 0;
-        if (head) { key = keys[r]; head = (r == lo) || keys[r - 1] != key; }
+        if (head) {
+            key = keys[r];
+            const uint32_t prev = r == lo ? ~0u : keys[r - 1];
+            head = (r == lo) || prev != key;
+            if (lines && (r == lo || prev / (uint32_t)kLineSlots != key / (uint32_t)kLineSlots)) lines[key / (uint32_t)kLineSlots] = 1;
+        }
         float x = 0.0f;
         uint32_t j = r;
         bool more = false;
@@ -468,20 +488,53 @@ __global__ void __launch_bounds__(256) k_evaporate(float4* __restrict__ tau4, si
     }
 }
 
-// The same pass over the DIRTY tiles of a clean-tile field only (16 KB tiles, four float4 in flight per thread).
-__global__ void __launch_bounds__(256) k_evaporate_tiles(float4* __restrict__ tau4, unsigned ntiles, float rho, const uint8_t* __restrict__ dirty, int cs)
+// The same pass over the dirty LINES of a clean-tile field only.  One warp per 16 KB tile: each lane reads 4 of the tile's
+// 128 line flags (one coalesced 128-byte load, the next tile's already in flight), the warp compacts the dirty lines into a
+// shared list and streams them 16 lines per round — 8 lanes x float4 per line, 4 independent loads per lane before the first
+// store.  A tile without dirty lines costs its flag load and nothing else.
+constexpr int kEvapLinesPerRound = 16;
+constexpr int kEvapCtasPerSm = 6;   // 40 registers; the grid is one wave of them
+__global__ void __launch_bounds__(256, kEvapCtasPerSm) k_evaporate_lines(float4* __restrict__ tau4, unsigned ntiles, float rho, const uint8_t* __restrict__ lines, int cs)
 {
-    for (unsigned t = blockIdx.x; t < ntiles; t += gridDim.x) {
-        if (!dirty[t]) continue;
-        float4* p = tau4 + ((size_t)t << 10) + threadIdx.x;
-        float4 v[4];
+    constexpr unsigned FULL = 0xffffffffu;
+    __shared__ uint8_t s_list[8][kTileLines];
+    const int lane = threadIdx.x & 31;
+    uint8_t* list = s_list[threadIdx.x >> 5];
+    const uint32_t* flags = reinterpret_cast<const uint32_t*>(lines) + lane;   // lines 4*lane .. 4*lane+3 of a tile
+    const unsigned stride = gridDim.x * 8u;
+    unsigned t = blockIdx.x * 8u + (threadIdx.x >> 5);
+    uint32_t f = t < ntiles ? flags[(size_t)t * 32] : 0u;
+    for (; t < ntiles; t += stride) {   // warp-uniform
+        const uint32_t fn = t + stride < ntiles ? flags[(size_t)(t + stride) * 32] : 0u;
+        int n = 0;
 #pragma unroll
-        for (int j = 0; j < 4; j++) v[j] = cs ? __ldcs(p + 256 * j) : p[256 * j];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            v[j].x = __fmul_rn(v[j].x, rho); v[j].y = __fmul_rn(v[j].y, rho); v[j].z = __fmul_rn(v[j].z, rho); v[j].w = __fmul_rn(v[j].w, rho);
-            if (cs) __stcs(p + 256 * j, v[j]); else p[256 * j] = v[j];
+        for (int k = 0; k < 4; k++) {
+            const bool d = (f >> (8 * k)) & 0xFFu;
+            const unsigned m = __ballot_sync(FULL, d);
+            if (d) list[n + __popc(m & ((1u << lane) - 1u))] = (uint8_t)(4 * lane + k);
+            n += __popc(m);
         }
+        f = fn;
+        if (n == 0) continue;
+        __syncwarp();
+        float4* tile = tau4 + ((size_t)t << 10) + (lane & 7);
+        for (int b = 0; b < n; b += kEvapLinesPerRound) {
+            float4 v[4];
+            int o[4];   // float4 offset of this lane's part of line j of the round in the tile, -1: none
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                const int i = b + 4 * j + (lane >> 3);
+                o[j] = i < n ? 8 * list[i] : -1;
+                if (o[j] >= 0) v[j] = cs ? __ldcs(tile + o[j]) : tile[o[j]];
+            }
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                if (o[j] < 0) continue;
+                v[j].x = __fmul_rn(v[j].x, rho); v[j].y = __fmul_rn(v[j].y, rho); v[j].z = __fmul_rn(v[j].z, rho); v[j].w = __fmul_rn(v[j].w, rho);
+                if (cs) __stcs(tile + o[j], v[j]); else tile[o[j]] = v[j];
+            }
+        }
+        __syncwarp();   // the list is rewritten for the next tile
     }
 }
 
@@ -535,16 +588,22 @@ constexpr int kFusedChunk = 8;       // plain tiles per queue grab (128 KB)
 
 // CS: streaming (evict-first) loads and stores for tiles nobody touches again this iteration, so that the pass does not
 // leave L2 full of dirty pheromone lines when the next walk starts gathering rows.
+// lf: the tile's 128 line flags (shared memory); only dirty lines are moved.  nullptr: the whole tile.
 template <bool CS = false>
-__device__ __forceinline__ void stream_tile(float* tau, unsigned t, float rho, int tid)
+__device__ __forceinline__ void stream_tile(float* tau, unsigned t, float rho, int tid, const uint8_t* lf = nullptr)
 {
     constexpr int kVec = kUpdTile / 4 / kUpdThreads;   // float4 per thread per tile
     float4* g4 = reinterpret_cast<float4*>(tau + (size_t)t * kUpdTile);
     float4 v[kVec];
+    bool on[kVec];
 #pragma unroll
-    for (int j = 0; j < kVec; j++) v[j] = CS ? __ldcs(g4 + j * kUpdThreads + tid) : g4[j * kUpdThreads + tid];
+    for (int j = 0; j < kVec; j++) {   // float4 j * kUpdThreads + tid lies in line j * (kUpdThreads / 8) + tid / 8
+        on[j] = !lf || lf[j * (kUpdThreads / 8) + (tid >> 3)];
+        if (on[j]) v[j] = CS ? __ldcs(g4 + j * kUpdThreads + tid) : g4[j * kUpdThreads + tid];
+    }
 #pragma unroll
     for (int j = 0; j < kVec; j++) {
+        if (!on[j]) continue;
         v[j].x = __fmul_rn(v[j].x, rho); v[j].y = __fmul_rn(v[j].y, rho); v[j].z = __fmul_rn(v[j].z, rho); v[j].w = __fmul_rn(v[j].w, rho);
         if (CS) __stcs(g4 + j * kUpdThreads + tid, v[j]); else g4[j * kUpdThreads + tid] = v[j];
     }
@@ -559,11 +618,13 @@ __global__ void __launch_bounds__(kUpdThreads, kFusedCtasPerSm) k_update_fused(f
                                                                                 const uint32_t* __restrict__ rec_vals,
                                                                                 const uint32_t* __restrict__ tile_off,
                                                                                 const uint32_t* __restrict__ dep_list, uint32_t* q, uint32_t* fin,
-                                                                                int cs, const IterState* st, uint8_t* dirty)
-{   // dirty[t] = 0: tile t is clean (sentinels and exact zeros only) and is neither read nor written; see "Clean-tile pheromone field"
+                                                                                int cs, const IterState* st, DirtyFlags dirty)
+{   // a clean tile or line (sentinels and exact zeros only) is neither read nor written; see "Clean-tile pheromone field"
+    static_assert(kFusedChunk * kTileLines == 4 * kUpdThreads, "one word of line flags per thread and chunk");
     const float base_new = __fmul_rn(st->base, rho);
     __shared__ unsigned s_next;
     __shared__ uint32_t s_off[kFusedChunk + 1];
+    __shared__ uint32_t s_lines[kFusedChunk * kTileLines / 4];
     const int tid = threadIdx.x;
     const unsigned dep_n = q[2];
     if (EMIT && blockIdx.x == 0 && tid == 0) fin[1] = dep_n;   // sharded: this rank's share of the "tiles that received deposits" statistic
@@ -575,21 +636,25 @@ __global__ void __launch_bounds__(kUpdThreads, kFusedCtasPerSm) k_update_fused(f
         if (i >= dep_n) break;
         const unsigned t = dep_list[i];
         const uint32_t lo = tile_off[t], hi = tile_off[t + 1];
-        if (dirty[t]) stream_tile(tau, t, rho, tid);   // CTA-uniform
+        if (dirty.tile[t]) stream_tile(tau, t, rho, tid);   // CTA-uniform; the clean lines of the tile are streamed too (harmless: rho keeps them)
         __syncthreads();   // the scaled tile is visible to the whole CTA
-        apply_runs<EMIT>(tau, 0u, rec_keys, rec_vals, lo, hi, (uint32_t)(tid & ~31), (uint32_t)kUpdThreads, fin, base_new);
-        if (tid == 0) dirty[t] = 1;
+        apply_runs<EMIT>(tau, 0u, rec_keys, rec_vals, lo, hi, (uint32_t)(tid & ~31), (uint32_t)kUpdThreads, fin, base_new, dirty.line);
+        if (tid == 0) dirty.tile[t] = 1;
     }
     while (true) {   // ---- everything else: pure streaming ----
         if (tid == 0) s_next = atomicAdd(&q[1], (unsigned)kFusedChunk);
         __syncthreads();
         const unsigned c0 = s_next;
         if (c0 < ntiles && tid <= kFusedChunk) s_off[tid] = tile_off[min(c0 + tid, ntiles)];
+        if (c0 < ntiles) s_lines[tid] = c0 + tid / 32u < ntiles ? reinterpret_cast<const uint32_t*>(dirty.line)[(size_t)c0 * 32 + tid] : 0u;
         __syncthreads();
         if (c0 >= ntiles) break;
         const unsigned c1 = min(c0 + kFusedChunk, ntiles);
+        const uint8_t* lf = reinterpret_cast<const uint8_t*>(s_lines);
         for (unsigned t = c0; t < c1; t++)
-            if (s_off[t - c0] == s_off[t - c0 + 1] && dirty[t]) { if (cs) stream_tile<true>(tau, t, rho, tid); else stream_tile<false>(tau, t, rho, tid); }
+            if (s_off[t - c0] == s_off[t - c0 + 1] && dirty.tile[t]) {
+                if (cs) stream_tile<true>(tau, t, rho, tid, lf + (t - c0) * kTileLines); else stream_tile<false>(tau, t, rho, tid, lf + (t - c0) * kTileLines);
+            }
         __syncthreads();   // s_off / s_next are reused by the next grab
     }
 }
@@ -656,7 +721,7 @@ __global__ void k_save_result(const IterState* st, const int* __restrict__ best_
 // The same pass is the next walk's L2 warm-up: the slots that just received deposits are where the colony walks next, so
 // the tau lines are left in L2 — the other ranks' by the writes, this rank's own slice by a touch.
 __global__ void __launch_bounds__(256) k_pull_finals(PeerBarrier pb, const IterState* st, float* tau, const uint32_t* const* __restrict__ bufs, int npeers,
-                                                      int me, uint8_t* dirty, uint32_t* upd_q)
+                                                      int me, DirtyFlags dirty, uint32_t* upd_q)
 {
     peer_barrier(pb, st, 2u);   // every rank's list of final values is complete
     uint32_t acc = 0;
@@ -671,7 +736,7 @@ __global__ void __launch_bounds__(256) k_pull_finals(PeerBarrier pb, const IterS
         const uint2* rec = reinterpret_cast<const uint2*>(buf + 4);
         for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < cnt; i += gridDim.x * blockDim.x) {
             const uint2 r = __ldcg(rec + i);
-            if (p != me) { tau[r.x] = __uint_as_float(r.y); dirty[r.x / (uint32_t)kUpdTile] = 1; }
+            if (p != me) { tau[r.x] = __uint_as_float(r.y); dirty.mark(r.x); }
             else acc ^= __ldcg(reinterpret_cast<const uint32_t*>(tau) + r.x);
         }
     }
@@ -695,19 +760,22 @@ __global__ void k_tau_fill(float* tau, size_t n, float v)
 {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) tau[i] = v;
 }
-// reset() on a clean-tile field: every slot back to "tau0" = the sentinel with base = tau0.  all = 0: only the dirty tiles
-// need rewriting (after the first reset() the out-of-bounds slots hold the sentinel too, like the reference's, :307-315).
-__global__ void __launch_bounds__(256) k_tau_reset_tiles(float4* __restrict__ tau4, unsigned ntiles, uint8_t* __restrict__ dirty, int all)
+// reset() on a clean-tile field: every slot back to "tau0" = the sentinel with base = tau0, every flag back to 0.  all = 0:
+// only the dirty lines of the dirty tiles need rewriting (after the first reset() the out-of-bounds slots hold the sentinel
+// too, like the reference's, :307-315); all = 1: every line.
+__global__ void __launch_bounds__(256) k_tau_reset_lines(float4* __restrict__ tau4, unsigned ntiles, DirtyFlags dirty, int all)
 {
     const float s = __uint_as_float(kSentinelBits);
     const float4 v = make_float4(s, s, s, s);
     for (unsigned t = blockIdx.x; t < ntiles; t += gridDim.x) {
-        if (!all && !dirty[t]) continue;
+        if (!all && !dirty.tile[t]) continue;
         float4* p = tau4 + ((size_t)t << 10) + threadIdx.x;
+        const uint8_t* lf = dirty.line + (size_t)t * kTileLines + threadIdx.x / 8;
 #pragma unroll
-        for (int j = 0; j < 4; j++) p[256 * j] = v;
-        __syncthreads();
-        if (threadIdx.x == 0) dirty[t] = 0;
+        for (int j = 0; j < 4; j++) if (all || lf[32 * j]) p[256 * j] = v;
+        __syncthreads();   // every flag of the tile has been read
+        if (threadIdx.x < kTileLines / 4) reinterpret_cast<uint32_t*>(dirty.line)[(size_t)t * (kTileLines / 4) + threadIdx.x] = 0u;
+        if (threadIdx.x == 0) dirty.tile[t] = 0;
     }
 }
 // clean-tile form: the host passes the sentinel as tau0 (the in-bounds slots' value is then IterState::base)

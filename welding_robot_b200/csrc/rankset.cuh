@@ -21,7 +21,7 @@
 //                     find or claim the block of (slot, rank >> 10), set bit (rank & 1023); claimed blocks -> `list`
 //   k_rankset_publish / k_rankset_merge   sharded colonies: the claimed blocks (key + 32 words) are copied to the peer
 //                     slab, and every rank ORs every peer's blocks into its own table
-//   k_evaporate_tiles (acs_kernels.cuh) tau *= rho over the dirty tiles, :268-272 — the one HBM stream of the update
+//   k_evaporate_lines (acs_kernels.cuh) tau *= rho over the dirty lines, :268-272 — the one HBM stream of the update
 //   k_rankset_apply   per slot, the block of its lowest group leads: it adds the ranks' values of group 0, 1, 2 ... to
 //                     tau[slot] in ascending rank order (the higher groups' blocks are looked up) = the reference's
 //                     additions in the reference's order; then the blocks and keys are wiped for the next iteration
@@ -194,7 +194,7 @@ __device__ __forceinline__ uint32_t rankset_find(const RankSet& rs, unsigned lon
 // contribute +0, the identity of the chain.
 // groups_max == 1 (colonies up to 5120 ants): no look-ups happen, so every block is wiped as soon as it is consumed;
 // otherwise k_rankset_clear follows (a wipe during the look-ups would cut other slots' probe chains).
-__global__ void __launch_bounds__(256) k_rankset_apply(const IterState* st, float* tau, RankSet rs, float rho, uint8_t* dirty, int groups_max)
+__global__ void __launch_bounds__(256) k_rankset_apply(const IterState* st, float* tau, RankSet rs, float rho, DirtyFlags dirty, int groups_max)
 {
     if (!st->use_rankset) return;
     const bool overflow = rs.count[3] != 0u;   // the table is incomplete: wipe only, k_deposit_serial applies the deposits
@@ -252,7 +252,7 @@ __global__ void __launch_bounds__(256) k_rankset_apply(const IterState* st, floa
                 }
             }
             tau[slot] = x;
-            dirty[slot / (uint32_t)kUpdTile] = 1;
+            dirty.mark(slot);
         }
         unsigned hm = __ballot_sync(FULL, heavy);
         while (hm) {
@@ -287,7 +287,7 @@ __global__ void __launch_bounds__(256) k_rankset_apply(const IterState* st, floa
                     for (int i = 0; i < 32; i++) x = __fadd_rn(x, __shfl_sync(FULL, v[w], i));
                 }
             }
-            if (lane == 0) { tau[ss] = x; dirty[ss / (uint32_t)kUpdTile] = 1; }
+            if (lane == 0) { tau[ss] = x; dirty.mark(ss); }
         }
         __syncwarp();
         if (has && wipe_here) {   // leave the table empty for the next iteration
@@ -344,7 +344,7 @@ __global__ void __launch_bounds__(256) k_rankset_clear(const IterState* st, Rank
 __global__ void __launch_bounds__(1024) k_deposit_serial(const IterState* st, const uint32_t* __restrict__ rank_keys, const uint32_t* __restrict__ rank_vals,
                                                           const uint32_t* const* __restrict__ ids_tab, const uint8_t* const* __restrict__ dirs_tab, int cap,
                                                           int shard_chunk, int goal, const float* __restrict__ Ltab, const uint32_t* __restrict__ onbest,
-                                                          const uint32_t* __restrict__ over, float* tau, float rho, uint8_t* dirty, int K,
+                                                          const uint32_t* __restrict__ over, float* tau, float rho, DirtyFlags dirty, int K,
                                                           const int* __restrict__ steps26)
 {
     if (!st->use_rankset || *over == 0u) return;
@@ -367,7 +367,7 @@ __global__ void __launch_bounds__(1024) k_deposit_serial(const IterState* st, co
             const bool onb = ((onbest[node >> 5] >> (node & 31)) & 1u) && ((onbest[next >> 5] >> (next & 31)) & 1u);
             const uint32_t slot = node * (uint32_t)K + pdir[i];
             tau[slot] = __fadd_rn(tau_or_base(tau[slot], base_new), onb ? with_elite : without);
-            dirty[slot / (uint32_t)kUpdTile] = 1;
+            dirty.mark(slot);
         }
         __syncthreads();
     }
