@@ -175,6 +175,9 @@ int wr_acs_set_timing(wr_acs* a, int enabled);
 /* WR_UPDATE_RANKSET: [0] the last iteration took the rank-set path, [1] pheromone tiles that received deposits in the last
  * record-path iteration, [2] distinct slots in the last rank-set iteration, [3] rank-set iterations since begin */
 int wr_acs_update_stats(wr_acs* a, uint32_t out[4]);
+/* Group deposits of converged rank-set iterations: [0] eligible ranks of the last iteration whose ant walked exactly the best
+ * path (verified, WR_WALK_VERIFY) and whose rank bits were therefore set once per best-path slot, [1] the same summed since begin */
+int wr_acs_group_stats(wr_acs* a, uint64_t out[2]);
 /* Converged iterations check the best path against roulette thresholds instead of walking it (WR_WALK_VERIFY, default on):
  * [0] ants completed by that check alone, [1] ant-steps it decided, both cumulative since the handle was created */
 int wr_acs_walk_stats(wr_acs* a, uint64_t out[2]);

@@ -36,7 +36,7 @@ wr_grid_create_from_triangles wr_grid_create_from_occupancy wr_grid_destroy wr_g
 wr_grid_bbox wr_grid_coords wr_grid_download_bits wr_grid_download_isfree wr_grid_stats
 wr_acs_default_params wr_acs_create wr_acs_destroy wr_acs_set_points wr_acs_set_endpoints wr_acs_snap_points wr_acs_search_pairs wr_acs_search_batch wr_acs_result_path wr_acs_batch_stats wr_acs_begin wr_acs_set_next_search
 wr_acs_iterate wr_acs_sync wr_acs_reset wr_acs_best wr_acs_download_pheromone wr_acs_upload_pheromone
-wr_acs_last_colony wr_acs_last_ant wr_acs_counters wr_acs_kernel_ms wr_acs_update_stats wr_acs_walk_stats wr_acs_field_stats wr_acs_field_lines wr_acs_stream_kernel_ms wr_acs_set_timing wr_acs_bench_kernel wr_acs_set_stream
+wr_acs_last_colony wr_acs_last_ant wr_acs_counters wr_acs_kernel_ms wr_acs_update_stats wr_acs_group_stats wr_acs_walk_stats wr_acs_field_stats wr_acs_field_lines wr_acs_stream_kernel_ms wr_acs_set_timing wr_acs_bench_kernel wr_acs_set_stream
 wr_comm_unique_id wr_acs_comm_init wr_acs_set_shard wr_acs_peer_export wr_acs_peer_import wr_acs_peer_set_pointers
 wr_gtsp_create wr_gtsp_destroy wr_gtsp_iterate wr_gtsp_solve wr_gtsp_sync wr_gtsp_best wr_gtsp_download_pheromone wr_gtsp_tau0
 wr_gtsp_kernel_ms wr_bspline_eval""".split()
@@ -77,7 +77,7 @@ def lib():
         "wr_acs_begin": [vp, f32], "wr_acs_set_next_search": [vp, C.c_uint32], "wr_acs_iterate": [vp, i32], "wr_acs_sync": [vp], "wr_acs_reset": [vp],
         "wr_acs_best": [vp, vp, vp, i32, vp, vp], "wr_acs_download_pheromone": [vp, vp, C.c_size_t],
         "wr_acs_upload_pheromone": [vp, vp, C.c_size_t], "wr_acs_last_colony": [vp, vp, vp, vp],
-        "wr_acs_last_ant": [vp, i32, vp, vp, i32, vp, vp, vp], "wr_acs_counters": [vp, vp], "wr_acs_kernel_ms": [vp, vp], "wr_acs_update_stats": [vp, vp], "wr_acs_walk_stats": [vp, vp], "wr_acs_field_stats": [vp, vp], "wr_acs_field_lines": [vp, vp], "wr_acs_stream_kernel_ms": [vp, vp, vp],
+        "wr_acs_last_ant": [vp, i32, vp, vp, i32, vp, vp, vp], "wr_acs_counters": [vp, vp], "wr_acs_kernel_ms": [vp, vp], "wr_acs_update_stats": [vp, vp], "wr_acs_group_stats": [vp, vp], "wr_acs_walk_stats": [vp, vp], "wr_acs_field_stats": [vp, vp], "wr_acs_field_lines": [vp, vp], "wr_acs_stream_kernel_ms": [vp, vp, vp],
         "wr_acs_set_timing": [vp, i32], "wr_acs_bench_kernel": [vp, i32, i32, vp], "wr_acs_set_stream": [vp, vp], "wr_acs_set_shard": [vp, i32, i32],
         "wr_comm_unique_id": [vp], "wr_acs_comm_init": [vp, vp, i32, i32],
         "wr_acs_peer_export": [vp, vp, vp], "wr_acs_peer_import": [vp, vp], "wr_acs_peer_set_pointers": [vp, vp],

@@ -490,10 +490,15 @@ class ACS_Rank(GridMap):
         return dict(walk=float(out[0]), rank=float(out[1]), deposit_build=float(out[2]), update=float(out[3]), total=float(out[4]))
 
     def updateStats(self):
-        """WR_UPDATE_RANKSET: which deposit path the last iteration took and how concentrated the deposits were."""
+        """WR_UPDATE_RANKSET: which deposit path the last iteration took and how concentrated the deposits were; group_ranks:
+        eligible ranks of the last iteration whose bits were set once per best-path slot (ants verified on the whole best path),
+        group_ranks_total: the same summed since begin."""
         out = np.zeros(4, np.uint32)
         check(lib().wr_acs_update_stats(self._need(), ptr(out)))
-        return dict(rankset_last=int(out[0]), deposit_tiles=int(out[1]), distinct_slots=int(out[2]), rankset_iterations=int(out[3]))
+        grp = np.zeros(2, np.uint64)
+        check(lib().wr_acs_group_stats(self._need(), ptr(grp)))
+        return dict(rankset_last=int(out[0]), deposit_tiles=int(out[1]), distinct_slots=int(out[2]), rankset_iterations=int(out[3]),
+                    group_ranks=int(grp[0]), group_ranks_total=int(grp[1]))
 
     def walkStats(self):
         """Converged iterations: ants completed by checking the best path against roulette thresholds, and the ant-steps that

@@ -150,7 +150,7 @@ struct wr_acs {
     float4* d_thr = nullptr;
     uint2* d_pmap = nullptr;
     uint32_t pmap_entries = 0;
-    int2* d_pv = nullptr;
+    int2* d_pv = nullptr;            // [0] {D, full} [1] {fresh: set by k_path_thresholds, consumed by k_rank_small, 0}; 16-byte aligned (one int4 load)
     int* d_vdev = nullptr;           // [chunk] steps each ant followed the best path
     // per-colony buffers (sized at begin)
     int* d_ant_steps = nullptr;      // global colony order (ranking input)
@@ -176,6 +176,7 @@ struct wr_acs {
     RankSet rs = {};
     size_t rs_entries = 0;
     int rs_groups = 1;                // apply launches per iteration: ceil(w_max / 1024)
+    uint32_t* d_grp_mask = nullptr;   // [rs_groups][32] group-deposit masks (k_rank_small -> k_rankset_gen): bit r = rank r is in the group
     int rs_policy = 0;                // 0 adaptive, 1 rank sets always, 2 records always (WR_RANKSET_POLICY)
     // adaptive choice: device -> host feedback through mapped pinned memory, host kept <= kRsAhead iterations ahead
     uint32_t* h_feedback = nullptr;   // ring of kFeedbackRing x {generation << 16 | iteration, path of the previous iteration, deposit tiles, row blocks}
@@ -341,6 +342,7 @@ static void free_colony_buffers(wr_acs* a)
     free_rankset(a);
     pool_free(a->d_ant_steps, s); pool_free(a->d_overflow, s); pool_free(a->d_ant_L, s); a->d_ant_L = nullptr;
     pool_free(a->d_vdev, s); a->d_vdev = nullptr;
+    pool_free(a->d_grp_mask, s); a->d_grp_mask = nullptr;
     if (!a->d_slab) { pool_free(a->d_path_ids, s); pool_free(a->d_path_dirs, s); }
     pool_free(a->d_gkeys, s); pool_free(a->d_gmasks, s); pool_free(a->d_resume, s); a->d_resume = nullptr; pool_free(a->d_rec_off, s); pool_free(a->d_order, s);
     a->d_local_steps = nullptr;   // aliases d_ant_steps (one GPU) or lives in the slab (sharded)
@@ -462,6 +464,7 @@ static int alloc_colony_buffers(wr_acs* a, int colony_max)
         a->rs_entries = R;
         a->rs.rmask = (uint32_t)(R - 1); a->rs.shift = 32 - log2R; a->rs.limit = limit;
         a->rs_groups = (a->w_max + kRsGroupRanks - 1) / kRsGroupRanks;
+        WR_CUDA(dmalloc(&a->d_grp_mask, (size_t)a->rs_groups * kRsRowWords * sizeof(uint32_t), s));
         if (!a->rs_ev[0]) {
             int rc = feedback_acquire(&a->h_feedback, &a->d_feedback);
             if (rc != WR_OK) return rc;
@@ -648,7 +651,8 @@ extern "C" int wr_acs_create(wr_grid* g, const wr_acs_params* p, wr_acs** out)
         while (a->pmap_entries < 2u * ((uint32_t)a->cap + 1)) a->pmap_entries <<= 1;
         WR_CUDA_A(dmalloc(&a->d_thr, ((size_t)a->cap + 1) * sizeof(float4), a->stream));
         WR_CUDA_A(dmalloc(&a->d_pmap, 2 * (size_t)a->pmap_entries * sizeof(uint2), a->stream));
-        WR_CUDA_A(dmalloc(&a->d_pv, sizeof(int2), a->stream));
+        WR_CUDA_A(dmalloc(&a->d_pv, 2 * sizeof(int2), a->stream));
+        WR_CUDA_A(cudaMemsetAsync(a->d_pv, 0, 2 * sizeof(int2), a->stream));
     }
     WR_CUDA_A(dmalloc(&a->d_tile_off, ((size_t)a->ntiles + 2) * sizeof(uint32_t), a->stream));
     WR_CUDA_A(dmalloc(&a->d_dep_list, ((size_t)a->ntiles + 2) * sizeof(uint32_t), a->stream));
@@ -895,8 +899,11 @@ static int launch_rank(wr_acs* a, const int* d_all_steps)
     const float* d_L = a->K == kK26 ? a->d_ant_L : nullptr;
     a->ants_in_b = false;
     if (cm <= 2 * kRankChunk) {   // the whole ranking in one single-CTA kernel
+        // group deposits: K = 6 rank-set handles, whose walk may verify the best path (k_rank_small decides per iteration on the device)
+        const bool grp = a->K == 6 && a->rankset && a->d_grp_mask && walk_verify() && a->rs_groups * kRsRowWords <= kRankGroupWords;
         k_rank_small<<<1, kRankSmallThreads, kRankSmallSmem, s>>>(a->d_state, d_all_steps, d_L, a->cap, a->rank_bits, a->d_Ltab, a->sort_ants.keys_a, a->sort_ants.vals_a,
-                                                                   a->d_rec_off, a->d_order, a->d_best_n, a->d_best_ids, a->d_onbest);
+                                                                   a->d_rec_off, a->d_order, a->d_best_n, a->d_best_ids, a->d_onbest, grp ? a->d_vdev : nullptr,
+                                                                   a->d_pv, a->rank * a->chunk, a->chunk, a->d_grp_mask, a->rs_groups * kRsRowWords);
     } else {                     // chunks of 4096 ants sorted in parallel, merged by rank counting, prefix-only finish
         const int nchunks = (cm + kRankChunk - 1) / kRankChunk;
         k_rank_chunks<<<nchunks, kRankSmallThreads, kRankChunkSmem, s>>>(a->d_state, d_all_steps, d_L, a->cap, a->rank_bits, a->sort_ants.keys_b, a->sort_ants.vals_b);
@@ -994,8 +1001,8 @@ static int launch_rankset_update(wr_acs* a)
 {
     cudaStream_t s = a->stream;
     const int first = a->rank * a->chunk;
-    k_rankset_gen<<<a->w_max, 128, 0, s>>>(a->d_state, rank_keys(a), rank_vals(a), a->d_path_ids, a->d_path_dirs, a->cap, (int)a->goal, a->d_Ltab, a->d_onbest,
-                                           a->rs, a->K, a->K == kK26 ? a->d_ant_steps : nullptr, first, a->chunk);
+    k_rankset_gen<<<a->w_max + kRsGroupCtas, kRsGenThreads, 0, s>>>(a->d_state, rank_keys(a), rank_vals(a), a->d_path_ids, a->d_path_dirs, a->cap, (int)a->goal, a->d_Ltab,
+                                                          a->d_onbest, a->rs, a->K, a->K == kK26 ? a->d_ant_steps : nullptr, first, a->chunk, a->d_grp_mask);
     if (a->nranks > 1) {
         k_rankset_publish<<<kNumSMs, 256, 0, s>>>(a->d_state, a->rs, a->pub_buf());
         k_rankset_merge<<<barrier_grid(a, kNumSMs * 2), 256, 0, s>>>(barrier_args(a), a->d_state, a->rs, reinterpret_cast<const uint32_t* const*>(a->tab(4, 0)), a->nranks, a->rank);
@@ -1859,6 +1866,16 @@ extern "C" int wr_acs_update_stats(wr_acs* a, uint32_t out[4])
     IterState st;
     WR_CUDA(cudaMemcpy(&st, a->d_state, sizeof st, cudaMemcpyDeviceToHost));
     out[0] = (uint32_t)st.use_rankset; out[1] = st.spread_tiles; out[2] = st.spread_slots; out[3] = st.rankset_iters;
+    return WR_OK;
+}
+
+extern "C" int wr_acs_group_stats(wr_acs* a, uint64_t out[2])
+{
+    WR_REQUIRE(a && out, WR_ERR_INVALID, "wr_acs_group_stats: null");
+    WR_CUDA(cudaStreamSynchronize(a->stream));
+    IterState st;
+    WR_CUDA(cudaMemcpy(&st, a->d_state, sizeof st, cudaMemcpyDeviceToHost));
+    out[0] = st.grp_ranks; out[1] = st.grp_ranks_total + st.grp_ranks;
     return WR_OK;
 }
 

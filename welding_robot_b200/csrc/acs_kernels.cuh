@@ -151,6 +151,7 @@ __global__ void k_begin(IterState* st, float predict)
     st->colony = 0; st->lambda = 0; st->Q = 0;
     st->n_eligible = 0; st->n_records = 0; st->n_records_sort = 0;
     st->use_rankset = 0; st->spread_tiles = 0xFFFFFFFFu; st->spread_slots = 0xFFFFFFFFu; st->rankset_iters = 0;
+    st->grp_rep = -1; st->grp_steps = 0; st->grp_ranks = 0; st->grp_ranks_total = 0;
 }
 
 // advance: the previous iteration's k_iter_end folded in (iterations enqueued back to back); upd_q: the fused update's
@@ -168,6 +169,7 @@ __global__ void k_iter_begin(IterState* st, int fixed_colony, int colony_max, fl
                              float rho = 1.0f)
 {   // :247-249
     if (advance) { st->iter++; st->cnt[6]++; st->base = __fmul_rn(st->base, rho); }
+    st->grp_ranks_total += st->grp_ranks; st->grp_ranks = 0;   // the previous iteration's group deposits (k_rank_small)
     if (rankset_count) {
         const int prev = st->use_rankset;
         if (st->iter > 0) { if (prev) st->spread_slots = rankset_count[1]; else if (upd_q) st->spread_tiles = upd_q[2]; }

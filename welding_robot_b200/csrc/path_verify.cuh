@@ -41,7 +41,8 @@ __device__ __forceinline__ uint32_t pos_lookup(const uint2* map, uint32_t mask, 
 
 // Thresholds of every best-path position t < best_n - 1 and the verifiable prefix D: the first t whose step k_walk3 might
 // not take the way thr[t] describes (any content of best_ids / best_dirs is checked, so a stale or broken path only
-// shortens D).  pv = {D, best_n - 1 if D == best_n - 1 else -1}.  map: 2 * map_entries entries (a power of two >= 2 * (cap + 1)).
+// shortens D).  pv[0] = {D, best_n - 1 if D == best_n - 1 else -1}; pv[1].x = 1 tells the ranking that follows that this
+// iteration's dev values are fresh (k_rank_small consumes it).  map: 2 * map_entries entries (a power of two >= 2 * (cap + 1)).
 __global__ void __launch_bounds__(kPathThreads) k_path_thresholds(const IterState* st, const int* best_n, const uint32_t* __restrict__ best_ids,
                                                                   const uint8_t* __restrict__ best_dirs, const float* __restrict__ tau,
                                                                   const float* __restrict__ heur, int alpha, int rx, int ry, int rz, int start, int goal,
@@ -51,7 +52,7 @@ __global__ void __launch_bounds__(kPathThreads) k_path_thresholds(const IterStat
     __shared__ uint32_t s_warp[kPathThreads / 32];
     const int n = *best_n;
     if (n < 2 || n > cap + 1) {   // no best path yet
-        if (threadIdx.x == 0) *pv = make_int2(0, -1);
+        if (threadIdx.x == 0) { pv[0] = make_int2(0, -1); pv[1] = make_int2(1, 0); }
         return;
     }
     const uint32_t N = (uint32_t)rx * (uint32_t)ry * (uint32_t)rz;
@@ -136,7 +137,8 @@ __global__ void __launch_bounds__(kPathThreads) k_path_thresholds(const IterStat
     }
     if (threadIdx.x == 0) {
         const int D = s_fail;
-        *pv = make_int2(D, D == n - 1 ? n - 1 : -1);
+        pv[0] = make_int2(D, D == n - 1 ? n - 1 : -1);
+        pv[1] = make_int2(1, 0);
     }
 }
 

@@ -8,6 +8,9 @@
 // (same warp, earlier round) or (same round, lower lane): a key's position inside its digit is
 //     prefix over (digit, warp) of the per-warp counts  +  count of this warp's earlier rounds  +  match-any rank
 // which makes every pass stable, hence the result the oracle's total order (key, ant index).
+// On rank-set iterations whose walk verified the whole best path, k_rank_small also marks the eligible ranks whose local ant
+// followed it (complete) in one 1024-bit mask per rank group, and names one of those ants the representative: k_rankset_gen
+// then sets their bits from that one trail (rankset.cuh).
 #pragma once
 #include "acs_kernels.cuh"
 
@@ -16,27 +19,37 @@ namespace wr {
 constexpr int kRankSmallMax = 16384;
 constexpr int kRankSmallThreads = 1024;
 constexpr int kRankSmallRounds = kRankSmallMax / kRankSmallThreads;   // 32-key rounds per warp
+constexpr int kRankGroupWords = 128;          // k_rank_small: group-mask words it can produce (4 rank groups: w_max <= 4096)
+constexpr uint16_t kRankComplete = 0x8000;   // k_rank_small: value bit of a complete ant (ant indices < kRankSmallMax use 14 bits)
 // dynamic shared memory: keys[2][max] (u32) + vals[2][max] (u16: ant indices < 65536) + whist[32][256] (u32) = 224 KB
 constexpr size_t kRankSmallSmem = (size_t)2 * kRankSmallMax * sizeof(uint32_t) + (size_t)2 * kRankSmallMax * sizeof(uint16_t) + (size_t)32 * 256 * sizeof(uint32_t);
 
-// Keys + stable sort of ants [first, first + n) in shared memory; returns which ping-pong buffer holds the result
-// (kbuf[src] keys, vbuf[src] ant indices relative to `first`).  All 1024 threads of the CTA take part.
-__device__ __forceinline__ int rank_sort_chunk(uint32_t* const kbuf[2], uint16_t* const vbuf[2], uint32_t* whist, uint32_t* warp_sum, const int* __restrict__ ant_steps,
-                                               const float* __restrict__ ant_L, int first, int n, int cap, int key_bits)
+// Keys of ants [first, first + n) -> kbuf[0], their indices relative to `first` -> vbuf[0] (k_rank_keys / k_rank_keys26).
+// full >= 0 (k_rank_small, group deposits): a local ant whose dev (k_path_verify) equals full is complete; its value gets
+// kRankComplete.  The dev loads run beside the step loads instead of behind the sort.
+__device__ __forceinline__ void rank_keys_chunk(uint32_t* kbuf0, uint16_t* vbuf0, const int* __restrict__ ant_steps, const float* __restrict__ ant_L, int first, int n, int cap,
+                                                const int* __restrict__ vdev = nullptr, int full = -1, int shard_first = 0, int shard_chunk = 0)
+{
+    const bool k26 = ant_L != nullptr;
+    for (int i = threadIdx.x; i < n; i += kRankSmallThreads) {
+        const int s = ant_steps[first + i];
+        const int la = first + i - shard_first;
+        const int dev = (vdev && la >= 0 && la < shard_chunk) ? vdev[la] : -2;   // not behind `full`: both loads in flight at once
+        const bool complete = full >= 0 && dev == full;
+        kbuf0[i] = k26 ? (s < 0 ? 0x7F800000u : __float_as_uint(ant_L[first + i])) : (s < 0 ? (uint32_t)(cap + 1) : (uint32_t)s);
+        vbuf0[i] = (uint16_t)i | (complete ? kRankComplete : (uint16_t)0);
+    }
+    __syncthreads();
+}
+
+// Stable sort of the n (key, value) pairs in kbuf[0] / vbuf[0]; returns which ping-pong buffer holds the result.  All 1024
+// threads of the CTA take part.
+__device__ __forceinline__ int rank_radix_sort(uint32_t* const kbuf[2], uint16_t* const vbuf[2], uint32_t* whist, uint32_t* warp_sum, int n, int key_bits)
 {
     constexpr unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const bool k26 = ant_L != nullptr;
     const int rounds = (n + kRankSmallThreads - 1) / kRankSmallThreads;   // per warp
     const int chunk = rounds * 32;
-
-    // ---- keys (k_rank_keys / k_rank_keys26) ----
-    for (int i = threadIdx.x; i < n; i += kRankSmallThreads) {
-        const int s = ant_steps[first + i];
-        kbuf[0][i] = k26 ? (s < 0 ? 0x7F800000u : __float_as_uint(ant_L[first + i])) : (s < 0 ? (uint32_t)(cap + 1) : (uint32_t)s);
-        vbuf[0][i] = (uint16_t)i;
-    }
-    __syncthreads();
 
     // ---- stable LSD radix sort, 8 bits per pass ----
     int src = 0;
@@ -101,12 +114,21 @@ __device__ __forceinline__ int rank_sort_chunk(uint32_t* const kbuf[2], uint16_t
     return src;
 }
 
+// Keys + stable sort of ants [first, first + n) in shared memory (kbuf[src] keys, vbuf[src] ant indices relative to `first`)
+__device__ __forceinline__ int rank_sort_chunk(uint32_t* const kbuf[2], uint16_t* const vbuf[2], uint32_t* whist, uint32_t* warp_sum, const int* __restrict__ ant_steps,
+                                               const float* __restrict__ ant_L, int first, int n, int cap, int key_bits)
+{
+    rank_keys_chunk(kbuf[0], vbuf[0], ant_steps, ant_L, first, n, cap);
+    return rank_radix_sort(kbuf, vbuf, whist, warp_sum, n, key_bits);
+}
+
 // steps26 / ant_L: K = 26 (key = bits of L); else key = steps (cap+1 for a dead ant), as k_rank_keys / k_rank_keys26.
 __global__ void __launch_bounds__(kRankSmallThreads) k_rank_small(IterState* st, const int* __restrict__ ant_steps, const float* __restrict__ ant_L, int cap,
                                                                    int key_bits, const float* __restrict__ Ltab, uint32_t* __restrict__ out_keys,
                                                                    uint32_t* __restrict__ out_vals, uint32_t* __restrict__ rec_off,
                                                                    int* __restrict__ order_of_ant, const int* __restrict__ best_n,
-                                                                   const uint32_t* __restrict__ best_ids, uint32_t* onbest)
+                                                                   const uint32_t* __restrict__ best_ids, uint32_t* onbest, const int* __restrict__ vdev,
+                                                                   int2* pv, int shard_first, int shard_chunk, uint32_t* __restrict__ gmask, int gwords)
 {
     extern __shared__ __align__(16) uint32_t rs_smem[];
     uint32_t* kbuf[2] = {rs_smem, rs_smem + kRankSmallMax};
@@ -115,12 +137,26 @@ __global__ void __launch_bounds__(kRankSmallThreads) k_rank_small(IterState* st,
     uint32_t* whist = rs_smem + 3 * kRankSmallMax;   // [warp][digit]
     __shared__ uint32_t warp_sum[32];
     __shared__ uint32_t carry, elig_total;
+    __shared__ uint32_t grp_cnt[32], grp_first[32];   // per warp: group ranks, lowest group rank (no shared atomics)
+    __shared__ uint32_t grp_words[kRankGroupWords];   // the masks, written to gmask once after the loop
 
     constexpr unsigned FULL = 0xffffffffu;
     const int n = st->colony;
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const bool k26 = ant_L != nullptr;
-    const int src = rank_sort_chunk(kbuf, vbuf, whist, warp_sum, ant_steps, ant_L, 0, n, cap, key_bits);
+    // group deposits (rankset.cuh, k_rankset_gen): only when k_path_thresholds ran in this very iteration (pv[1].x, consumed
+    // below) on a rank-set iteration — a device-side decision, so it also holds inside a captured iteration
+    int grp_full = -1;   // best_n - 1 if the whole path verified
+    if (vdev) {          // pv[0] and pv[1] in one load, beside use_rankset: no chain of dependent loads in front of the keys
+        const int4 p = *reinterpret_cast<const int4*>(pv);
+        const int use = st->use_rankset;
+        grp_full = (p.z != 0 && use) ? p.y : -1;
+    }
+    if (threadIdx.x < 32) { grp_cnt[threadIdx.x] = 0; grp_first[threadIdx.x] = 0xFFFFFFFFu; }
+    // complete ants (k_path_verify saw them follow the whole best path) carry bit 15 of their value through the sort
+    rank_keys_chunk(kbuf[0], vbuf[0], ant_steps, ant_L, 0, n, cap, vdev, grp_full, shard_first, shard_chunk);
+    if (vdev && threadIdx.x == 0) pv[1] = make_int2(0, 0);   // consumed: every thread has read it (before the barrier above)
+    const int src = rank_radix_sort(kbuf, vbuf, whist, warp_sum, n, key_bits);
     const uint32_t* keys = kbuf[src];
     const uint16_t* vals = vbuf[src];
 
@@ -133,15 +169,15 @@ __global__ void __launch_bounds__(kRankSmallThreads) k_rank_small(IterState* st,
             if (L0 < st->best_L) { st->best_steps = ant_steps[vals[0]]; st->best_L = L0; st->best_changed = 1; st->best_ant = (int)vals[0]; }
         } else if (n > 0) {
             const int s = (int)keys[0];
-            if (s <= cap && s < st->best_steps) { st->best_steps = s; st->best_L = Ltab[s]; st->best_changed = 1; st->best_ant = (int)vals[0]; }
+            if (s <= cap && s < st->best_steps) { st->best_steps = s; st->best_L = Ltab[s]; st->best_changed = 1; st->best_ant = (int)(vals[0] & ~kRankComplete); }
         }
     }
     __syncthreads();
     for (int base = 0; base < n; base += kRankSmallThreads) {
         const int r = base + threadIdx.x;
-        uint32_t len = 0; bool el = false;
+        uint32_t len = 0; bool el = false, grp = false;
         if (r < n) {
-            const uint32_t key = keys[r], ant = vals[r];
+            const uint32_t key = keys[r], ant = vals[r] & ~kRankComplete;
             out_keys[r] = key; out_vals[r] = ant;
             const int s = k26 ? ant_steps[ant] : (int)key;
             const bool arrived = k26 ? key != 0x7F800000u : s <= cap;
@@ -149,12 +185,21 @@ __global__ void __launch_bounds__(kRankSmallThreads) k_rank_small(IterState* st,
             order_of_ant[ant] = order;
             el = arrived && !((float)order > __fsub_rn(lambda, 1.0f));   // :200
             len = el ? (uint32_t)s : 0u;
+            // complete: a local ant that k_path_verify saw follow the whole best path (k_walk3 booked it with best_n - 1 steps and
+            // its trail rows are the best path's)
+            grp = el && (vals[r] & kRankComplete);
         }
         uint32_t incl = len;
         for (int o = 1; o < 32; o <<= 1) { const uint32_t u = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += u; }
         if (lane == 31) warp_sum[w] = incl;
         const unsigned em = __ballot_sync(FULL, el);
         if (lane == 0 && em) atomicAdd(&elig_total, (uint32_t)__popc(em));
+        if (grp_full >= 0) {   // CTA-uniform; word r >> 5 of the masks: bit r & 31 set iff rank r is in the group
+            const unsigned gm = __ballot_sync(FULL, grp);
+            const int word = (base >> 5) + w;
+            if (lane == 0 && word < gwords) grp_words[word] = gm;
+            if (lane == 0 && gm) { grp_cnt[w] += __popc(gm); grp_first[w] = min(grp_first[w], (uint32_t)(word * 32 + __ffs(gm) - 1)); }
+        }
         __syncthreads();
         if (w == 0) {
             const uint32_t s = warp_sum[lane];
@@ -170,6 +215,17 @@ __global__ void __launch_bounds__(kRankSmallThreads) k_rank_small(IterState* st,
         __syncthreads();
     }
     if (threadIdx.x == 0) { st->n_eligible = (int)elig_total; st->n_records = (int)carry; st->n_records_sort = st->use_rankset ? 0 : (int)carry; st->cnt[7] += carry; }
+    if (grp_full >= 0)   // every word of the groups the loop reached (eligible ranks are a prefix of them)
+        for (int i = threadIdx.x; i < gwords && i < ((n + kRankSmallThreads - 1) / kRankSmallThreads) * 32; i += kRankSmallThreads) gmask[i] = grp_words[i];
+    if (w == 0) {   // the group: its size and its representative, the ant of the lowest group rank (k_iter_begin adds the size to the total)
+        uint32_t c = grp_cnt[lane], f = grp_first[lane];
+        for (int o = 16; o > 0; o >>= 1) { c += __shfl_xor_sync(FULL, c, o); f = min(f, __shfl_xor_sync(FULL, f, o)); }
+        if (lane == 0) {
+            st->grp_rep = c ? (int)(vals[f] & ~kRankComplete) - shard_first : -1;
+            st->grp_steps = c ? grp_full : 0;
+            st->grp_ranks = c;
+        }
+    }
 
     // ---- k_best_clear: best = agentK (:264) drops the old best path's membership bits ----
     if (st->best_changed) {   // written by thread 0 before the barrier above
@@ -308,7 +364,10 @@ __global__ void __launch_bounds__(1024) k_rank_finish_prefix(IterState* st, cons
         if (threadIdx.x == 1023) carry = excl + len;
         __syncthreads();
     }
-    if (threadIdx.x == 0) { st->n_eligible = (int)elig_total; st->n_records = (int)carry; st->n_records_sort = st->use_rankset ? 0 : (int)carry; st->cnt[7] += carry; }
+    if (threadIdx.x == 0) {
+        st->n_eligible = (int)elig_total; st->n_records = (int)carry; st->n_records_sort = st->use_rankset ? 0 : (int)carry; st->cnt[7] += carry;
+        st->grp_rep = -1; st->grp_steps = 0; st->grp_ranks = 0;   // every eligible rank builds its own bits (k_rankset_gen)
+    }
     if (st->best_changed) {   // k_best_clear: written by thread 0 before the first barrier above
         const int nb = *best_n;
         for (int i = threadIdx.x; i < nb; i += 1024) {

@@ -18,7 +18,11 @@
 // k_deposit_serial — the reference's own loop order, exact for any input, slow, and in practice never taken.
 //
 //   k_rankset_gen     one CTA per eligible rank: value pair of the rank -> vtab; every step of its (local) trail:
-//                     find or claim the block of (slot, rank >> 10), set bit (rank & 1023); claimed blocks -> `list`
+//                     find or claim the block of (slot, rank >> 10), set bit (rank & 1023); claimed blocks -> `list`.
+//                     Group deposits (converged iterations): the ranks whose local ant k_path_verify saw follow the whole
+//                     best path cross the same slots with the same on-best bits, so k_rank_small lists them in one mask per
+//                     rank group and kRsGroupCtas CTAs of the same launch walk ONE such trail, OR-ing the masks into each
+//                     step's blocks; their own CTAs only write the vtab pair.  Same (key, bits) in the table, same field.
 //   k_rankset_publish / k_rankset_merge   sharded colonies: the claimed blocks (key + 32 words) are copied to the peer
 //                     slab, and every rank ORs every peer's blocks into its own table
 //   k_evaporate_lines (acs_kernels.cuh) tau *= rho over the dirty lines, :268-272 — the one HBM stream of the update
@@ -65,14 +69,81 @@ __device__ __forceinline__ uint32_t rankset_find_or_claim(const RankSet& rs, uns
     return 0xFFFFFFFFu;   // table completely full: cannot happen below the claim limit
 }
 
-// path_ids/path_dirs: THIS rank's trails (local ant index = global - shard_first); eligible ranks whose ant lives on
-// another rank only contribute their vtab pair here (their owner sets their bits and the merge brings them over).
-__global__ void __launch_bounds__(128) k_rankset_gen(const IterState* st, const uint32_t* __restrict__ rank_keys, const uint32_t* __restrict__ rank_vals,
-                                                      const uint32_t* __restrict__ path_ids, const uint8_t* __restrict__ path_dirs, int cap, int goal,
-                                                      const float* __restrict__ Ltab, const uint32_t* __restrict__ onbest, RankSet rs, int K,
-                                                      const int* __restrict__ steps26, int shard_first, int shard_chunk)
+constexpr int kRsGenThreads = 256;                 // k_rankset_gen: threads per CTA = steps per trip of one rank's trail
+constexpr int kRsGroupCtas = 1024 / kRsGenThreads;  // CTAs behind the per-rank ones that set the group's bits (1024 steps per trip)
+
+// The group's bits (k_rank_small: the eligible ranks whose local ant followed the whole best path): every such ant crossed the
+// same slots with the same on-best bits, so the representative's trail is walked ONCE and each group's 32 mask words are
+// OR-ed into the block of every step, one lane per word — instead of one find-or-claim + atomicOr per step and rank.  The
+// trail rows are the representative's own: k_best_copy may already have replaced the best path of this iteration.
+__device__ __forceinline__ void rankset_gen_group(const IterState* st, const uint32_t* __restrict__ path_ids, const uint8_t* __restrict__ path_dirs, int cap,
+                                                  int goal, const uint32_t* __restrict__ onbest, const RankSet& rs, int K, const uint32_t* __restrict__ gmask, int gc)
 {
     constexpr unsigned FULL = 0xffffffffu;
+    const int steps = st->grp_steps;
+    const size_t ant = (size_t)st->grp_rep;
+    const uint32_t* pid = path_ids + ant * cap;
+    const uint8_t* pdir = path_dirs + ant * cap;
+    const uint32_t groups = ((uint32_t)st->n_eligible + kRsGroupRanks - 1) / kRsGroupRanks;
+    const int lane = threadIdx.x & 31;
+    volatile uint32_t* over = rs.count + 3;
+    for (int i0 = gc * blockDim.x; i0 < steps; i0 += kRsGroupCtas * blockDim.x) {   // CTA-uniform trips
+        const int i = i0 + threadIdx.x;
+        uint32_t slot = 0;
+        bool onb = false;
+        if (i < steps) {   // the same expressions as the per-rank loop below
+            const uint32_t node = pid[i];
+            slot = node * (uint32_t)K + pdir[i];
+            const uint32_t next = (i + 1 < steps) ? pid[i + 1] : (uint32_t)goal;
+            onb = ((onbest[node >> 5] >> (node & 31)) & 1u) && ((onbest[next >> 5] >> (next & 31)) & 1u);
+        }
+        for (uint32_t g = 0; g < groups; g++) {
+            const uint32_t mw = gmask[g * kRsRowWords + lane];   // lane j holds word j of the group's mask
+            if (!__any_sync(FULL, mw != 0u)) continue;         // warp-uniform: no rank of this group is in the group path
+            const bool valid = i < steps && *over == 0u;
+            uint32_t h = 0xFFFFFFFFu;
+            bool claimed = false;
+            if (valid) {
+                const unsigned long long want = (unsigned long long)(slot + 1u) | ((unsigned long long)g << 32) | (onb ? (1ull << 63) : 0ull);
+                h = rankset_find_or_claim(rs, want, rankset_hash(slot, g) >> rs.shift, claimed);
+            }
+            const unsigned cm = __ballot_sync(FULL, claimed);
+            if (cm) {   // one counter update per warp, as in the per-rank loop
+                uint32_t at = 0;
+                if (lane == __ffs(cm) - 1) at = atomicAdd(rs.count, (uint32_t)__popc(cm));
+                at = __shfl_sync(FULL, at, __ffs(cm) - 1);
+                const uint32_t mine = at + __popc(cm & ((1u << lane) - 1u));
+                if (claimed) {
+                    if (mine < rs.limit) rs.list[mine] = h;
+                    else *over = 1u;
+                }
+            }
+            unsigned hm = __ballot_sync(FULL, h != 0xFFFFFFFFu);
+            while (hm) {   // the warp's steps one after the other, the 32 words of each block at once
+                const int src = __ffs(hm) - 1;
+                hm &= hm - 1;
+                const uint32_t hs = __shfl_sync(FULL, h, src);
+                if (mw) atomicOr(rs.rows + (size_t)hs * kRsRowWords + lane, mw);
+            }
+        }
+    }
+}
+
+// path_ids/path_dirs: THIS rank's trails (local ant index = global - shard_first); eligible ranks whose ant lives on
+// another rank only contribute their vtab pair here (their owner sets their bits and the merge brings them over).
+// Grid: w_max CTAs, one per rank, then kRsGroupCtas for the group (gmask, st->grp_rep).  A rank in the group only writes its
+// vtab pair: the group CTAs set its bits.
+__global__ void __launch_bounds__(kRsGenThreads) k_rankset_gen(const IterState* st, const uint32_t* __restrict__ rank_keys, const uint32_t* __restrict__ rank_vals,
+                                                      const uint32_t* __restrict__ path_ids, const uint8_t* __restrict__ path_dirs, int cap, int goal,
+                                                      const float* __restrict__ Ltab, const uint32_t* __restrict__ onbest, RankSet rs, int K,
+                                                      const int* __restrict__ steps26, int shard_first, int shard_chunk, const uint32_t* __restrict__ gmask)
+{
+    constexpr unsigned FULL = 0xffffffffu;
+    const int gc = (int)blockIdx.x - (int)(gridDim.x - kRsGroupCtas);
+    if (gc >= 0) {
+        if (st->use_rankset && st->grp_rep >= 0) rankset_gen_group(st, path_ids, path_dirs, cap, goal, onbest, rs, K, gmask, gc);
+        return;
+    }
     const int r = blockIdx.x;
     if (r >= st->n_eligible || !st->use_rankset) return;
     const int ant_global = (int)rank_vals[r];
@@ -86,6 +157,7 @@ __global__ void __launch_bounds__(128) k_rankset_gen(const IterState* st, const 
         rs.vtab[2 * r + 1] = __fadd_rn(base, elite);
     }
     if (ant_global < shard_first || ant_global >= shard_first + shard_chunk) return;   // another rank holds this trail
+    if (st->grp_rep >= 0 && ((gmask[r >> 5] >> (r & 31)) & 1u)) return;               // set by the group CTAs
     const size_t ant = (size_t)(ant_global - shard_first);
     const uint32_t* pid = path_ids + ant * cap;
     const uint8_t* pdir = path_dirs + ant * cap;

@@ -121,6 +121,12 @@ struct IterState {
     unsigned overflow_n; // ants whose shared-memory visited table overflowed (pass 2)
     unsigned long long cnt[9];
     unsigned long long verified[2];   // k_walk3: ants completed by path verification, ant-steps it decided (wr_acs_walk_stats)
+    // group deposits of a converged rank-set iteration (k_rank_small -> k_rankset_gen): eligible ranks whose local ant walked
+    // exactly the best path set their bits once per best-path slot, from the trail of one of them (the representative)
+    int grp_rep;         // local index of the representative ant, -1: no group this iteration
+    int grp_steps;       // its step count (best_n - 1 of the path it verified against)
+    unsigned grp_ranks;  // eligible ranks in the group this iteration (0 on iterations without rank sets; wr_acs_group_stats)
+    unsigned long long grp_ranks_total;   // the same, summed over the earlier iterations since begin (k_iter_begin adds grp_ranks)
 };
 
 }  // namespace wr
