@@ -280,6 +280,41 @@ public:
         }
         return const_cast<Vertex3<T>***>(cuboid_.data());
     }
+    // additions: clearance (include/wr_gpu.h, "Clearance").  Squared INDEX distance of every node to the nearest occupied
+    // node, z,y,x order; UINT32_MAX everywhere when none is occupied.
+    std::vector<uint32_t> clearanceMap()
+    {
+        std::vector<uint32_t> d2((size_t)size_of_map());
+        wr::check(wr_grid_clearance(grid_, d2.data(), d2.size()));
+        return d2;
+    }
+    // nearest node per point (per axis argmin |p - c[i]| in double, lowest index on ties) and its d2; either output may be NULL
+    void clearanceAt(const std::vector<Point3<T>>& pts, std::vector<int64_t>* ids, std::vector<uint32_t>* d2)
+    {
+        std::vector<float> xyz(3 * pts.size() + 3);
+        for (size_t i = 0; i < pts.size(); i++) { xyz[3 * i] = pts[i].x; xyz[3 * i + 1] = pts[i].y; xyz[3 * i + 2] = pts[i].z; }
+        if (ids) ids->resize(pts.size());
+        if (d2) d2->resize(pts.size());
+        wr::check(wr_grid_clearance_at(grid_, xyz.data(), (int)pts.size(), ids ? ids->data() : nullptr, d2 ? d2->data() : nullptr));
+    }
+    // replace the grid by its obstacles inflated by `radius` (world units): occupied iff d2 <= floor((radius / precision)^2).
+    // precision and wall keep their values; an ACS_Rank releases its search handle (release_grid) and creates a new one on next use.
+    void inflateGridMap(T radius)
+    {
+        if (!grid_) throw wr::Error(WR_ERR_STATE, "inflateGridMap: no grid map");
+        if (!(radius >= 0)) throw wr::Error(WR_ERR_INVALID, "inflateGridMap: radius must be >= 0");
+        const double r = (double)radius / (double)precision;
+        const double r2 = floor(r * r);
+        wr_grid* inflated = nullptr;
+        wr::check(wr_grid_inflate(grid_, r2 >= 4294967295.0 ? 0xffffffffu : (uint32_t)r2, &inflated));
+        const T p = precision;
+        const int w = wall;
+        release_grid();
+        grid_ = inflated;
+        adopt();
+        precision = p; wall = w;
+    }
+
     int size_of_map() const { return rangeX * rangeY * rangeZ; }
     void plot_grid_map(int) {}   // plotting (model_grid_map.hpp:368-379) is out of scope
     void show_plot() {}

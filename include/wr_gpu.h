@@ -75,6 +75,28 @@ int wr_grid_download_isfree(const wr_grid* g, uint8_t* isfree, size_t n);
 int wr_grid_stats(const wr_grid* g, uint64_t* occupied, uint64_t* tests, float* kernel_ms);
 
 /* ------------------------------------------------------------------------------------------
+ * Clearance — an addition with no reference counterpart (the reference never asks how close a
+ * path comes to the part).  d2 of a node = min over occupied nodes of the squared INDEX distance
+ * (dx^2 + dy^2 + dz^2), exact, 0 on occupied nodes.  World distance ~= sqrt(d2) * precision in the
+ * interior; the max-side wall planes are irregular (possibly a duplicate plane), so no exact
+ * world-unit figure exists there.  The field is built on the device on first use (three
+ * separable passes) and cached in the grid handle (4 B per node) until wr_grid_destroy.  Grids
+ * with an axis longer than 32768 nodes give WR_ERR_INVALID.
+ * ---------------------------------------------------------------------------------------- */
+/* squared index distance of every node to the nearest occupied node (N entries, z,y,x order); UINT32_MAX if none is occupied */
+int wr_grid_clearance(wr_grid* g, uint32_t* d2, size_t n);
+/* per point (3 floats): the nearest node on each axis = argmin_i |p - c[i]| evaluated in double, lowest index on ties
+ * (duplicate planes, midpoints); points beyond the grid map to the boundary node; a non-finite coordinate gives
+ * ids[i] = -1, d2[i] = UINT32_MAX.  ids / d2 may each be NULL. */
+int wr_grid_clearance_at(wr_grid* g, const float* pts_xyz, int npoints, int64_t* ids, uint32_t* d2);
+/* a NEW grid: node occupied iff d2 <= r2 (r2 = 0: the same occupancy).  Same dims, coordinates, precision, wall, bbox;
+ * wr_grid_stats of the result: its own occupied count, tests = 0, kernel_ms = 0.  Every wr_acs_* call works on it unchanged
+ * (a route point whose 1.2*precision box holds no free node any more fails to snap, as on any grid). */
+int wr_grid_inflate(wr_grid* g, uint32_t r2, wr_grid** out);
+/* device ms of the passes that built the field (CUDA events; 0 before the first build) */
+int wr_grid_clearance_ms(const wr_grid* g, float* ms);
+
+/* ------------------------------------------------------------------------------------------
  * Rank-based 3-D ant colony search — replaces ACS_Rank (core/ACSRank_3D.hpp).
  * ---------------------------------------------------------------------------------------- */
 typedef struct {

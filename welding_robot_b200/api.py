@@ -198,6 +198,40 @@ class GridMap:
         check(lib().wr_grid_stats(self._g, C.byref(occ), C.byref(tests), C.byref(ms)))
         return dict(occupied=occ.value, tests=tests.value, kernel_ms=ms.value)
 
+    # -- clearance (an addition: the reference never measures how close a path comes to the part) --------------------
+    def clearanceMap(self):
+        """uint32[N] in z,y,x order: squared INDEX distance of every node to the nearest occupied node (0 on occupied nodes,
+        UINT32_MAX everywhere when none is occupied).  World distance ~= sqrt(d2) * precision away from the max-side wall
+        planes.  Built on the device on first use and kept with the grid."""
+        out = np.zeros(self.size_of_map(), np.uint32)
+        check(lib().wr_grid_clearance(self._g, ptr(out), out.size))
+        return out
+
+    def clearanceAt(self, points):
+        """Per point: the nearest node (per axis argmin |p - c[i]| in double, lowest index on ties; beyond the grid: the
+        boundary node) and its d2.  -> (int64 ids, uint32 d2); a non-finite coordinate gives -1 / UINT32_MAX."""
+        pts = np.ascontiguousarray(np.asarray(points, np.float32).reshape(-1, 3))
+        ids = np.zeros(len(pts), np.int64); d2 = np.zeros(len(pts), np.uint32)
+        check(lib().wr_grid_clearance_at(self._g, ptr(pts), len(pts), ptr(ids), ptr(d2)))
+        return ids, d2
+
+    def inflateGridMap(self, radius):
+        """Replace the grid by its obstacles inflated by `radius` (world units): a node becomes occupied iff its squared index
+        distance to the part is <= floor((radius / precision)^2).  Dims, coordinates, precision and wall stay; an ACS_Rank
+        drops its search handle and creates a new one on next use."""
+        if self._g is None:
+            raise _lib.WrError(-4, "inflateGridMap: no grid map")
+        if not radius >= 0:
+            raise ValueError("inflateGridMap: radius must be >= 0")
+        r2 = min(math.floor((float(radius) / float(self.precision)) ** 2), 0xFFFFFFFF)
+        h = C.c_void_p()
+        check(lib().wr_grid_inflate(self._g, r2, C.byref(h)))
+        precision, wall = self.precision, self.wall
+        self._destroy_grid()
+        self._adopt(h)
+        self.precision, self.wall = precision, wall
+        return self
+
     def node(self, node_id):
         """The Vertex3 of a node id (materialised on demand; ptr_grid_map()'s cuboid is never built)."""
         xs, ys, zs = self.coords()

@@ -238,7 +238,7 @@ static float axis_coord(int i, int range, int wall, float mn, float mx, float pr
     return i < wall ? mn - (wall - i) * precision : (i >= (range - wall) ? mx + (i - range + wall) * precision : mn + (i - wall) * precision);
 }
 
-static int grid_alloc_common(wr_grid* g)
+int grid_alloc_common(wr_grid* g)
 {
     WR_CUDA(cudaGetDevice(&g->device));
     g->N = (size_t)g->rx * g->ry * g->rz;
@@ -405,7 +405,7 @@ extern "C" int wr_grid_create_from_occupancy(const uint8_t* isfree, int rx, int 
 extern "C" int wr_grid_destroy(wr_grid* g)
 {
     if (!g) return WR_OK;
-    pool_free(g->d_coords, 0); pool_free(g->d_bits, 0); pool_free(g->d_open6, 0);
+    pool_free(g->d_coords, 0); pool_free(g->d_bits, 0); pool_free(g->d_open6, 0); pool_free(g->d_clear, 0);
     delete g;
     return WR_OK;
 }

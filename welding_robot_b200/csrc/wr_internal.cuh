@@ -16,14 +16,19 @@ struct wr_grid {
     size_t nwords = 0;
     uint8_t* d_open6 = nullptr;           // per node: bit k set <=> neighbour k in bounds and free (built on demand)
     std::vector<uint32_t> h_bits;         // host mirror for endpoint snapping (filled on demand)
+    uint32_t* d_clear = nullptr;          // per node: squared index distance to the nearest occupied node (built on demand)
     uint64_t occupied = 0, tests = 0;
     float vox_ms = 0;
+    float clear_ms = 0;                   // device ms of the passes that built d_clear
 };
 
 namespace wr {
 // grid.cu
+int grid_alloc_common(wr_grid* g);
 int grid_ensure_open6(wr_grid* g, cudaStream_t s);
 int grid_ensure_host_bits(wr_grid* g);
+// clearance.cu
+int grid_ensure_clearance(wr_grid* g);
 inline bool grid_is_free_host(const wr_grid* g, size_t id) { return !((g->h_bits[id >> 5] >> (id & 31)) & 1u); }
 
 // radix_sort.cu — stable LSD radix sort of (u32 key, u32 value) pairs, count on the device.
