@@ -301,18 +301,48 @@ public:
     // precision and wall keep their values; an ACS_Rank releases its search handle (release_grid) and creates a new one on next use.
     void inflateGridMap(T radius)
     {
-        if (!grid_) throw wr::Error(WR_ERR_STATE, "inflateGridMap: no grid map");
-        if (!(radius >= 0)) throw wr::Error(WR_ERR_INVALID, "inflateGridMap: radius must be >= 0");
-        const double r = (double)radius / (double)precision;
-        const double r2 = floor(r * r);
+        const uint32_t r2 = radius_r2(radius, "inflateGridMap");
         wr_grid* inflated = nullptr;
-        wr::check(wr_grid_inflate(grid_, r2 >= 4294967295.0 ? 0xffffffffu : (uint32_t)r2, &inflated));
+        wr::check(wr_grid_inflate(grid_, r2, &inflated));
         const T p = precision;
         const int w = wall;
         release_grid();
         grid_ = inflated;
         adopt();
         precision = p; wall = w;
+    }
+
+    // addition: greedy line-of-sight shortcutting of node rows (include/wr_gpu.h, wr_grid_shortcut_paths), all rows in one
+    // launch.  Segments keep clear of every node with d2 <= floor((radius / precision)^2) (radius 0: of occupied nodes); from
+    // each waypoint the next is the furthest row node, at most max_span ahead (0: no bound), whose segment is clear, else the
+    // next node (counted in `blocked`).
+    struct ShortcutRow {
+        std::vector<int64_t> ids;    // waypoint node ids
+        std::vector<int32_t> keep;   // their indices into the row
+        int blocked = 0;             // segments kept by the fallback
+        double length = 0;           // world length of the waypoint polyline
+    };
+    std::vector<ShortcutRow> shortcutPaths(const std::vector<std::vector<int64_t>>& paths, T radius = 0, int max_span = 0)
+    {
+        const uint32_t r2 = radius_r2(radius, "shortcutPaths");
+        const int nrows = (int)paths.size();
+        std::vector<int64_t> off(paths.size() + 1, 0), ids;
+        for (int p = 0; p < nrows; p++) {
+            off[p + 1] = off[p] + (int64_t)paths[p].size();
+            ids.insert(ids.end(), paths[p].begin(), paths[p].end());
+        }
+        std::vector<int32_t> keep(ids.size() + 1), nkeep(paths.size() + 1), blocked(paths.size() + 1);
+        std::vector<double> length(paths.size() + 1);
+        wr::check(wr_grid_shortcut_paths(grid_, ids.data(), off.data(), nrows, r2, max_span, keep.data(), nkeep.data(), blocked.data(),
+                                         length.data()));
+        std::vector<ShortcutRow> out(paths.size());
+        for (int p = 0; p < nrows; p++) {
+            out[p].keep.assign(keep.begin() + off[p], keep.begin() + off[p] + nkeep[p]);
+            for (int32_t k : out[p].keep) out[p].ids.push_back(paths[p][k]);
+            out[p].blocked = blocked[p];
+            out[p].length = length[p];
+        }
+        return out;
     }
 
     int size_of_map() const { return rangeX * rangeY * rangeZ; }
@@ -327,6 +357,15 @@ public:
 protected:
     wr_grid* grid_ = nullptr;
     std::vector<float> xs_, ys_, zs_;
+    // a world radius as a squared index radius: floor((radius / precision)^2), saturating at UINT32_MAX
+    uint32_t radius_r2(T radius, const char* who) const
+    {
+        if (!grid_) throw wr::Error(WR_ERR_STATE, std::string(who) + ": no grid map");
+        if (!(radius >= 0)) throw wr::Error(WR_ERR_INVALID, std::string(who) + ": radius must be >= 0");
+        const double r = (double)radius / (double)precision;
+        const double r2 = floor(r * r);
+        return r2 >= 4294967295.0 ? 0xffffffffu : (uint32_t)r2;
+    }
     void load_coords()
     {
         if (!xs_.empty()) return;
@@ -546,6 +585,38 @@ public:
         }
     }
 
+    // addition: best_matrix with every best path shortcut (shortcutPaths, one launch for all pairs): Agents whose path is the
+    // waypoint nodes, with no node_index and L = the waypoint polyline's world length; read_all_segments stitches it like
+    // best_matrix.  Entries without a path are copied as they are.  Owned by this object and freed with best_matrix (by the
+    // next searchBestPathOfPoints or shortcutBestMatrix, or the destructor).
+    Agent<float>** shortcutBestMatrix(float radius = 0, int max_span = 0)
+    {
+        if (!best_matrix) throw wr::Error(WR_ERR_STATE, "shortcutBestMatrix: no best_matrix (run searchBestPathOfPoints first)");
+        std::vector<std::pair<int, int>> pairs;
+        std::vector<std::vector<int64_t>> rows;
+        for (int i = 0; i < matrix_n_; i++)
+            for (int j = i + 1; j < matrix_n_; j++) {
+                const std::vector<ACS_Node<float>*>* path = best_matrix[i][j].getPath();
+                if (path->empty()) continue;
+                pairs.push_back(std::make_pair(i, j));
+                rows.emplace_back();
+                for (auto nd : *path) rows.back().push_back((int64_t)nd->id);
+            }
+        const std::vector<ShortcutRow> res = shortcutPaths(rows, radius, max_span);
+        free_shortcut_matrix();
+        shortcut_matrix_ = new Agent<float>*[matrix_n_];
+        for (int i = 0; i < matrix_n_; i++) {
+            shortcut_matrix_[i] = new Agent<float>[matrix_n_];
+            for (int j = 0; j < matrix_n_; j++) shortcut_matrix_[i][j] = best_matrix[i][j];
+        }
+        for (size_t q = 0; q < pairs.size(); q++) {
+            const int i = pairs[q].first, j = pairs[q].second;
+            make_agent(shortcut_matrix_[i][j], res[q].ids.data(), nullptr, (int)res[q].ids.size(), (float)res[q].length);
+            shortcut_matrix_[j][i] = shortcut_matrix_[i][j];
+        }
+        return shortcut_matrix_;
+    }
+
     void plot_path(Agent<float>&, int) {}   // :567-598, plotting out of scope
     void plot_route_point(int) {}
 
@@ -561,6 +632,7 @@ private:
     Agent<float> best_;
     std::deque<ACS_Node<float>> pool_;   // nodes handed out through paths; stable addresses for the object's lifetime
     int matrix_n_ = 0;
+    Agent<float>** shortcut_matrix_ = NULL;
 
     void need() { if (!acs_) initFromGridMap(); }
     void release_acs()
@@ -568,13 +640,22 @@ private:
         if (acs_) wr_acs_destroy(acs_);
         acs_ = nullptr;
     }
+    void free_shortcut_matrix()
+    {
+        if (!shortcut_matrix_) return;
+        for (int i = 0; i < matrix_n_; i++) delete[] shortcut_matrix_[i];
+        delete[] shortcut_matrix_;
+        shortcut_matrix_ = NULL;
+    }
     void free_matrix()
     {
+        free_shortcut_matrix();
         if (!best_matrix) return;
         for (int i = 0; i < matrix_n_; i++) delete[] best_matrix[i];
         delete[] best_matrix;
         best_matrix = NULL;
     }
+    // dirs == NULL: a path of waypoints, which has no node_index
     void make_agent(Agent<float>& out, const int64_t* ids, const int* dirs, int n, float L)
     {
         std::vector<ACS_Node<float>*> p;
@@ -584,7 +665,8 @@ private:
             nd.id = (unsigned long)ids[i]; nd.isFree = true; nd.pt = node_point(nd.id);
             p.push_back(&nd);
         }
-        std::vector<int> d(dirs, dirs + (n > 0 ? n - 1 : 0));
+        std::vector<int> d;
+        if (dirs) d.assign(dirs, dirs + (n > 0 ? n - 1 : 0));
         out.assign(p, d, L);
     }
     void fetch_best(Agent<float>& out)

@@ -97,6 +97,27 @@ int wr_grid_inflate(wr_grid* g, uint32_t r2, wr_grid** out);
 int wr_grid_clearance_ms(const wr_grid* g, float* ms);
 
 /* ------------------------------------------------------------------------------------------
+ * Shortcutting — an addition with no reference counterpart: pull node rows (searched paths, ant
+ * trails, any polyline of node ids) straight wherever the free space allows.  In index space a
+ * node (x,y,z) owns the closed cube [x-1/2, x+1/2] x [y-1/2, y+1/2] x [z-1/2, z+1/2]; the cover of
+ * the segment between two nodes is every cube that meets the closed segment (through an edge or a
+ * corner: every cube that shares it).  A cube blocks iff d2 <= r2 (r2 = 0: iff it is occupied; the
+ * field is then never built), so shortcutting g at r2 equals shortcutting wr_grid_inflate(g, r2)
+ * at 0.  Greedy waypoints: w0 = 0; w_{k+1} = the largest j in (w_k, min(n-1, w_k + span)] whose
+ * segment (p[w_k], p[j]) has no blocking cube, else w_k + 1 (the row's own segment is kept and
+ * counted in `blocked`); span = max_span > 0 ? max_span : n.  Length: sum in order of the world
+ * segment lengths in double from the float coordinate tables.  Index straightness is world
+ * straightness except across the irregular max-side wall planes.  One launch for all rows.
+ * r2 > 0 builds the clearance field if needed (axes longer than 32768 nodes: WR_ERR_INVALID).
+ * ---------------------------------------------------------------------------------------- */
+/* rows: row p = ids[offsets[p] .. offsets[p+1]); offsets[0] = 0, non-decreasing.  keep[offsets[p] .. + nkeep[p]) receives the
+ * indices (into row p) of its greedy waypoints; blocked[p] = segments kept by the fallback; length[p] = world length of
+ * the waypoint polyline.  Any output pointer but keep/nkeep may be NULL.  Ids outside [0, N), bad offsets, a row longer
+ * than INT32_MAX, nrows < 0 or max_span < 0: WR_ERR_INVALID, nothing written.  A 0-node row gives nkeep = 0, length 0. */
+int wr_grid_shortcut_paths(wr_grid* g, const int64_t* ids, const int64_t* offsets, int nrows, uint32_t r2, int max_span,
+                           int32_t* keep, int32_t* nkeep, int32_t* blocked, double* length);
+
+/* ------------------------------------------------------------------------------------------
  * Rank-based 3-D ant colony search — replaces ACS_Rank (core/ACSRank_3D.hpp).
  * ---------------------------------------------------------------------------------------- */
 typedef struct {

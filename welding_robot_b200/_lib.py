@@ -34,7 +34,7 @@ class AcsParams(C.Structure):
 SYMBOLS = """wr_last_error wr_version wr_device_count wr_set_device wr_release_caches wr_stl_parse
 wr_grid_create_from_triangles wr_grid_create_from_occupancy wr_grid_destroy wr_grid_dims wr_grid_precision
 wr_grid_bbox wr_grid_coords wr_grid_download_bits wr_grid_download_isfree wr_grid_stats
-wr_grid_clearance wr_grid_clearance_at wr_grid_inflate wr_grid_clearance_ms
+wr_grid_clearance wr_grid_clearance_at wr_grid_inflate wr_grid_clearance_ms wr_grid_shortcut_paths
 wr_acs_default_params wr_acs_create wr_acs_destroy wr_acs_set_points wr_acs_set_endpoints wr_acs_snap_points wr_acs_search_pairs wr_acs_search_batch wr_acs_result_path wr_acs_batch_stats wr_acs_begin wr_acs_set_next_search
 wr_acs_iterate wr_acs_sync wr_acs_reset wr_acs_best wr_acs_download_pheromone wr_acs_upload_pheromone
 wr_acs_last_colony wr_acs_last_ant wr_acs_counters wr_acs_kernel_ms wr_acs_update_stats wr_acs_group_stats wr_acs_walk_stats wr_acs_field_stats wr_acs_field_lines wr_acs_stream_kernel_ms wr_acs_set_timing wr_acs_bench_kernel wr_acs_set_stream
@@ -73,6 +73,7 @@ def lib():
         "wr_grid_download_isfree": [vp, vp, C.c_size_t], "wr_grid_stats": [vp, vp, vp, vp],
         "wr_grid_clearance": [vp, vp, C.c_size_t], "wr_grid_clearance_at": [vp, vp, i32, vp, vp],
         "wr_grid_inflate": [vp, C.c_uint32, vp], "wr_grid_clearance_ms": [vp, vp],
+        "wr_grid_shortcut_paths": [vp, vp, vp, i32, C.c_uint32, i32, vp, vp, vp, vp],
         "wr_acs_default_params": [C.POINTER(AcsParams)], "wr_acs_create": [vp, C.POINTER(AcsParams), vp],
         "wr_acs_destroy": [vp], "wr_acs_set_points": [vp, vp, vp, vp], "wr_acs_set_endpoints": [vp, i64, i64],
         "wr_acs_snap_points": [vp, vp, i32, vp], "wr_acs_search_pairs": [vp, vp, vp, i32, f32, i32, vp, vp, vp, vp, i32],

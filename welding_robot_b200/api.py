@@ -215,15 +215,19 @@ class GridMap:
         check(lib().wr_grid_clearance_at(self._g, ptr(pts), len(pts), ptr(ids), ptr(d2)))
         return ids, d2
 
+    def _radius_r2(self, radius, who):
+        """A world radius as a squared index radius: floor((radius / precision)^2), saturating at UINT32_MAX."""
+        if self._g is None:
+            raise _lib.WrError(-4, "%s: no grid map" % who)
+        if not radius >= 0:
+            raise ValueError("%s: radius must be >= 0" % who)
+        return min(math.floor((float(radius) / float(self.precision)) ** 2), 0xFFFFFFFF)
+
     def inflateGridMap(self, radius):
         """Replace the grid by its obstacles inflated by `radius` (world units): a node becomes occupied iff its squared index
         distance to the part is <= floor((radius / precision)^2).  Dims, coordinates, precision and wall stay; an ACS_Rank
         drops its search handle and creates a new one on next use."""
-        if self._g is None:
-            raise _lib.WrError(-4, "inflateGridMap: no grid map")
-        if not radius >= 0:
-            raise ValueError("inflateGridMap: radius must be >= 0")
-        r2 = min(math.floor((float(radius) / float(self.precision)) ** 2), 0xFFFFFFFF)
+        r2 = self._radius_r2(radius, "inflateGridMap")
         h = C.c_void_p()
         check(lib().wr_grid_inflate(self._g, r2, C.byref(h)))
         precision, wall = self.precision, self.wall
@@ -231,6 +235,27 @@ class GridMap:
         self._adopt(h)
         self.precision, self.wall = precision, wall
         return self
+
+    def shortcutPaths(self, paths, radius=0.0, max_span=0):
+        """Greedy line-of-sight shortcutting of node rows (include/wr_gpu.h, wr_grid_shortcut_paths), all rows in one launch.
+        A segment between two nodes is kept clear of every node whose squared index distance to the part is <=
+        floor((radius / precision)^2) (radius 0: of occupied nodes); from each waypoint the next one is the furthest row
+        node, at most `max_span` ahead (0: no bound), whose segment is clear, else the next node.  -> per row
+        (waypoint ids, keep indices into the row, blocked = segments kept by that fallback, world length in double)."""
+        r2 = self._radius_r2(radius, "shortcutPaths")
+        rows = [np.asarray(p, np.int64).ravel() for p in paths]
+        off = np.zeros(len(rows) + 1, np.int64)
+        off[1:] = np.cumsum([len(r) for r in rows])
+        ids = np.ascontiguousarray(np.concatenate(rows) if rows else np.zeros(0, np.int64))
+        keep = np.zeros(max(len(ids), 1), np.int32)
+        nkeep = np.zeros(max(len(rows), 1), np.int32); blocked = np.zeros_like(nkeep); length = np.zeros(len(nkeep), np.float64)
+        check(lib().wr_grid_shortcut_paths(self._g, ptr(ids), ptr(off), len(rows), r2, int(max_span), ptr(keep), ptr(nkeep),
+                                           ptr(blocked), ptr(length)))
+        out = []
+        for p, r in enumerate(rows):
+            k = keep[off[p]:off[p] + nkeep[p]].copy()
+            out.append((r[k], k, int(blocked[p]), float(length[p])))
+        return out
 
     def node(self, node_id):
         """The Vertex3 of a node id (materialised on demand; ptr_grid_map()'s cuboid is never built)."""
@@ -485,6 +510,21 @@ class ACS_Rank(GridMap):
                 for L in lengths:
                     fp.write("%.3f\n" % L)
             print("[ACS 3D] %d Result has been written to \"%s\" \r" % (len(lengths), output_file))
+
+    def shortcutBestMatrix(self, radius=0.0, max_span=0):
+        """best_matrix with every best path shortcut (GridMap.shortcutPaths, one launch for all pairs): a new matrix of Agents
+        whose ids are the waypoint ids, with empty dirs and L = float32 of the waypoint polyline's world length; [i][j] and
+        [j][i] share one object as in best_matrix.  ACS_GTSP.read_all_segments stitches it like best_matrix.  Entries
+        without a path are copied as they are."""
+        if self.best_matrix is None:
+            raise _lib.WrError(-4, "shortcutBestMatrix: no best_matrix (run searchBestPathOfPoints first)")
+        n = len(self.best_matrix)
+        pairs = [(i, j) for i in range(n) for j in range(i + 1, n) if len(self.best_matrix[i][j].ids)]
+        res = self.shortcutPaths([self.best_matrix[i][j].ids for i, j in pairs], radius, max_span)
+        out = [[Agent(self, L=self.best_matrix[i][j].L) for j in range(n)] for i in range(n)]
+        for (i, j), (ids, _, _, L) in zip(pairs, res):
+            out[i][j] = out[j][i] = Agent(self, ids, None, float(np.float32(L)))
+        return out
 
     # -- introspection (parity tests, bench) -----------------------------------------------
     def pheromone(self):
